@@ -269,7 +269,10 @@ typedef struct {
 } msnv_cov_blocks;
 
 /* Per contig: cov_sum[k] = sum of coverage over indices [0, chrSize) and hist[k][c] for
- * c = 0..max_cov = number of indices with min(coverage, max_cov) == c (qaCompute.cpp:142-165). */
+ * c = 0..max_cov = number of indices with min(coverage, max_cov) == c (qaCompute.cpp:142-165).
+ * Any max_cov is exact; the histograms of one call may hold at most MSNV_COV_MAX_COUNTERS counters
+ * (n_contigs x (max_cov + 1), 8 bytes each on the device and in `hist`), more is MSNV_E_LIMIT. */
+#define MSNV_COV_MAX_COUNTERS (1u << 27)
 int msnv_cov_run(msnv_ctx* ctx, const msnv_cov_blocks* blocks, uint32_t max_cov, uint64_t* cov_sum, uint64_t* hist);
 
 #ifdef __cplusplus

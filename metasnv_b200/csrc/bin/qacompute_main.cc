@@ -164,6 +164,10 @@ int main(int argc, char* argv[])
 
     // ---- GPU: per-contig coverage sum and clamped histogram (qaCompute.cpp:142-165)
     const uint32_t K = (uint32_t)seen_tid.size();
+    if ((uint64_t)std::max<uint32_t>(K, 1) * ((uint64_t)maxCoverage + 1) > MSNV_COV_MAX_COUNTERS) {
+        fprintf(stderr, "qaCompute: -c %d needs more than %u histogram counters for %u contigs\n", maxCoverage, (unsigned)MSNV_COV_MAX_COUNTERS, K);
+        return 1;
+    }
     const uint32_t bins = (uint32_t)maxCoverage + 1;
     std::vector<uint64_t> cov_sum(K, 0), hist((size_t)K * bins, 0);
     if (K) {

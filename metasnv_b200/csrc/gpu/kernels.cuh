@@ -1664,10 +1664,12 @@ __global__ void text_tiles_kernel(const uint64_t* __restrict__ acgt, const uint1
 // of COV_CHUNK. A block [beg,end) contributes +1 at beg and -1 at end like the reference's
 // difference array, but every chunk it enters gets its own +1 at the chunk's first index, so each
 // chunk is prefix-summed independently by one CTA: no carries between CTAs, one pass over HBM.
+// The histogram's first COV_MAX_BINS bins are collected in shared memory; coverage values above
+// them (qaCompute -c 1024 and more, deep spots only) go straight to the global histogram.
 // ------------------------------------------------------------------------------------------------
 constexpr int COV_CHUNK = 4096;
 constexpr int COV_THREADS = 256;              // x 16 positions per thread = one chunk
-constexpr int COV_MAX_BINS = 1024;
+constexpr int COV_MAX_BINS = 1024;            // bins held in shared memory
 
 __global__ void __launch_bounds__(256)
 cov_scatter_kernel(const uint32_t* __restrict__ beg, const uint32_t* __restrict__ end, const uint64_t* __restrict__ blk_off,
@@ -1702,7 +1704,9 @@ cov_scan_kernel(const int32_t* __restrict__ diff, const uint32_t* __restrict__ c
     const uint32_t k = chunk_contig[blockIdx.x];
     const uint32_t first = (blockIdx.x - contig_chunk0[k]) * COV_CHUNK;        // contig coordinate of the chunk's first index
     const uint32_t len = contig_len[k];
-    for (uint32_t i = tid; i <= max_cov; i += COV_THREADS) s_hist[i] = 0;
+    const uint32_t n_shared = max_cov < (uint32_t)COV_MAX_BINS ? max_cov + 1u : (uint32_t)COV_MAX_BINS;
+    unsigned long long* const g_hist = hist + (size_t)k * ((size_t)max_cov + 1);
+    for (uint32_t i = tid; i < n_shared; i += COV_THREADS) s_hist[i] = 0;
     if (tid == 0) s_sum = 0;
     const int4* src = reinterpret_cast<const int4*>(diff + (size_t)blockIdx.x * COV_CHUNK) + 4 * tid;
     const int4 v[4] = {src[0], src[1], src[2], src[3]};
@@ -1729,14 +1733,17 @@ cov_scan_kernel(const int32_t* __restrict__ diff, const uint32_t* __restrict__ c
         if (!valid) bin = 0xffffffffu;
         else local += (unsigned long long)(cv < 0 ? 0 : cv);
         const uint32_t peers = __match_any_sync(0xffffffffu, bin);
-        if (valid && lane == (uint32_t)(__ffs(peers) - 1)) atomicAdd(&s_hist[bin], (uint32_t)__popc(peers));
+        if (valid && lane == (uint32_t)(__ffs(peers) - 1)) {
+            if (bin < n_shared) atomicAdd(&s_hist[bin], (uint32_t)__popc(peers));
+            else atomicAdd(g_hist + bin, (unsigned long long)__popc(peers));
+        }
     }
     #pragma unroll
     for (int d = 16; d > 0; d >>= 1) local += __shfl_down_sync(0xffffffffu, local, d);
     if (lane == 0 && local) atomicAdd(&s_sum, local);
     __syncthreads();
-    for (uint32_t i = tid; i <= max_cov; i += COV_THREADS)
-        if (s_hist[i]) atomicAdd(hist + (size_t)k * (max_cov + 1) + i, (unsigned long long)s_hist[i]);
+    for (uint32_t i = tid; i < n_shared; i += COV_THREADS)
+        if (s_hist[i]) atomicAdd(g_hist + i, (unsigned long long)s_hist[i]);
     if (tid == 0 && s_sum) atomicAdd(cov_sum + k, s_sum);
 }
 

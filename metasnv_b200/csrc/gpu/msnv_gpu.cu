@@ -1213,8 +1213,10 @@ int msnv_get_timings(const msnv_ctx* ctx, msnv_timings* out)
 int msnv_cov_run(msnv_ctx* ctx, const msnv_cov_blocks* b, uint32_t max_cov, uint64_t* cov_sum, uint64_t* hist)
 {
     if (!ctx || !b || !cov_sum || !hist) return MSNV_E_ARG;
-    if (max_cov + 1 > (uint32_t)COV_MAX_BINS) return fail(ctx, MSNV_E_LIMIT, "msnv_cov_run: max_cov must be below %d", COV_MAX_BINS);
     const uint32_t K = b->n_contigs;
+    if (max_cov >= MSNV_COV_MAX_COUNTERS || (uint64_t)K * ((uint64_t)max_cov + 1) > MSNV_COV_MAX_COUNTERS)
+        return fail(ctx, MSNV_E_LIMIT, "msnv_cov_run: %u contigs x (max_cov %u + 1) histogram counters exceed the limit of %u",
+                    K, max_cov, (unsigned)MSNV_COV_MAX_COUNTERS);
     if (K == 0) return MSNV_OK;
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;

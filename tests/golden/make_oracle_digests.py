@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Regenerate tests/golden/oracle_digests.json: SHA-256 and line count of every oracle output that
-tests/test_gpu_parity.py compares the product with, on the same seeded inputs. Needs no GPU:
+tests/test_gpu_parity.py and tests/test_gpu_kernel_edges.py compare the product with, on the same seeded inputs. Needs no GPU:
     python tests/golden/make_oracle_digests.py
 The oracle is `mpileup_oracle | snpCall`, with the upstream snpCall build when oracle/_ref has it and the
 C restatement otherwise (the two agree on every vector of tests/golden/snpcall_vectors.json).
@@ -19,6 +19,7 @@ import __graft_entry__  # noqa: E402
 from metasnv_b200 import harness as H  # noqa: E402
 from metasnv_b200.paths import bin_path  # noqa: E402
 from cases import LIVE, WINDOWED, data_key, file_digest  # noqa: E402
+import edge_set  # noqa: E402
 
 EMPTY_SAM = "@HD\tVN:1.6\tSO:coordinate\n@SQ\tSN:ctgA\tLN:40\n@SQ\tSN:ctgB\tLN:40\n"
 
@@ -96,6 +97,16 @@ def main():
         lst = os.path.join(d, name + ".list")
         open(lst, "w").write("\n".join(bams) + "\n")
         oracle("hand/empty/" + name, d, all_samples=lst, c=1, t=1)
+
+    # tests/test_gpu_kernel_edges.py: the edge set under every option set it is called with
+    d = edge_set.write_edge_set(os.path.join(work, "edge"))
+    for samples, calls in (("all_samples", edge_set.EDGE_CALLS), ("narrow_samples", edge_set.NARROW_CALLS)):
+        for opts in calls:
+            prefix = os.path.join(work, "out")
+            rc, err = edge_set.run_oracle_calls(d, opts, prefix, samples)
+            assert rc == 0, err
+            for ext in (".called", ".indiv"):
+                out[edge_set.edge_key(opts, samples) + ext] = file_digest(prefix + ext)
 
     with open(os.path.join(HERE, "oracle_digests.json"), "w") as f:
         json.dump(out, f, indent=1, sort_keys=True)

@@ -6,6 +6,7 @@ pairing, the position-aligned segments with their zero padding."""
 import json
 import os
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -14,6 +15,10 @@ from conftest import GOLDEN
 from metasnv_b200 import harness as H
 from metasnv_b200.paths import bin_path
 from pileup_counts import ARRAYS, RAW_ARRAYS, check_layout, expand_raw, numpy_counts, oracle_counts
+
+sys.path.insert(0, GOLDEN)
+import edge_set  # noqa: E402
+from edge_set import write_edge_set  # noqa: E402
 
 
 def _decode(ref, lst, out, raw=False):
@@ -49,10 +54,17 @@ def _compare(lay, samples, pile_path):
     return total
 
 
-@pytest.mark.parametrize("preset,scale,samples", [("c1", 0.03, 8), ("c4", 0.002, 2), ("c5", 0.002, 4), ("c3", 0.0005, 6)])
+@pytest.mark.parametrize("preset,scale,samples", [("c1", 0.03, 8), ("c4", 0.002, 2), ("c5", 0.002, 4), ("c3", 0.0005, 6), ("edge", None, 310)])
 def test_decoder_batches_recount_to_the_oracle_text(preset, scale, samples, datasets, tmp_path):
-    data = datasets(preset, scale, samples)
+    """Synthetic sets, and the edge set of tests/golden/edge_set.py: 255 reads on one position in 270 samples, 250..260 reads
+    on one tile, 1200x from one BAM, overlapping mates whose corrected qualities land on 12 and 13, reads of 4096 bases
+    (one in 128 segments) at both ends of a contig whose length is not a multiple of 4."""
+    if preset == "edge":
+        data = write_edge_set(str(tmp_path / "edge"))
+    else:
+        data = datasets(preset, scale, samples)
     lay, batches = _decode(os.path.join(data, "ref.fa"), os.path.join(data, "all_samples"), str(tmp_path / "dump"))
+    assert len(batches) == samples
     pile = str(tmp_path / "pile.txt")
     with open(pile, "wb") as f:
         subprocess.run([H.oracle_bin("mpileup_oracle"), "mpileup", "-f", os.path.join(data, "ref.fa"), "-B", "-b",
@@ -62,6 +74,9 @@ def test_decoder_batches_recount_to_the_oracle_text(preset, scale, samples, data
         assert sum(m["dropped_by_cap"] for m in lay["samples"]) > 0, "the deep preset must exercise mpileup's depth cap"
     if preset == "c1":
         assert sum(m["pairs"] for m in lay["samples"]) > 0, "overlapping mates expected"
+    if preset == "edge":
+        assert max(m["max_span"] for m in lay["samples"]) == 4096 + 127 * 2, "the 128-segment read"
+        assert lay["samples"][edge_set.MATES_SAMPLE]["pairs"] == 12
 
 
 @pytest.mark.parametrize("sams,pile", [(("s1", "s2"), "expected.pileup"), (("s4_ops", "s1"), "expected_ops.pileup"),
@@ -110,3 +125,27 @@ def test_bam_shaped_batches_expand_to_the_aligned_layout(built, tmp_path):
                 assert np.array_equal(x[k], e[k]), k
             n_reads += e["pos"].size
     assert n_reads > 1000
+
+
+@pytest.mark.parametrize("what", ["bases", "segments"])
+def test_decoder_refuses_reads_above_the_length_limits(what, built, tmp_path):
+    """A read of 4097 bases, or of 129 aligned segments, is beyond MSNV_MAX_READ_BASES / MSNV_MAX_READ_SEGMENTS (the pileup
+    kernel's smallest stage is sized for one read at these limits): the decoder stops with an error naming the read instead
+    of handing it on. One read exactly at both limits (tests/golden/edge_set.py) decodes."""
+    if what == "bases":
+        cigar, n = "4097M", 4097
+    else:
+        cigar, n = "1M1D" * 128 + "1M", 129
+    sam = str(tmp_path / "big.sam")
+    open(sam, "w").write("@HD\tVN:1.6\tSO:coordinate\n@SQ\tSN:c\tLN:5000\n"
+                         "ok\t0\tc\t1\t60\t10M\t*\t0\t0\t%s\t%s\n" % ("A" * 10, "I" * 10) +
+                         "big\t0\tc\t5\t60\t%s\t*\t0\t0\t%s\t%s\n" % (cigar, "C" * n, "I" * n))
+    bam = str(tmp_path / "big.bam")
+    subprocess.run([bin_path("msnv_synth"), "--sam", sam, "--bam", bam], check=True)
+    open(str(tmp_path / "list"), "w").write(bam + "\n")
+    open(str(tmp_path / "ref.fa"), "w").write(">c\n" + "ACGT" * 1250 + "\n")
+    os.makedirs(str(tmp_path / "dump"))
+    r = subprocess.run([bin_path("msnv_decode_dump"), str(tmp_path / "ref.fa"), str(tmp_path / "list"), str(tmp_path / "dump")],
+                       capture_output=True, text=True)
+    assert r.returncode != 0
+    assert "read big exceeds the supported length (4096 bases / 128 aligned segments)" in r.stderr, r.stderr

@@ -40,15 +40,23 @@ def _expected_lines(h, ref, kind):
     return "".join(out)
 
 
-@pytest.mark.parametrize("S,L,seed,opts", [(3, 700, 1, (4, 4, 0.01)), (17, 1500, 2, (4, 4, 0.01)), (5, 512, 3, (10, 2, 0.3)), (1, 100, 4, (1, 1, 0.0))])
+# (c, t, p) with Poisson counts; (c, t, p, "placed"): every count is thr-1, thr or thr+1 (or small), so the integer test of
+# the wide (text-mode) items decides on both sides of thresholds that take the HI_THR form of call_kernel (t > 128)
+@pytest.mark.parametrize("S,L,seed,opts", [(3, 700, 1, (4, 4, 0.01)), (17, 1500, 2, (4, 4, 0.01)), (5, 512, 3, (10, 2, 0.3)), (1, 100, 4, (1, 1, 0.0))] +
+                         [(4, 600, 10 + t, (4, t, p, "placed")) for t in (128, 129, 255, 256) for p in (0.01, 1.0)])
 def test_call_counts_matches_snpcall_oracle(S, L, seed, opts, built, tmp_path):
     from metasnv_b200 import abi
     abi.load()
     TILE = abi.TILE
     rng = np.random.default_rng(seed)
-    cnt = rng.poisson(0.6, (L, S, 4)).astype(np.uint64) * (rng.random((L, S, 4)) < 0.3)
-    cnt[rng.random((L, S, 4)) < 0.01] = 40
-    match = rng.poisson(6, (L, S)).astype(np.uint16)
+    if len(opts) == 4:
+        thr = opts[1]
+        cnt = rng.choice(np.array([0, 0, 0, 1, 5, thr - 1, thr, thr + 1], np.uint64), (L, S, 4))
+        match = rng.choice(np.array([0, 3, thr - 1, thr, thr + 1], np.uint16), (L, S))
+    else:
+        cnt = rng.poisson(0.6, (L, S, 4)).astype(np.uint64) * (rng.random((L, S, 4)) < 0.3)
+        cnt[rng.random((L, S, 4)) < 0.01] = 40
+        match = rng.poisson(6, (L, S)).astype(np.uint16)
     ref = "".join(rng.choice(list("ACGTacgtNnR"), L))
     P = (L + TILE - 1) // TILE * TILE
     nt = P // TILE
@@ -60,7 +68,7 @@ def test_call_counts_matches_snpcall_oracle(S, L, seed, opts, built, tmp_path):
         t, o = divmod(i, TILE)
         acgt[t, :, o] = cnt[i, :, 0] | (cnt[i, :, 1] << np.uint64(16)) | (cnt[i, :, 2] << np.uint64(32)) | (cnt[i, :, 3] << np.uint64(48))
         mt[t, :, o] = match[i]
-    c, t_, p = opts
+    c, t_, p = opts[:3]
     with abi.Context(0) as ctx:
         h = ctx.call_counts(S, refb, acgt, mt, c, t_, p)
     assert np.all(np.diff(h.pos.astype(np.int64)) > 0)                    # ascending, no duplicates
@@ -70,24 +78,38 @@ def test_call_counts_matches_snpcall_oracle(S, L, seed, opts, built, tmp_path):
     assert r.returncode == 0
     assert _expected_lines(h, ref, "pop") == r.stdout.decode()
     assert _expected_lines(h, ref, "ind") == open(ind).read()
+    if len(opts) == 4:
+        assert r.stdout if p < 1.0 else open(ind).read()          # p = 1.0: the individual test decides
 
 
-@pytest.mark.parametrize("seed,max_cov", [(1, 10), (2, 30), (3, 1)])
+@pytest.mark.parametrize("seed,max_cov", [(1, 10), (2, 30), (3, 1), (4, 1023), (5, 1024), (6, 5000)])
 def test_cov_run_matches_numpy(seed, max_cov, built):
+    """Random blocks, plus: one position under 10 000 blocks (coverage values above the 1024 bins held in shared memory),
+    blocks that end exactly on a 4096-position chunk boundary, start on one, or cross several chunks, and contigs without
+    blocks between contigs with blocks."""
     from metasnv_b200 import abi
     rng = np.random.default_rng(seed)
-    lens = np.array([1, 5, 4095, 4096, 4097, 20000, 123457], np.uint32)
+    lens = np.array([1, 5, 4095, 4096, 4097, 20000, 123457, 9000, 7, 50000], np.uint32)
     begs, ends, off = [], [], [0]
-    for ln in lens:
+    for k, ln in enumerate(lens):
         n = int(rng.integers(0, 400)) if ln > 10 else 2
+        if k in (7, 8):
+            n = 0
         b = np.sort(rng.integers(0, max(1, ln - 1), n)).astype(np.uint32)
         e = np.minimum(b + rng.integers(1, 9000 if ln > 10000 else 150, n).astype(np.uint32), ln - 1).astype(np.uint32)
+        if k == 5:                                    # 10 000 blocks over position 8192 (a chunk boundary), coverage ramps 0 -> 10 000
+            b = np.concatenate([b, 8000 + np.arange(10000, dtype=np.uint32) % 193])
+            e = np.concatenate([e, 8193 + np.arange(10000, dtype=np.uint32) % 211])
+        if k == 9:                                    # ending on, starting on and crossing 4096-position chunks
+            b = np.concatenate([b, np.array([100, 4096, 4095, 8191, 0, 12288, 5000, 40960 - 7], np.uint32)])
+            e = np.concatenate([e, np.array([4096, 8192, 4097, 8192, 49999, 40960, 45000, 40960], np.uint32)])
         keep = e > b
         begs.append(b[keep]); ends.append(e[keep]); off.append(off[-1] + int(keep.sum()))
     beg = np.concatenate(begs) if off[-1] else np.zeros(0, np.uint32)
     end = np.concatenate(ends) if off[-1] else np.zeros(0, np.uint32)
     with abi.Context(0) as ctx:
         cov_sum, hist = ctx.cov_run(lens, np.array(off, np.uint64), beg, end, max_cov)
+    top = 0
     for k, ln in enumerate(lens):
         d = np.zeros(int(ln) + 1, np.int64)
         np.add.at(d, begs[k], 1)
@@ -97,6 +119,26 @@ def test_cov_run_matches_numpy(seed, max_cov, built):
         want = np.bincount(np.minimum(cov, max_cov), minlength=max_cov + 1)
         assert np.array_equal(hist[k], want.astype(np.uint64)), k
         assert hist[k].sum() == ln
+        top = max(top, int(cov.max()) if ln else 0)
+    assert top >= 10000
+
+
+def test_cov_run_refuses_histograms_above_the_limit(built):
+    """max_cov = 0xFFFFFFFF (where max_cov + 1 wraps to 0 in 32 bits) and histograms beyond MSNV_COV_MAX_COUNTERS are refused
+    with MSNV_E_LIMIT before anything is launched; the context stays usable."""
+    import ctypes as C
+    from metasnv_b200 import abi
+    lens = np.array([5000, 7000], np.uint32)
+    off = np.array([0, 1, 1], np.uint64)
+    beg, end = np.array([10], np.uint32), np.array([20], np.uint32)
+    b = abi.CovBlocks(2, abi._ptr(lens), abi._ptr(off), abi._ptr(beg), abi._ptr(end))
+    cov_sum, hist = np.zeros(2, np.uint64), np.zeros(16, np.uint64)
+    with abi.Context(0) as ctx:
+        for max_cov in (0xFFFFFFFF, 1 << 27, (1 << 26)):
+            assert ctx.lib.msnv_cov_run(ctx.h, C.byref(b), max_cov, abi._ptr(cov_sum), abi._ptr(hist)) == -4, max_cov     # MSNV_E_LIMIT
+            assert "exceed the limit" in ctx.lib.msnv_last_error(ctx.h).decode()
+        s, h = ctx.cov_run(lens, off, beg, end, 3)
+    assert s.tolist() == [10, 0] and h[0].tolist() == [4990, 10, 0, 0] and h[1].tolist() == [7000, 0, 0, 0]
 
 
 def _called_positions(path, offsets):
