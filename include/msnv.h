@@ -34,9 +34,12 @@ extern "C" {
 #ifndef MSNV_TILE
 #define MSNV_TILE 1024
 #endif
-/* Limits of the tiled pileup kernel (longer reads are rejected with MSNV_E_LIMIT). */
+/* Limits of the tiled pileup kernel (longer reads are rejected with MSNV_E_LIMIT). The reference span of a read (pos to
+ * its last covered position, deletions and skips included) bounds how far back the index looks for a tile's reads: every
+ * read starting within the span in front of a tile is a candidate of the tile. */
 #define MSNV_MAX_READ_BASES 4096
 #define MSNV_MAX_READ_SEGMENTS 128
+#define MSNV_MAX_READ_SPAN (8 * MSNV_MAX_READ_BASES)
 
 typedef enum {
     MSNV_OK = 0,

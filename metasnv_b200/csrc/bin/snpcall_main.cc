@@ -368,7 +368,7 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
     const HitWriter::Locator locate = HitWriter::shard_locator(ctgs, ref.data());
 
     double t_add = 0, t_wait_upload = 0, t_run = 0, t_format = 0, t_decode_wait = 0;
-    uint64_t h2d_bytes = 0, pageable_bytes = 0, n_hits_total = 0, items_total = 0;
+    uint64_t h2d_bytes = 0, pageable_bytes = 0, n_hits_total = 0, items_total = 0, ranges_total = 0;
     msnv_timings tm_sum; memset(&tm_sum, 0, sizeof tm_sum);
     bool masked = false;
     int64_t first_col = -1;
@@ -437,6 +437,7 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
         msnv_timings tm; msnv_get_timings(ctx, &tm);
         tm_sum.ms_index += tm.ms_index; tm_sum.ms_pileup += tm.ms_pileup; tm_sum.ms_call += tm.ms_call; tm_sum.ms_compact += tm.ms_compact;
         tm_sum.ms_gather += tm.ms_gather; tm_sum.kernel_launches += tm.kernel_launches; items_total += tm.n_items;
+        ranges_total += tm.n_ranges;            // ranges of tiles the tile budget cut this window into
 
         // test hook: per-sample, per-position A,C,G,T,N counts of the whole shard (msnv_shard_counts)
         if (dump) {
@@ -493,14 +494,14 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
                     "\"h2d_s\": %.6f, \"h2d_not_hidden_s\": %.6f, \"waiting_for_decode_s\": %.6f, "
                     "\"gpu_run_wall_s\": %.6f, \"format_s\": %.6f, \"total_s\": %.6f, "
                     "\"ms_index\": %.4f, \"ms_pileup\": %.4f, \"ms_call\": %.4f, \"ms_compact\": %.4f, \"ms_gather\": %.4f, "
-                    "\"items\": %llu, \"launches\": %u}\n",
+                    "\"items\": %llu, \"launches\": %u, \"ranges\": %llu}\n",
                     dev, S, layout.n_positions, n_windows, n_indexed, (unsigned long long)tot.records, (unsigned long long)tot.accepted,
                     (unsigned long long)tot.aligned_bases, (unsigned long long)tot.pairs, (unsigned long long)tot.dropped_by_cap,
                     (unsigned long long)bam_bytes_total, (unsigned long long)tot.compressed_bytes, (unsigned long long)h2d_bytes,
                     (unsigned long long)pageable_bytes, (unsigned long long)n_hits_total, raw_mode ? 1 : 0, n_threads * inflate_threads,
                     t_dec1 - t_dec0, tot.seconds, tot.inflate_seconds, t_add, t_wait_upload, t_decode_wait, t_run, t_format, t_end - t_start,
                     tm_sum.ms_index, tm_sum.ms_pileup, tm_sum.ms_call, tm_sum.ms_compact, tm_sum.ms_gather, (unsigned long long)items_total,
-                    tm_sum.kernel_launches);
+                    tm_sum.kernel_launches, (unsigned long long)ranges_total);
             fclose(f);
         }
     }

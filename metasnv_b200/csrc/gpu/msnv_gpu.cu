@@ -745,7 +745,7 @@ int msnv_window_add_sample(msnv_ctx* ctx, uint32_t slot, uint32_t sample, const 
     if (sample >= ctx->S) return fail(ctx, MSNV_E_ARG, "msnv_window_add_sample: sample %u out of range", sample);
     if (w.h_samples[sample].n_reads) return fail(ctx, MSNV_E_STATE, "msnv_window_add_sample: sample %u added twice", sample);
     if (r->n_reads == 0) return MSNV_OK;
-    if (r->max_span > 8u * MSNV_MAX_READ_BASES) return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit", sample, r->max_span);
+    if (r->max_span > (uint32_t)MSNV_MAX_READ_SPAN) return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit of %u", sample, r->max_span, (uint32_t)MSNV_MAX_READ_SPAN);
     CU(cudaSetDevice(ctx->device));
     const size_t n = r->n_reads, n1 = n + 1;
     const size_t n_seg = r->seg_off[n] - r->seg_off[0], n_q4 = r->q4_off[n] - r->q4_off[0];
@@ -803,7 +803,7 @@ int msnv_window_add_sample_raw(msnv_ctx* ctx, uint32_t slot, uint32_t sample, co
     if (sample >= ctx->S) return fail(ctx, MSNV_E_ARG, "msnv_window_add_sample_raw: sample %u out of range", sample);
     if (w.h_samples[sample].n_reads) return fail(ctx, MSNV_E_STATE, "msnv_window_add_sample_raw: sample %u added twice", sample);
     if (r->n_reads == 0) return MSNV_OK;
-    if (r->max_span > 8u * MSNV_MAX_READ_BASES) return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit", sample, r->max_span);
+    if (r->max_span > (uint32_t)MSNV_MAX_READ_SPAN) return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit of %u", sample, r->max_span, (uint32_t)MSNV_MAX_READ_SPAN);
     CU(cudaSetDevice(ctx->device));
     const size_t n = r->n_reads, n1 = n + 1;
     if (r->seg_off[0] != 0 || r->q4_off[0] != 0 || r->raw_off[0] != 0) return fail(ctx, MSNV_E_ARG, "sample %u: seg_off / q4_off / raw_off must start at 0", sample);

@@ -367,6 +367,11 @@ bool SampleDecoder::window_impl(uint32_t pos_lo, uint32_t pos_hi, const SampleRe
                   " bases / " + std::to_string(MSNV_MAX_READ_SEGMENTS) + " aligned segments)";
             return false;
         }
+        if (rlen > MSNV_MAX_READ_SPAN) {
+            err = bam_path + ": read " + r.qname + " spans " + std::to_string(rlen) + " reference positions, more than the supported " +
+                  std::to_string(MSNV_MAX_READ_SPAN) + " (deletions and skips included)";
+            return false;
+        }
         const ShardLayout::Ctg& ctg = layout.ctgs[slot];
         // ---- a read of a later window: keep it for the next call (its bytes live in the reader's buffer only until the next record)
         if ((uint64_t)ctg.offset + (uint32_t)c.pos >= pos_hi) {

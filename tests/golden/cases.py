@@ -27,6 +27,17 @@ FILTER_OPTS = {
 }
 
 
+def oracle_mpileup(ref, samples, out, bed=None):
+    """The oracle's mpileup text of the BAMs listed in `samples` (`mpileup_oracle mpileup -f ref [-l bed] -B -b samples`),
+    written to out; returns out."""
+    import subprocess
+    from metasnv_b200 import harness as H
+    with open(out, "wb") as f:
+        subprocess.run([H.oracle_bin("mpileup_oracle"), "mpileup", "-f", ref] + (["-l", bed] if bed else []) + ["-B", "-b", samples],
+                       stdout=f, check=True)
+    return out
+
+
 def file_digest(path):
     data = open(path, "rb").read()
     return {"sha256": hashlib.sha256(data).hexdigest(), "lines": data.count(b"\n")}

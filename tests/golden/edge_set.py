@@ -208,13 +208,10 @@ def stack_intervals():
 def oracle_pileup(d, bed=False, samples="all_samples"):
     """The oracle's mpileup text of the set in d (or of its stacks.bed; samples: all_samples or narrow_samples), written
     once into d."""
-    from metasnv_b200 import harness as H
+    from cases import oracle_mpileup
     path = os.path.join(d, "pile_%s%s.txt" % (samples, "_bed" if bed else ""))
     if not os.path.exists(path):
-        with open(path, "wb") as f:
-            subprocess.run([H.oracle_bin("mpileup_oracle"), "mpileup", "-f", os.path.join(d, "ref.fa")] +
-                           (["-l", os.path.join(d, "stacks.bed")] if bed else []) + ["-B", "-b", os.path.join(d, samples)],
-                           stdout=f, check=True)
+        oracle_mpileup(os.path.join(d, "ref.fa"), os.path.join(d, samples), path, os.path.join(d, "stacks.bed") if bed else None)
     return path
 
 

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Regenerate tests/golden/oracle_digests.json: SHA-256 and line count of every oracle output that
-tests/test_gpu_parity.py and tests/test_gpu_kernel_edges.py compare the product with, on the same seeded inputs. Needs no GPU:
+tests/test_gpu_parity.py, tests/test_gpu_kernel_edges.py and tests/test_gpu_long_spans.py compare the product with, on the same seeded inputs. Needs no GPU:
     python tests/golden/make_oracle_digests.py
 The oracle is `mpileup_oracle | snpCall`, with the upstream snpCall build when oracle/_ref has it and the
 C restatement otherwise (the two agree on every vector of tests/golden/snpcall_vectors.json).
@@ -20,6 +20,7 @@ from metasnv_b200 import harness as H  # noqa: E402
 from metasnv_b200.paths import bin_path  # noqa: E402
 from cases import LIVE, WINDOWED, data_key, file_digest  # noqa: E402
 import edge_set  # noqa: E402
+import span_set  # noqa: E402
 
 EMPTY_SAM = "@HD\tVN:1.6\tSO:coordinate\n@SQ\tSN:ctgA\tLN:40\n@SQ\tSN:ctgB\tLN:40\n"
 
@@ -107,6 +108,15 @@ def main():
             assert rc == 0, err
             for ext in (".called", ".indiv"):
                 out[edge_set.edge_key(opts, samples) + ext] = file_digest(prefix + ext)
+
+    # tests/test_gpu_long_spans.py: the span set under every option set it is called with
+    d = span_set.write_span_set(os.path.join(work, "span"))
+    for opts in span_set.SPAN_CALLS:
+        prefix = os.path.join(work, "out")
+        rc, err = span_set.run_oracle_calls(d, opts, prefix)
+        assert rc == 0, err
+        for ext in (".called", ".indiv"):
+            out[span_set.span_key(opts) + ext] = file_digest(prefix + ext)
 
     with open(os.path.join(HERE, "oracle_digests.json"), "w") as f:
         json.dump(out, f, indent=1, sort_keys=True)

@@ -8,7 +8,12 @@ numpy_counts()    recounts one sample from the structure-of-arrays batch of incl
                   both mates of a pair cover are corrected by htslib's tweak_overlap_quality (Annex A.2): equal bases ->
                   the earlier read gets min(qa+qb, 127... htslib: 200) and the later one 0; different bases -> the better one keeps
                   int(0.8*q), the other 0, ties go to the earlier read.
+decode_dump()     runs bin/msnv_decode_dump and loads the batches it writes.
 """
+import json
+import os
+import subprocess
+
 import numpy as np
 
 ARRAYS = (("pos", np.int32), ("seg_off", np.uint32), ("q4_off", np.uint32), ("mate", np.int32),
@@ -125,6 +130,17 @@ def numpy_counts(e, P):
     return flat.reshape(P, 5).astype(np.uint16)
 
 
+def first_difference(want, got, layout):
+    """Description of where [S][P][5] counts `got` first differ from `want` ('' if equal); layout: [(name, offset, len)]."""
+    bad = np.argwhere(want != got)
+    if not bad.size:
+        return ""
+    s, p, c = bad[0]
+    ctg = max((o, n) for n, o, _ in layout if o <= p)
+    return ("%d differing counts; first: sample %d, %s:%d (shard position %d), channel %s: oracle %d, GPU %d"
+            % (len(bad), s, ctg[1], p - ctg[0] + 1, p, "ACGTN"[c], want[s, p, c], got[s, p, c]))
+
+
 RAW_ARRAYS = (("raw_pos", np.int32), ("raw_mate", np.int32), ("raw_seg_off", np.uint32), ("raw_q4_off", np.uint32),
               ("raw_off", np.uint32), ("raw_n_cigar", np.uint16), ("raw_l_seq", np.uint16), ("raw", np.uint32))
 
@@ -168,3 +184,42 @@ def expand_raw(r):
         assert k == int(r["raw_seg_off"][i + 1]) and Q == int(r["raw_q4_off"][i + 1]) and qy <= ls
     return {"pos": r["raw_pos"], "mate": r["raw_mate"], "seg_off": r["raw_seg_off"], "q4_off": r["raw_q4_off"],
             "seg_pos": seg_pos, "seg_len": seg_len, "seq2": seq2, "qual": qual}
+
+
+def _load_batch(out, prefix, meta, raw):
+    e = {k: np.fromfile(os.path.join(out, "%s%s.bin" % (prefix, k)), dt) for k, dt in ARRAYS}
+    e["max_span"] = meta["max_span"]
+    if raw:
+        for k, dt in RAW_ARRAYS:
+            e[k] = np.fromfile(os.path.join(out, "%s%s.bin" % (prefix, k)), dt)
+    assert e["pos"].size == meta["n_reads"] and e["seg_pos"].size == meta["n_segs"] and e["seq2"].size == meta["n_q4"]
+    return e
+
+
+def decode_dump(ref, lst, out, raw=False, windows=0):
+    """Run msnv_decode_dump: (layout.json, [the whole shard's batch per sample]); with windows=N also
+    [per window: [its batch per sample]] (the decoder's windows, carried reads included)."""
+    from metasnv_b200.paths import bin_path
+    os.makedirs(out, exist_ok=True)
+    env = dict(os.environ)
+    if raw:
+        env["MSNV_DUMP_RAW"] = "1"
+    if windows:
+        env["MSNV_DUMP_WINDOWS"] = str(windows)
+    r = subprocess.run([bin_path("msnv_decode_dump"), ref, lst, out], capture_output=True, text=True, env=env)
+    assert r.returncode == 0, r.stderr
+    lay = json.load(open(os.path.join(out, "layout.json")))
+    samples = [_load_batch(out, "s%d." % s, meta, raw) for s, meta in enumerate(lay["samples"])]
+    if not windows:
+        return lay, samples
+    wins = []
+    for k, w in enumerate(lay["windows"]):
+        batches = []
+        for s, meta in enumerate(w["samples"]):
+            e = _load_batch(out, "w%d.s%d." % (k, s), meta, raw)
+            if raw:
+                assert e["raw_pos"].size == meta["raw_n_reads"]
+                e["raw_max_span"] = meta["raw_max_span"]
+            batches.append(e)
+        wins.append(batches)
+    return lay, samples, wins

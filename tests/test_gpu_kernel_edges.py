@@ -17,7 +17,7 @@ import pytest
 from conftest import GOLDEN
 from metasnv_b200 import harness as H
 from metasnv_b200.paths import bin_path
-from pileup_counts import oracle_counts
+from pileup_counts import first_difference, oracle_counts
 
 sys.path.insert(0, GOLDEN)
 import edge_set as E  # noqa: E402
@@ -52,16 +52,6 @@ class Edge:
 @pytest.fixture(scope="module")
 def edge(built, tmp_path_factory):
     return Edge(E.write_edge_set(str(tmp_path_factory.mktemp("edge") / "set")))
-
-
-def _first_difference(want, got, layout):
-    bad = np.argwhere(want != got)
-    if not bad.size:
-        return ""
-    s, p, c = bad[0]
-    ctg = max((o, n) for n, o, _ in layout if o <= p)
-    return ("%d differing counts; first: sample %d, %s:%d (shard position %d), channel %s: oracle %d, GPU %d"
-            % (len(bad), s, ctg[1], p - ctg[0] + 1, p, "ACGTN"[c], want[s, p, c], got[s, p, c]))
 
 
 def _same(a, b):
@@ -99,7 +89,7 @@ def test_edge_counts_match_oracle_text(env, edge, tmp_path):
         assert want[list(E.SWEEP), deep + E.X2, 0].tolist() == list(range(250, 261))
         assert want[E.DEEP_COV_SAMPLE, deep + E.DEEP_COV_AT:deep + E.DEEP_COV_AT + 200, :4].sum(axis=1).max() == 1200
         edge.want_counts = want
-    d = _first_difference(edge.want_counts, got, layout)
+    d = first_difference(edge.want_counts, got, layout)
     assert not d, d
 
 
@@ -141,7 +131,7 @@ def test_shard_whose_largest_items_hold_255_reads(opts, edge, tmp_path):
         got, layout, _ = _dump_counts(edge, str(tmp_path / "counts"), {}, "narrow_samples")
         want = oracle_counts(E.oracle_pileup(edge.dir, samples="narrow_samples"), got.shape[0], layout, got.shape[1])
         assert (want.sum(axis=2) == 255).any() and not (want.sum(axis=2) > 255).any()
-        d = _first_difference(want, got, layout)
+        d = first_difference(want, got, layout)
         assert not d, d
     o = edge.oracle_calls(opts, "narrow_samples")
     g = str(tmp_path / "gpu")
