@@ -54,43 +54,16 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes)
 {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-// hint_ns > 0: the hardware may park the thread for up to that long between polls (fewer issue slots spent spinning)
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, uint32_t hint_ns = 0)
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity)
 {
     uint32_t done;
-    if (hint_ns) {
-        do {
-            asm volatile(
-                "{\n\t.reg .pred p;\n\t"
-                "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-                "selp.u32 %0, 1, 0, p;\n\t}"
-                : "=r"(done) : "r"(smem_u32(bar)), "r"(parity), "r"(hint_ns) : "memory");
-        } while (!done);
-    } else {
-        do {
-            asm volatile(
-                "{\n\t.reg .pred p;\n\t"
-                "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                "selp.u32 %0, 1, 0, p;\n\t}"
-                : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        } while (!done);
-    }
-}
-// the producer's wait for a free stage: it is long (the consumers work on an item for microseconds) and a warp that polls
-// takes issue slots from them (a tenth of all executed instructions in the profile), so sleep between polls
-__device__ __forceinline__ void mbar_wait_parked(uint64_t* bar, uint32_t parity, uint32_t sleep_ns)
-{
-    if (!sleep_ns) { mbar_wait(bar, parity); return; }
-    while (true) {
-        uint32_t done;
+    do {
         asm volatile(
             "{\n\t.reg .pred p;\n\t"
-            "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
             "selp.u32 %0, 1, 0, p;\n\t}"
             : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (done) break;
-        __nanosleep(sleep_ns);
-    }
+    } while (!done);
 }
 // global -> shared bulk copy (TMA, SASS UBLKCP); dst/src 16-byte aligned, bytes a multiple of 16
 __device__ __forceinline__ void tma_load_1d(void* dst, const void* src, uint32_t bytes, uint64_t* bar)
@@ -564,10 +537,9 @@ constexpr uint32_t CHUNK_SEGS_MIN = MSNV_MAX_READ_SEGMENTS;
 constexpr uint32_t CHUNK_FIRST = 1u, CHUNK_LAST = 2u, CHUNK_WIDE = 4u, CHUNK_STOP = 8u, CHUNK_FIX = 16u /* the sample has mate verdicts */;
 
 // limits of one staged chunk, chosen per launch from the shape of the shard
-struct PileupShape { uint32_t max_reads, max_segs, chunk_q4, has_fix /* some sample carries mate verdicts */, wait_hint_ns, ablate /* measurement only: phases to skip */,
+struct PileupShape { uint32_t max_reads, max_segs, chunk_q4, has_fix /* some sample carries mate verdicts */,
                      gather /* stages carry the gather kernel's segment records and ranges instead of the scatter kernel's tags */,
-                     stages /* of the ring, 2 .. PL_STAGES_MAX */,
-                     producer_hint_ns /* the producer warp sleeps this long between polls for a free stage (0: it spins) */; };
+                     stages /* of the ring, 2 .. PL_STAGES_MAX */; };
 
 struct ChunkHdr { uint32_t m, nq4, q4_0, sg_0, nseg, c0, item, sample, tile, flags, pad[6]; };
 static_assert(sizeof(ChunkHdr) == 64, "header is one 64-byte block");
@@ -619,6 +591,7 @@ __device__ __forceinline__ uint4 lds_v4(uint32_t a)
     return v;
 }
 __device__ __forceinline__ void red_shared_add(uint32_t a, uint32_t v) { asm volatile("red.shared.add.u32 [%0], %1;" :: "r"(a), "r"(v) : "memory"); }
+__device__ __forceinline__ uint32_t and3(uint32_t a, uint32_t b, uint32_t c) { uint32_t r; asm("lop3.b32 %0, %1, %2, %3, 0x80;" : "=r"(r) : "r"(a), "r"(b), "r"(c)); return r; }
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar)
 {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -656,30 +629,21 @@ __device__ __forceinline__ ChunkCopies chunk_copies(const SrcPtrs& p, uint32_t c
     c.src[6] = p.qual + 4u * (size_t)(q4_0 - dq); c.bytes[6] = up_to(dq + nq4, 4) * 4u;
     return c;
 }
-__device__ __forceinline__ void prefetch_l2(const void* src, uint32_t bytes)
-{
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-}
-// bring a chunk's source bytes into L2 ahead of the copy that stages them. Measured (profiles/r02_pileup_ablations.txt): it
-// buys nothing - the consumers, not the refill, bound a CTA's rate - and costs DRAM reads (lines evicted before their copy
-// are fetched twice), so it is OFF; MSNV_ABLATE bit 64 switches it on for measurements.
-__device__ __forceinline__ void prefetch_chunk(const SrcPtrs& p, uint32_t c0, uint32_t m, uint32_t q4_0, uint32_t nq4, uint32_t sg_0, uint32_t nseg)
-{
-    const ChunkCopies c = chunk_copies(p, c0, m, q4_0, nq4, sg_0, nseg);
-    #pragma unroll
-    for (int i = 2; i < 7; ++i) if (c.bytes[i]) prefetch_l2(c.src[i], c.bytes[i]);      // the offsets were touched when the item was sized
-}
 
-// ---- producer: one chunk into the next stage of the ring (whole warp waits; lane `issuer` writes the header and issues)
-__device__ __forceinline__ void pileup_issue_chunk(uint8_t* smem, const PileupSmem& L, const PileupShape& sh, uint32_t& chunk_no, uint32_t issuer, const SrcPtrs& src,
+// ---- producer: one chunk of sample `sd` into the next stage of the ring (whole warp waits; lane `issuer` reads the sample's
+// array pointers, writes the header and issues: no lane holds seven pointers across the producer's loops)
+__device__ __forceinline__ void pileup_issue_chunk(uint8_t* smem, const PileupSmem& L, const PileupShape& sh, uint32_t& chunk_no, uint32_t issuer, const SampleDev* __restrict__ sd,
                                                    const uint8_t* __restrict__ expect, uint32_t item, uint32_t sample, uint32_t tile, uint32_t c0,
                                                    uint32_t m, uint32_t q4_0, uint32_t nq4, uint32_t sg_0, uint32_t nseg, uint32_t flags)
 {
     uint64_t* full = (uint64_t*)(smem + L.bar);
     uint64_t* empty = full + sh.stages;
     const uint32_t s = chunk_no % sh.stages, ph = (chunk_no / sh.stages) & 1u;
-    mbar_wait_parked(empty + s, ph ^ 1u, sh.producer_hint_ns);
+    // the producer spins for a free stage: sleeping 200 or 1000 ns between polls measured the same, 3000 ns slower
+    // (profiles/r02_pileup_ablations.txt, D)
+    mbar_wait(empty + s, ph ^ 1u);
     if ((threadIdx.x & 31) == issuer) {
+        const SrcPtrs src = load_src_ptrs(sd);
         uint8_t* stage = smem + L.stage0 + s * L.stage_bytes;
         ChunkHdr* h = (ChunkHdr*)(stage + L.o_hdr);
         h->m = m; h->nq4 = nq4; h->q4_0 = q4_0; h->sg_0 = sg_0; h->nseg = nseg; h->c0 = c0;
@@ -699,8 +663,6 @@ __device__ __forceinline__ void pileup_issue_chunk(uint8_t* smem, const PileupSm
     ++chunk_no;
 }
 
-constexpr uint32_t PREFETCH_AHEAD = 4;       // items between a chunk's L2 prefetch and its copy
-
 __device__ __forceinline__ void pileup_producer(uint8_t* smem, const PileupSmem& L, const PileupShape sh, const SampleDev* __restrict__ samples,
                                                 const Item* __restrict__ items, uint32_t n_items, const uint8_t* __restrict__ expect,
                                                 int* __restrict__ err_flag)
@@ -708,26 +670,23 @@ __device__ __forceinline__ void pileup_producer(uint8_t* smem, const PileupSmem&
     const uint32_t lane = threadIdx.x & 31, G = gridDim.x;
     uint32_t chunk_no = 0;
     for (uint64_t base = blockIdx.x; base < n_items; base += 32ull * G) {
-        // ---- 32 upcoming items of this CTA, one per lane: item record, source arrays and the offsets that size the item
+        // ---- 32 upcoming items of this CTA, one per lane: item record and the offsets that size the item
         const uint64_t mine = base + (uint64_t)lane * G;
         uint4 it = make_uint4(0u, 0u, 0u, 0u);
         uint32_t q_lo = 0, q_hi = 0, g_lo = 0, g_hi = 0;
-        SrcPtrs src{};
         bool whole = false;                  // the item fits one stage
         if (mine < n_items) {
             it = __ldg(reinterpret_cast<const uint4*>(items) + mine);
-            src = load_src_ptrs(samples + it.x);
+            const SrcPtrs src = load_src_ptrs(samples + it.x);
             q_lo = __ldg(src.q4_off + it.z); q_hi = __ldg(src.q4_off + it.w);
             g_lo = __ldg(src.seg_off + it.z); g_hi = __ldg(src.seg_off + it.w);
             whole = it.w - it.z <= sh.max_reads && q_hi - q_lo <= sh.chunk_q4 && g_hi - g_lo <= sh.max_segs;
-            if (whole && lane < PREFETCH_AHEAD && (sh.ablate & 64u)) prefetch_chunk(src, it.z, it.w - it.z, q_lo, q_hi - q_lo, g_lo, g_hi - g_lo);
         }
         for (uint32_t k = 0; k < 32u; ++k) {
             const uint64_t idx = base + (uint64_t)k * G;
             if (idx >= n_items) break;
-            if (lane == k + PREFETCH_AHEAD && whole && (sh.ablate & 64u)) prefetch_chunk(src, it.z, it.w - it.z, q_lo, q_hi - q_lo, g_lo, g_hi - g_lo);
             if (__shfl_sync(0xffffffffu, (int)whole, k)) {                   // the lane that owns the item issues it from its own registers
-                pileup_issue_chunk(smem, L, sh, chunk_no, k, src, expect, (uint32_t)mine, it.x, it.y, it.z, it.w - it.z, q_lo, q_hi - q_lo, g_lo,
+                pileup_issue_chunk(smem, L, sh, chunk_no, k, samples + it.x, expect, (uint32_t)mine, it.x, it.y, it.z, it.w - it.z, q_lo, q_hi - q_lo, g_lo,
                                    g_hi - g_lo, CHUNK_FIRST | CHUNK_LAST | (item_is_wide(it.z, it.w) ? CHUNK_WIDE : 0u));
                 continue;
             }
@@ -735,8 +694,7 @@ __device__ __forceinline__ void pileup_producer(uint8_t* smem, const PileupSmem&
             const uint32_t sample = __shfl_sync(0xffffffffu, it.x, k), tile = __shfl_sync(0xffffffffu, it.y, k);
             const uint32_t r_lo = __shfl_sync(0xffffffffu, it.z, k), r_hi = __shfl_sync(0xffffffffu, it.w, k);
             const uint32_t ql = __shfl_sync(0xffffffffu, q_lo, k), gl = __shfl_sync(0xffffffffu, g_lo, k);
-            const SrcPtrs sp = load_src_ptrs(samples + sample);
-            const uint32_t* q4p = sp.q4_off; const uint32_t* sgp = sp.seg_off;
+            const uint32_t* q4p = samples[sample].q4_off; const uint32_t* sgp = samples[sample].seg_off;
             const uint32_t wide = item_is_wide(r_lo, r_hi) ? CHUNK_WIDE : 0u;
             uint32_t c0 = r_lo, qc = ql, gc = gl;
             while (c0 < r_hi) {
@@ -752,13 +710,11 @@ __device__ __forceinline__ void pileup_producer(uint8_t* smem, const PileupSmem&
                 const uint32_t n_ok = okmask == 0xffffffffu ? 32u : (uint32_t)__ffs((int)~okmask) - 1u;      // leading chunks that fit
                 if (n_ok) {
                     const uint32_t fl = (b_l == r_lo ? CHUNK_FIRST : 0u) | (e_l == r_hi ? CHUNK_LAST : 0u) | wide;
-                    if (lane < PREFETCH_AHEAD && lane < n_ok && e_l > b_l && (sh.ablate & 64u)) prefetch_chunk(sp, b_l, e_l - b_l, qb, qe - qb, gb, ge - gb);
                     uint32_t done_to = c0, done_q = qc, done_g = gc;
                     for (uint32_t kk = 0; kk < n_ok; ++kk) {
                         const uint32_t bk = __shfl_sync(0xffffffffu, b_l, kk), ek = __shfl_sync(0xffffffffu, e_l, kk);
                         if (ek == bk) break;                                             // past the end of the item
-                        if (lane == kk + PREFETCH_AHEAD && lane < n_ok && e_l > b_l && (sh.ablate & 64u)) prefetch_chunk(sp, b_l, e_l - b_l, qb, qe - qb, gb, ge - gb);
-                        pileup_issue_chunk(smem, L, sh, chunk_no, kk, sp, expect, (uint32_t)idx, sample, tile, b_l, e_l - b_l, qb, qe - qb, gb, ge - gb, fl);
+                        pileup_issue_chunk(smem, L, sh, chunk_no, kk, samples + sample, expect, (uint32_t)idx, sample, tile, b_l, e_l - b_l, qb, qe - qb, gb, ge - gb, fl);
                         done_to = ek; done_q = __shfl_sync(0xffffffffu, qe, kk); done_g = __shfl_sync(0xffffffffu, ge, kk);
                     }
                     c0 = done_to; qc = done_q; gc = done_g;
@@ -779,11 +735,11 @@ __device__ __forceinline__ void pileup_producer(uint8_t* smem, const PileupSmem&
                 const uint32_t first = c0 == r_lo ? CHUNK_FIRST : 0u;
                 if (m == 0) {                        // a single read over the documented limits: host validation failed
                     if (lane == 0) atomicExch(err_flag, 1);
-                    pileup_issue_chunk(smem, L, sh, chunk_no, 0u, sp, expect, (uint32_t)idx, sample, tile, c0, 0u, qc, 0u, gc, 0u, first | CHUNK_LAST | wide);
+                    pileup_issue_chunk(smem, L, sh, chunk_no, 0u, samples + sample, expect, (uint32_t)idx, sample, tile, c0, 0u, qc, 0u, gc, 0u, first | CHUNK_LAST | wide);
                     break;
                 }
                 const uint32_t qn = __ldg(q4p + c0 + m), gn = __ldg(sgp + c0 + m);
-                pileup_issue_chunk(smem, L, sh, chunk_no, 0u, sp, expect, (uint32_t)idx, sample, tile, c0, m, qc, qn - qc, gc, gn - gc,
+                pileup_issue_chunk(smem, L, sh, chunk_no, 0u, samples + sample, expect, (uint32_t)idx, sample, tile, c0, m, qc, qn - qc, gc, gn - gc,
                                    first | (c0 + m == r_hi ? CHUNK_LAST : 0u) | wide);
                 c0 += m; qc = qn; gc = gn;
             }
@@ -793,16 +749,97 @@ __device__ __forceinline__ void pileup_producer(uint8_t* smem, const PileupSmem&
     uint64_t* full = (uint64_t*)(smem + L.bar);
     uint64_t* empty = full + sh.stages;
     const uint32_t s = chunk_no % sh.stages, ph = (chunk_no / sh.stages) & 1u;
-    mbar_wait_parked(empty + s, ph ^ 1u, sh.producer_hint_ns);
+    mbar_wait(empty + s, ph ^ 1u);
     if (lane == 0) {
         ((ChunkHdr*)(smem + L.stage0 + s * L.stage_bytes + L.o_hdr))->flags = CHUNK_STOP;
         mbar_arrive(full + s);
     }
 }
 
+// ---- what both forms share
+// CTA start: the ring's barriers (a stage is free again after `empty_count` arrivals) and cleared count planes; then the
+// producer warp runs the producer. Returns true to the producer warp, which leaves the kernel.
+template <int CONSUMERS>
+__device__ __forceinline__ bool pileup_cta_start(uint8_t* smem, const PileupSmem& L, const PileupShape& sh, uint32_t empty_count,
+                                                 const SampleDev* __restrict__ samples, const Item* __restrict__ items, uint32_t n_items,
+                                                 const uint8_t* __restrict__ expect, int* __restrict__ err_flag)
+{
+    uint64_t* full = (uint64_t*)(smem + L.bar);
+    uint64_t* empty = full + sh.stages;
+    uint32_t* s_cnt = (uint32_t*)(smem + L.cnt);
+    if (threadIdx.x == 0) {
+        for (uint32_t s = 0; s < sh.stages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, empty_count); }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    for (uint32_t k = threadIdx.x; k < (uint32_t)(N_PLANES * TILE_QUADS); k += CONSUMERS + 32) s_cnt[k] = 0;
+    __syncthreads();
+    if (threadIdx.x < CONSUMERS) return false;
+    pileup_producer(smem, L, sh, samples, items, n_items, expect, err_flag);
+    return true;
+}
+
+// Wide items (more than 255 reads) are counted in 16-bit lanes held in registers, per plane and owned quad QPT * tid + k
+// (QPT = TILE_QUADS / CONSUMERS, 2 or 1): [0] = positions 0 and 2, [1] = positions 1 and 3. HAS_WIDE: the shard has such
+// items (deep coverage); without them one plane's worth is declared and never used.
+template <int CONSUMERS, bool HAS_WIDE> using WideAcc = uint32_t[HAS_WIDE ? N_PLANES : 1][TILE_QUADS / CONSUMERS][2];
+
+// this thread's words of the byte planes into its 16-bit lanes (a chunk stages at most 255 reads: no byte lane has
+// overflowed); the words are cleared
+template <int CONSUMERS, bool HAS_WIDE>
+__device__ __forceinline__ void wide_fold(WideAcc<CONSUMERS, HAS_WIDE>& acc, uint32_t* s_cnt, uint32_t tid)
+{
+    constexpr int QPT = TILE_QUADS / CONSUMERS;
+    #pragma unroll
+    for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
+        #pragma unroll
+        for (int k = 0; k < QPT; ++k) {
+            const uint32_t slot = c * TILE_QUADS + QPT * tid + k;
+            const uint32_t w = s_cnt[slot];
+            s_cnt[slot] = 0;
+            acc[c][k][0] += w & 0x00ff00ffu; acc[c][k][1] += (w >> 8) & 0x00ff00ffu;
+        }
+}
+
+// the item's 16-bit planes from this thread's lanes to its slot in HBM; the lanes are cleared
+template <int CONSUMERS, bool HAS_WIDE>
+__device__ __forceinline__ void wide_store(WideAcc<CONSUMERS, HAS_WIDE>& acc, uint8_t* slot, uint32_t tid)
+{
+    constexpr int QPT = TILE_QUADS / CONSUMERS;
+    uint2* dst = reinterpret_cast<uint2*>(slot);
+    #pragma unroll
+    for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
+        #pragma unroll
+        for (int k = 0; k < QPT; ++k) {
+            // 16-bit plane c, positions 4 * (QPT * tid + k) .. + 3
+            dst[c * (TILE / 4) + QPT * tid + k] = make_uint2((acc[c][k][0] & 0xffffu) | (acc[c][k][1] << 16), (acc[c][k][0] >> 16) | (acc[c][k][1] & 0xffff0000u));
+            acc[c][k][0] = acc[c][k][1] = 0;
+        }
+}
+
+// The pass test of one staged quad, on byte lanes (bit 0 of each): ok = the base counts (quality >= 13, A/C/G/T), nn = it
+// counts as N (it passes, but is not A/C/G/T). q: the four qualities, bit 7 of a lane set where the base is not A/C/G/T.
+// FIX (the sample carries mate verdicts): where the overlap rule spoke (low nibble of the verdict byte f) its verdict (high
+// nibble) replaces the quality test.
+template <bool FIX>
+__device__ __forceinline__ void quad_pass(uint32_t q, uint32_t f, uint32_t& ok, uint32_t& nn)
+{
+    if (!FIX) {
+        const uint32_t v = (q & 0x7f7f7f7fu) + 0x73737373u;                     // bit 7 of a lane: quality >= 13
+        asm("lop3.b32 %0, %1, %2, 0x80808080, 0x20;" : "=r"(ok) : "r"(v), "r"(q));    // v & ~q & 0x80808080: ... and A/C/G/T
+        ok >>= 7;
+        nn = and3(v, q, 0x80808080u) >> 7;
+    } else {
+        const uint32_t ovr = nibble_to_lanes(f), val = nibble_to_lanes(f >> 4);
+        const uint32_t qp = (((q & 0x7f7f7f7fu) + 0x73737373u) >> 7) & 0x01010101u;
+        const uint32_t pass = (qp & ~ovr) | (val & ovr);
+        const uint32_t fl = (q >> 7) & 0x01010101u;
+        ok = pass & ~fl;
+        nn = pass & fl;
+    }
+}
+
 // CONSUMERS: consumer threads (128: four CTAs per SM at the standard shape; 256: three larger ones).
-// HAS_WIDE: the shard has items with more than 255 reads (deep coverage); without them the 16-bit accumulators and
-// their registers do not exist.
+// HAS_WIDE: the shard has items with more than 255 reads (see WideAcc).
 template <int CONSUMERS, bool HAS_WIDE>
 __global__ void __launch_bounds__(CONSUMERS + 32, CONSUMERS == 128 ? 4 : 3)
 pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ items, uint32_t n_items, const PileupShape sh,
@@ -810,37 +847,20 @@ pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ it
 {
     extern __shared__ __align__(128) uint8_t smem[];
     const PileupSmem L = pileup_smem_layout(sh);
+    if (pileup_cta_start<CONSUMERS>(smem, L, sh, 1u, samples, items, n_items, expect, err_flag)) return;
+
+    // ------------------------------------------------------------------------------------ consumers
     uint64_t* full = (uint64_t*)(smem + L.bar);
     uint64_t* empty = full + sh.stages;
     uint32_t* s_cnt = (uint32_t*)(smem + L.cnt);
-
-    if (threadIdx.x == 0) {
-        for (uint32_t s = 0; s < sh.stages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    for (uint32_t k = threadIdx.x; k < (uint32_t)(N_PLANES * TILE_QUADS); k += CONSUMERS + 32) s_cnt[k] = 0;
-    __syncthreads();
-
-    if (threadIdx.x >= CONSUMERS) {
-        pileup_producer(smem, L, sh, samples, items, n_items, expect, err_flag);
-        return;
-    }
-
-    // ------------------------------------------------------------------------------------ consumers
     const uint32_t tid = threadIdx.x;
     uint8_t* s_tags = smem + L.tags;
-    // wide items: per plane and owned quad (QPT * tid + k), 16-bit lanes: [0] = positions 0 and 2, [1] = positions 1 and 3
-    constexpr int QPT = TILE_QUADS / CONSUMERS;                 // quads a thread folds (2 or 1)
-    uint32_t acc[HAS_WIDE ? N_PLANES : 1][QPT][2];
-    #pragma unroll
-    for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
-        #pragma unroll
-        for (int k = 0; k < QPT; ++k) acc[c][k][0] = acc[c][k][1] = 0;
+    WideAcc<CONSUMERS, HAS_WIDE> acc = {};
 
     for (uint32_t chunk_no = 0;; ++chunk_no) {
         const uint32_t st = chunk_no % sh.stages, ph = (chunk_no / sh.stages) & 1u;
         uint8_t* stage = smem + L.stage0 + st * L.stage_bytes;
-        mbar_wait(full + st, ph, sh.wait_hint_ns);
+        mbar_wait(full + st, ph);
         const ChunkHdr* h = (const ChunkHdr*)(stage + L.o_hdr);
         const uint32_t flags = h->flags;
         if (flags & CHUNK_STOP) break;
@@ -877,24 +897,23 @@ pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ it
                 for (int32_t i = i_hi; i < nq; ++i) mute(B + (uint32_t)i);
                 uint32_t g = B + (uint32_t)i_lo, tv = (uint32_t)(jw + i_lo);
                 const uint32_t e = B + (uint32_t)i_hi;                          // tags tv .. tv + (e - g) - 1 are within 0..255
-                if (!(sh.ablate & 2u)) {   // up to three single tags to a word boundary, words of four consecutive tags, up to three single tags
-                    uint32_t hn = (0u - g) & 3u; if (hn > e - g) hn = e - g;
-                    if (hn > 0u) s_tags[g] = (uint8_t)tv;
-                    if (hn > 1u) s_tags[g + 1] = (uint8_t)(tv + 1u);
-                    if (hn > 2u) s_tags[g + 2] = (uint8_t)(tv + 2u);
-                    g += hn; tv += hn;
-                    uint32_t wv = tv * 0x01010101u + 0x03020100u;                   // no lane passes 255: all four quads are on the tile
-                    uint32_t* tw = reinterpret_cast<uint32_t*>(s_tags + g);
-                    const uint32_t nw = (e - g) >> 2;
-                    uint32_t w = 0;
-                    for (; w + 2u <= nw; w += 2u, wv += 0x08080808u) { tw[w] = wv; tw[w + 1] = wv + 0x04040404u; }
-                    if (w < nw) { tw[w] = wv; ++w; }
-                    g += 4u * nw; tv += 4u * nw;
-                    const uint32_t tn = e - g;
-                    if (tn > 0u) s_tags[g] = (uint8_t)tv;
-                    if (tn > 1u) s_tags[g + 1] = (uint8_t)(tv + 1u);
-                    if (tn > 2u) s_tags[g + 2] = (uint8_t)(tv + 2u);
-                }
+                // up to three single tags to a word boundary, words of four consecutive tags, up to three single tags
+                uint32_t hn = (0u - g) & 3u; if (hn > e - g) hn = e - g;
+                if (hn > 0u) s_tags[g] = (uint8_t)tv;
+                if (hn > 1u) s_tags[g + 1] = (uint8_t)(tv + 1u);
+                if (hn > 2u) s_tags[g + 2] = (uint8_t)(tv + 2u);
+                g += hn; tv += hn;
+                uint32_t wv = tv * 0x01010101u + 0x03020100u;                       // no lane passes 255: all four quads are on the tile
+                uint32_t* tw = reinterpret_cast<uint32_t*>(s_tags + g);
+                const uint32_t nw = (e - g) >> 2;
+                uint32_t w = 0;
+                for (; w + 2u <= nw; w += 2u, wv += 0x08080808u) { tw[w] = wv; tw[w + 1] = wv + 0x04040404u; }
+                if (w < nw) { tw[w] = wv; ++w; }
+                g += 4u * nw; tv += 4u * nw;
+                const uint32_t tn = e - g;
+                if (tn > 0u) s_tags[g] = (uint8_t)tv;
+                if (tn > 1u) s_tags[g + 1] = (uint8_t)(tv + 1u);
+                if (tn > 2u) s_tags[g + 2] = (uint8_t)(tv + 2u);
                 B += (uint32_t)nq;
             }
             if (B != B_end) {                                                   // quads no segment owns: keep them out of the counts
@@ -912,7 +931,7 @@ pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ it
         {
             const uint32_t a_q = smem_u32(s_qw), a_s = smem_u32(stage + L.o_seq) + c12, a_f = smem_u32(stage + L.o_fix) + c12, a_g = smem_u32(s_tags);
             const uint32_t a_c = smem_u32(s_cnt), a_e = smem_u32(stage + L.o_exp);
-            for (uint32_t u = tid; u < ((sh.ablate & 1u) ? 0u : ngroups); u += CONSUMERS) {
+            for (uint32_t u = tid; u < ngroups; u += CONSUMERS) {
                 const uint4 qv = lds_v4(a_q + 16u * u);
                 const uint32_t sw = lds_u32(a_s + 4u * u), tw = lds_u32(a_g + 4u * u);
                 const uint32_t qa[4] = {qv.x, qv.y, qv.z, qv.w};
@@ -920,46 +939,34 @@ pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ it
                 if (!has_fix) {
                     #pragma unroll
                     for (int k = 0; k < 4; ++k) {
-                        const uint32_t q = qa[k];
                         const uint32_t j = __byte_perm(tw, 0u, 0x4440u + k);                // tile-relative quad
                         ac[k] = a_c + 4u * j;                                               // its word in plane D
                         xs[k] = msnv_spread_bases(__byte_perm(sw, 0u, 0x4440u + k));        // one 2-bit base per byte lane
-                        const uint32_t v = (q & 0x7f7f7f7fu) + 0x73737373u;                 // bit 7 of a lane: quality >= 13
-                        uint32_t ok;                                                        // ... and the base is A/C/G/T
-                        asm("lop3.b32 %0, %1, %2, 0x80808080, 0x20;" : "=r"(ok) : "r"(v), "r"(q));    // v & ~q & 0x80808080
-                        ok >>= 7;
+                        uint32_t ok;
+                        quad_pass<false>(qa[k], 0u, ok, nn[k]);
                         const uint32_t d = xs[k] ^ lds_u32(a_e + 4u * j);                   // differs from the expected letter?
                         red_shared_add(ac[k], ok);
                         mm[k] = (d | (d >> 1)) & ok;
                         mm_any |= mm[k];
-                        nn[k] = v & q;                                                      // bit 7: counted base that is not A/C/G/T
                         nn_any |= nn[k];
                     }
                 } else {
-                    // the sample has mate verdicts: where the overlap rule spoke (low nibble of the quad's fix byte) its verdict
-                    // (high nibble) replaces the quality test
-                    const uint32_t fw = lds_u32(a_f + 4u * u);
+                    const uint32_t fw = lds_u32(a_f + 4u * u);                              // the quads' verdict bytes
                     #pragma unroll
                     for (int k = 0; k < 4; ++k) {
-                        const uint32_t q = qa[k];
                         const uint32_t j = __byte_perm(tw, 0u, 0x4440u + k);
                         ac[k] = a_c + 4u * j;
                         xs[k] = msnv_spread_bases(__byte_perm(sw, 0u, 0x4440u + k));
-                        const uint32_t f = __byte_perm(fw, 0u, 0x4440u + k);
-                        const uint32_t ovr = nibble_to_lanes(f), val = nibble_to_lanes(f >> 4);
-                        const uint32_t qp = (((q & 0x7f7f7f7fu) + 0x73737373u) >> 7) & 0x01010101u;   // quality >= 13
-                        const uint32_t pass = (qp & ~ovr) | (val & ovr);
-                        const uint32_t fl = (q >> 7) & 0x01010101u;                         // the base is not A/C/G/T
-                        const uint32_t ok = pass & ~fl;
+                        uint32_t ok;
+                        quad_pass<true>(qa[k], __byte_perm(fw, 0u, 0x4440u + k), ok, nn[k]);
                         const uint32_t d = xs[k] ^ lds_u32(a_e + 4u * j);
                         red_shared_add(ac[k], ok);
                         mm[k] = (d | (d >> 1)) & ok;
                         mm_any |= mm[k];
-                        nn[k] = (pass & fl) << 7;
                         nn_any |= nn[k];
                     }
                 }
-                if (mm_any && !(sh.ablate & 32u)) {                                     // counted bases that are not the expected letter:
+                if (mm_any) {                                                           // counted bases that are not the expected letter:
                     #pragma unroll                                                      // only the lanes that hold one loop over their set bits
                     for (int k = 0; k < 4; ++k) {
                         uint32_t r = mm[k];
@@ -970,12 +977,10 @@ pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ it
                         }
                     }
                 }
-                if (nn_any & 0x80808080u) {                                             // rare: counted non-ACGT bases
+                if (nn_any) {                                                           // rare: counted non-ACGT bases
                     #pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        const uint32_t n7 = nn[k] & 0x80808080u;
-                        if (n7) red_shared_add(ac[k] + PLANE_N * (uint32_t)TILE, n7 >> 7);
-                    }
+                    for (int k = 0; k < 4; ++k)
+                        if (nn[k]) red_shared_add(ac[k] + PLANE_N * (uint32_t)TILE, nn[k]);
                 }
             }
         }
@@ -985,27 +990,9 @@ pileup_kernel(const SampleDev* __restrict__ samples, const Item* __restrict__ it
 
         // ---- 4. counts of the chunk
         if (HAS_WIDE && (flags & CHUNK_WIDE)) {
-            #pragma unroll
-            for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
-                #pragma unroll
-                for (int k = 0; k < QPT; ++k) {
-                    const uint32_t slot = c * TILE_QUADS + QPT * tid + k;
-                    const uint32_t w = s_cnt[slot];
-                    s_cnt[slot] = 0;
-                    acc[c][k][0] += w & 0x00ff00ffu; acc[c][k][1] += (w >> 8) & 0x00ff00ffu;
-                }
-            if (flags & CHUNK_LAST) {
-                uint2* dst = reinterpret_cast<uint2*>(tiles + (size_t)item * SLOT_BYTES);
-                #pragma unroll
-                for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
-                    #pragma unroll
-                    for (int k = 0; k < QPT; ++k) {
-                        // 16-bit plane c, positions 4 * (QPT * tid + k) .. + 3
-                        dst[c * (TILE / 4) + QPT * tid + k] = make_uint2((acc[c][k][0] & 0xffffu) | (acc[c][k][1] << 16), (acc[c][k][0] >> 16) | (acc[c][k][1] & 0xffff0000u));
-                        acc[c][k][0] = acc[c][k][1] = 0;
-                    }
-            }
-        } else if ((flags & CHUNK_LAST) && !(sh.ablate & 8u)) {
+            wide_fold<CONSUMERS, HAS_WIDE>(acc, s_cnt, tid);
+            if (flags & CHUNK_LAST) wide_store<CONSUMERS, HAS_WIDE>(acc, tiles + (size_t)item * SLOT_BYTES, tid);
+        } else if (flags & CHUNK_LAST) {
             uint4* cnt4 = reinterpret_cast<uint4*>(s_cnt);
             uint4* dst = reinterpret_cast<uint4*>(tiles + (size_t)item * SLOT_BYTES);
             for (uint32_t i = tid; i < (uint32_t)(N_PLANES * TILE / 16); i += CONSUMERS) {
@@ -1146,7 +1133,6 @@ __device__ __forceinline__ uint2 lds_v2(uint32_t a)
 }
 template <int OFF> __device__ __forceinline__ uint32_t lds_u32_at(uint32_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1+%2];" : "=r"(v) : "r"(a), "n"(OFF)); return v; }
 template <int OFF> __device__ __forceinline__ uint32_t lds_u8_at(uint32_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(v) : "r"(a), "n"(OFF)); return v; }
-__device__ __forceinline__ uint32_t and3(uint32_t a, uint32_t b, uint32_t c) { uint32_t r; asm("lop3.b32 %0, %1, %2, %3, 0x80;" : "=r"(r) : "r"(a), "r"(b), "r"(c)); return r; }
 
 // The records at shared addresses a_rec, a_rec + stride, ... < a_end against the NQ consecutive tile quads j0, j0 + 1, ...
 // of this thread (FIX: the sample carries mate verdicts). a_qj / a_sj / a_fj: shared addresses of the qualities / bases /
@@ -1180,20 +1166,7 @@ __device__ __forceinline__ void gather_quads(uint32_t j0, uint32_t a_rec, uint32
         for (int i = 0; i < NQ; ++i) {
             const uint32_t xs = msnv_spread_bases(st.sv[i]);                        // one 2-bit base per byte lane
             uint32_t ok, nn;
-            if (!FIX) {
-                const uint32_t v = (st.q[i] & 0x7f7f7f7fu) + 0x73737373u;           // bit 7 of a lane: quality >= 13
-                asm("lop3.b32 %0, %1, %2, 0x80808080, 0x20;" : "=r"(ok) : "r"(v), "r"(st.q[i]));        // ... and the base is A/C/G/T
-                ok >>= 7;
-                nn = and3(v, st.q[i], 0x80808080u) >> 7;                            // counted base that is not A/C/G/T
-            } else {
-                // where the overlap rule spoke (low nibble of the quad's fix byte) its verdict (high nibble) replaces the quality test
-                const uint32_t ovr = nibble_to_lanes(st.f[i]), val = nibble_to_lanes(st.f[i] >> 4);
-                const uint32_t qp = (((st.q[i] & 0x7f7f7f7fu) + 0x73737373u) >> 7) & 0x01010101u;
-                const uint32_t pass = (qp & ~ovr) | (val & ovr);
-                const uint32_t fl = (st.q[i] >> 7) & 0x01010101u;
-                ok = pass & ~fl;
-                nn = pass & fl;
-            }
+            quad_pass<FIX>(st.q[i], FIX ? st.f[i] : 0u, ok, nn);
             const uint32_t s1 = xs >> 1;
             D[i] += ok; N[i] += nn;
             X0[i] += xs & ok; X1[i] += s1 & ok; X01[i] += and3(xs, s1, ok);
@@ -1220,37 +1193,20 @@ pileup_gather_kernel(const SampleDev* __restrict__ samples, const Item* __restri
 {
     extern __shared__ __align__(128) uint8_t smem[];
     const PileupSmem L = pileup_smem_layout(sh);
-    uint64_t* full = (uint64_t*)(smem + L.bar);
-    uint64_t* empty = full + sh.stages;
-    uint32_t* s_cnt = (uint32_t*)(smem + L.cnt);
-    constexpr int N_WARPS = CONSUMERS / 32;
-
-    if (threadIdx.x == 0) {
-        for (uint32_t s = 0; s < sh.stages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, N_WARPS); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    for (uint32_t k = threadIdx.x; k < (uint32_t)(N_PLANES * TILE_QUADS); k += CONSUMERS + 32) s_cnt[k] = 0;
     // records and ranges start out empty: a failed consistency check (which fails the run) must not leave wild indices behind
     for (uint32_t s = 0; s < sh.stages; ++s) {
         uint32_t* z = (uint32_t*)(smem + L.stage0 + s * L.stage_bytes + L.o_set);
         for (uint32_t k = threadIdx.x; k < (L.stage_bytes - L.o_set) / 4u; k += CONSUMERS + 32) z[k] = 0;
     }
-    __syncthreads();
-
-    if (threadIdx.x >= CONSUMERS) {
-        pileup_producer(smem, L, sh, samples, items, n_items, expect, err_flag);
-        return;
-    }
+    if (pileup_cta_start<CONSUMERS>(smem, L, sh, CONSUMERS / 32, samples, items, n_items, expect, err_flag)) return;   // (a stage is free when every consumer warp has read it)
 
     // ------------------------------------------------------------------------------------ consumers
+    uint64_t* full = (uint64_t*)(smem + L.bar);
+    uint64_t* empty = full + sh.stages;
+    uint32_t* s_cnt = (uint32_t*)(smem + L.cnt);
     const uint32_t tid = threadIdx.x, lane = tid & 31u;
     constexpr int QPT = TILE_QUADS / CONSUMERS;                 // quad slots per thread (2 or 1): slots QPT * tid, QPT * tid + 1
-    // wide items: per plane and owned quad (QPT * tid + k), 16-bit lanes: [0] = positions 0 and 2, [1] = positions 1 and 3
-    uint32_t acc[HAS_WIDE ? N_PLANES : 1][QPT][2];
-    #pragma unroll
-    for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
-        #pragma unroll
-        for (int k = 0; k < QPT; ++k) acc[c][k][0] = acc[c][k][1] = 0;
+    WideAcc<CONSUMERS, HAS_WIDE> acc = {};
     uint32_t D[QPT], N[QPT], X0[QPT], X1[QPT], X01[QPT];        // counts of this thread's quads (see gather_quads)
     #pragma unroll
     for (int i = 0; i < QPT; ++i) D[i] = N[i] = X0[i] = X1[i] = X01[i] = 0;
@@ -1258,11 +1214,11 @@ pileup_gather_kernel(const SampleDev* __restrict__ samples, const Item* __restri
     for (uint32_t chunk_no = 0;; ++chunk_no) {
         const uint32_t st = chunk_no % sh.stages, ph = (chunk_no / sh.stages) & 1u;
         uint8_t* stage = smem + L.stage0 + st * L.stage_bytes;
-        mbar_wait(full + st, ph, sh.wait_hint_ns);
+        mbar_wait(full + st, ph);
         const ChunkHdr* h = (const ChunkHdr*)(stage + L.o_hdr);
         const uint32_t flags = h->flags;
         if (flags & CHUNK_STOP) break;
-        if (!(sh.ablate & 2u)) gather_setup<CONSUMERS>(stage, L, err_flag);
+        gather_setup<CONSUMERS>(stage, L, err_flag);
         const uint32_t nseg = h->nseg, item = h->item, c12 = h->q4_0 & 12u;
         const uint2* recs = (const uint2*)(stage + L.o_rec);
         const uint32_t* lohi = (const uint32_t*)(stage + L.o_lohi);
@@ -1293,7 +1249,7 @@ pileup_gather_kernel(const SampleDev* __restrict__ samples, const Item* __restri
         {
             // the quads of this thread that a segment of the chunk can cover: [ja, jb)
             const uint32_t ja = j0 > jmin ? j0 : jmin, jb = j0 + QPT < jmax ? j0 + QPT : jmax;
-            if (ja < jb && !(sh.ablate & 1u)) {
+            if (ja < jb) {
                 const uint32_t lo = no_ranges ? 0u : lohi[ja] & 0xffffu;
                 uint32_t hi = no_ranges ? nseg : lohi[jb - 1u] >> 16;
                 if (hi > nseg) hi = nseg;
@@ -1324,7 +1280,7 @@ pileup_gather_kernel(const SampleDev* __restrict__ samples, const Item* __restri
         if (lane == 0) mbar_arrive(empty + st);
 
         if (direct) {
-            if ((flags & CHUNK_LAST) && !(sh.ablate & 8u)) {
+            if (flags & CHUNK_LAST) {
                 #pragma unroll
                 for (int c = 0; c < N_PLANES; ++c) {
                     if (QPT == 2) reinterpret_cast<uint2*>(dst)[(c * TILE_QUADS + j0) >> 1] = make_uint2(out[0][c], out[QPT - 1][c]);     // (j0 is even)
@@ -1343,26 +1299,8 @@ pileup_gather_kernel(const SampleDev* __restrict__ samples, const Item* __restri
             }
         consumer_sync<CONSUMERS>();
         if (HAS_WIDE) {
-            #pragma unroll
-            for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
-                #pragma unroll
-                for (int k = 0; k < QPT; ++k) {
-                    const uint32_t slot = c * TILE_QUADS + QPT * tid + k;
-                    const uint32_t w = s_cnt[slot];
-                    s_cnt[slot] = 0;
-                    acc[c][k][0] += w & 0x00ff00ffu; acc[c][k][1] += (w >> 8) & 0x00ff00ffu;
-                }
-            if (flags & CHUNK_LAST) {
-                uint2* dst2 = reinterpret_cast<uint2*>(tiles + (size_t)item * SLOT_BYTES);
-                #pragma unroll
-                for (int c = 0; c < (HAS_WIDE ? N_PLANES : 1); ++c)
-                    #pragma unroll
-                    for (int k = 0; k < QPT; ++k) {
-                        // 16-bit plane c, positions 4 * (QPT * tid + k) .. + 3
-                        dst2[c * (TILE / 4) + QPT * tid + k] = make_uint2((acc[c][k][0] & 0xffffu) | (acc[c][k][1] << 16), (acc[c][k][0] >> 16) | (acc[c][k][1] & 0xffff0000u));
-                        acc[c][k][0] = acc[c][k][1] = 0;
-                    }
-            }
+            wide_fold<CONSUMERS, HAS_WIDE>(acc, s_cnt, tid);
+            if (flags & CHUNK_LAST) wide_store<CONSUMERS, HAS_WIDE>(acc, tiles + (size_t)item * SLOT_BYTES, tid);
         }
         consumer_sync<CONSUMERS>();             // the planes are folded and cleared before the next chunk adds to them
     }

@@ -294,20 +294,29 @@ static bool pileup_gather_mode(bool deep)
     return !deep;
 }
 
-static PileupShape choose_pileup_shape(uint64_t n_reads, uint64_t n_bases, uint64_t n_segs, uint64_t n_items, uint64_t item_reads, uint32_t item_reads_max, bool has_fix, int max_ctas, int& ctas)
+// the pileup kernel of a form, a number of consumer threads per CTA (128 or 256) and with or without the 16-bit accumulators
+using PileupKernelFn = void (*)(const SampleDev*, const Item*, uint32_t, const PileupShape, const uint8_t*, uint8_t*, int*);
+static PileupKernelFn pileup_kernel_for(bool gather, int consumers, bool has_wide)
+{
+    if (gather) {
+        if (consumers == 256) return has_wide ? pileup_gather_kernel<256, true> : pileup_gather_kernel<256, false>;
+        return has_wide ? pileup_gather_kernel<128, true> : pileup_gather_kernel<128, false>;
+    }
+    if (consumers == 256) return has_wide ? pileup_kernel<256, true> : pileup_kernel<256, false>;
+    return has_wide ? pileup_kernel<128, true> : pileup_kernel<128, false>;
+}
+
+// deep: the shard averages more than 200 reads per item (items take several chunks whatever the limits)
+static PileupShape choose_pileup_shape(uint64_t n_reads, uint64_t n_bases, uint64_t n_segs, uint64_t n_items, uint64_t item_reads, uint32_t item_reads_max, bool has_fix, bool deep,
+                                       int max_ctas, int& ctas)
 {
     const double reads_per_item = (double)item_reads / (double)(n_items ? n_items : 1);
     const double q4_per_read = (double)n_bases / 4.0 / (double)(n_reads ? n_reads : 1);
     const double segs_per_read = (double)n_segs / (double)(n_reads ? n_reads : 1);
-    const bool deep = reads_per_item > 200.0;          // items take several chunks whatever the limits
     PileupShape sh{};
     sh.gather = pileup_gather_mode(deep) ? 1u : 0u;
     sh.has_fix = has_fix ? 1u : 0u;
-    sh.wait_hint_ns = getenv("MSNV_WAIT_HINT_NS") ? (uint32_t)atoi(getenv("MSNV_WAIT_HINT_NS")) : 0u;
-    sh.ablate = getenv("MSNV_ABLATE") ? (uint32_t)atoi(getenv("MSNV_ABLATE")) : 0u;
     sh.stages = 2;
-    // (measured: sleeping 200 / 1000 ns between the producer's polls changes nothing, 3000 ns costs 5 %; the plain try_wait executes fewer instructions)
-    sh.producer_hint_ns = getenv("MSNV_PRODUCER_HINT_NS") ? (uint32_t)atoi(getenv("MSNV_PRODUCER_HINT_NS")) : 0u;
     if (const char* e = getenv("MSNV_STAGES")) { const int v = atoi(e); if (v >= 2 && v <= (int)PL_STAGES_MAX) sh.stages = (uint32_t)v; }
     uint32_t mr = deep ? (max_ctas <= 3 ? NARROW_MAX_READS : 96u) : (uint32_t)(reads_per_item * 1.3 + 24.0);
     if (!deep && item_reads_max && mr > item_reads_max) mr = item_reads_max;      // no item has more reads than this
@@ -427,28 +436,18 @@ static int launch_pileup(msnv_ctx* ctx, const msnv_ctx::Window& w, uint32_t a, u
     int ctas = 1;
     bool has_fix = false;
     for (const SampleDev& sd : w.h_samples) has_fix = has_fix || sd.fix;
-    const PileupShape sh = choose_pileup_shape(w.n_reads, w.n_bases, w.n_segs, n_items_window, item_reads, item_reads_max, has_fix, consumers == 256 ? 3 : 4, ctas);   // register-bound CTA counts
+    const PileupShape sh = choose_pileup_shape(w.n_reads, w.n_bases, w.n_segs, n_items_window, item_reads, item_reads_max, has_fix, deep, consumers == 256 ? 3 : 4, ctas);   // register-bound CTA counts
     const size_t smem = pileup_smem_layout(sh).total;
     const bool has_wide = item_reads_max > NARROW_MAX_READS;
     const int threads = consumers + 32;
+    const PileupKernelFn K = pileup_kernel_for(sh.gather, consumers, has_wide);
     int fit = 0;
-#define MSNV_PILEUP_DISPATCH(EXPR)                                                                  \
-    do {                                                                                            \
-        if (sh.gather) {                                                                            \
-            if (consumers == 256) { if (has_wide) { auto K = pileup_gather_kernel<256, true>; EXPR; } else { auto K = pileup_gather_kernel<256, false>; EXPR; } } \
-            else                  { if (has_wide) { auto K = pileup_gather_kernel<128, true>; EXPR; } else { auto K = pileup_gather_kernel<128, false>; EXPR; } } \
-        } else {                                                                                    \
-            if (consumers == 256) { if (has_wide) { auto K = pileup_kernel<256, true>; EXPR; } else { auto K = pileup_kernel<256, false>; EXPR; } } \
-            else                  { if (has_wide) { auto K = pileup_kernel<128, true>; EXPR; } else { auto K = pileup_kernel<128, false>; EXPR; } } \
-        }                                                                                           \
-    } while (0)
-    MSNV_PILEUP_DISPATCH(CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, K, threads, smem)));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, K, threads, smem));
     if (fit < 1) return fail(ctx, MSNV_E_CUDA, "pileup kernel does not fit an SM (%zu bytes of shared memory)", smem);
     if (fit < ctas) ctas = fit;
     uint64_t grid = (uint64_t)ctas * (uint64_t)ctx->sm_count;
     if (grid > n) grid = n;
-    MSNV_PILEUP_DISPATCH((K<<<(unsigned)grid, threads, smem, ctx->stream>>>(w.d_samples, ctx->d_items + a, n, sh, ctx->d_expect, ctx->d_tiles, ctx->d_err)));
-#undef MSNV_PILEUP_DISPATCH
+    K<<<(unsigned)grid, threads, smem, ctx->stream>>>(w.d_samples, ctx->d_items + a, n, sh, ctx->d_expect, ctx->d_tiles, ctx->d_err);
     ++launches;
     if (getenv("MSNV_VERBOSE"))
         fprintf(stderr, "msnv: pileup (%s) %u items (%.1f reads each, at most %u), %u CTAs (%d per SM) x %d threads%s, stage limits %u reads / %u segments / %u quads, %zu B shared memory\n",
@@ -647,14 +646,10 @@ int msnv_create(int device, msnv_ctx** out)
     CU(cudaMalloc((void**)&ctx->d_xstat, 16));
     CU(cudaMemset(ctx->d_xstat, 0, 16));
     CU(cudaMallocHost((void**)&ctx->h_scalar, 32));
-    CU(cudaFuncSetAttribute(pileup_kernel<128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_kernel<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_gather_kernel<128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_gather_kernel<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_gather_kernel<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
-    CU(cudaFuncSetAttribute(pileup_gather_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
+    for (bool gather : {false, true})
+        for (int consumers : {128, 256})
+            for (bool has_wide : {false, true})
+                CU(cudaFuncSetAttribute(pileup_kernel_for(gather, consumers, has_wide), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_PER_CTA_MAX));
     CU(cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device));
     return MSNV_OK;
 }

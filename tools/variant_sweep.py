@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Tuning aid: one device-generated shard, msnv_shard_run under several staging settings of the pileup kernel
-(MSNV_PILEUP_CTAS : MSNV_CHUNK_Q4 : MSNV_MAX_READS : MSNV_WAIT_HINT_NS : MSNV_CONSUMERS : MSNV_ABLATE : MSNV_PILEUP : MSNV_STAGES : MSNV_PRODUCER_HINT_NS, empty = the library's own choice)."""
+(MSNV_PILEUP_CTAS : MSNV_CHUNK_Q4 : MSNV_MAX_READS : MSNV_CONSUMERS : MSNV_PILEUP : MSNV_STAGES, empty = the library's own choice)."""
 import argparse, json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from metasnv_b200 import abi, harness as H
@@ -8,7 +8,7 @@ from metasnv_b200 import abi, harness as H
 ap = argparse.ArgumentParser()
 ap.add_argument("--preset", default="c2"); ap.add_argument("--scale", type=float, default=1.0)
 ap.add_argument("--samples", type=int, default=0); ap.add_argument("--steps", type=int, default=3)
-ap.add_argument("--no-hits", action="store_true", help="thresholds no position meets (for ablation runs whose counts are garbage)")
+ap.add_argument("--no-hits", action="store_true", help="thresholds no position meets (no hits to gather and copy)")
 ap.add_argument("--settings", default="::,2::,3::,4::,5::", help="comma list of <ctas per SM>:<chunk_q4>:<max_reads>, empty fields = default")
 a = ap.parse_args()
 desc = H.describe(a.preset, a.scale, a.samples)
@@ -18,8 +18,8 @@ if first >= 0:
     ctx.shard_mask_position(first)
 ref_hits = None
 for setting in a.settings.split(","):
-    fields = (setting.split(":") + [""] * 9)[:9]
-    for k, v in zip(("MSNV_PILEUP_CTAS", "MSNV_CHUNK_Q4", "MSNV_MAX_READS", "MSNV_WAIT_HINT_NS", "MSNV_CONSUMERS", "MSNV_ABLATE", "MSNV_PILEUP", "MSNV_STAGES", "MSNV_PRODUCER_HINT_NS"), fields):
+    fields = (setting.split(":") + [""] * 6)[:6]
+    for k, v in zip(("MSNV_PILEUP_CTAS", "MSNV_CHUNK_Q4", "MSNV_MAX_READS", "MSNV_CONSUMERS", "MSNV_PILEUP", "MSNV_STAGES"), fields):
         os.environ.pop(k, None)
         if v:
             os.environ[k] = v
