@@ -278,6 +278,42 @@ typedef struct {
 #define MSNV_COV_MAX_COUNTERS (1u << 27)
 int msnv_cov_run(msnv_ctx* ctx, const msnv_cov_blocks* blocks, uint32_t max_cov, uint64_t* cov_sum, uint64_t* hist);
 
+/* ---- BGZF inflate on the device (the decompression in front of every BAM decode) ----
+ * An inflater owns a stream, device buffers and page-locked staging buffers on one device. It is separate from the
+ * context: one inflater serves one host thread at a time, and different inflaters may be used from different threads
+ * at the same time as each other and as a context's calls. */
+typedef struct msnv_inflater msnv_inflater;
+
+/* One BGZF member of a batch: its raw-DEFLATE data comp[coff, coff + clen), the ISIZE and CRC32 of its trailer, and
+ * where its isize inflated bytes go in the output (out[ooff, ooff + isize)). */
+typedef struct { uint64_t coff; uint32_t clen, isize, crc, reserved; uint64_t ooff; } msnv_bgzf_member;
+
+/* Per-member result of msnv_inflate(). */
+typedef enum {
+    MSNV_INFLATE_OK = 0,
+    MSNV_INFLATE_TRUNCATED = 1,     /* the stream ends before its final block does */
+    MSNV_INFLATE_BAD_CODE = 2,      /* invalid block type, stored length, code lengths or code */
+    MSNV_INFLATE_BAD_DISTANCE = 3,  /* a match reaches in front of the member's first output byte */
+    MSNV_INFLATE_TOO_LONG = 4,      /* the stream holds more than isize bytes */
+    MSNV_INFLATE_TOO_SHORT = 5,     /* the stream holds fewer than isize bytes */
+    MSNV_INFLATE_BAD_CRC = 6        /* the inflated bytes do not have the trailer's CRC32 */
+} msnv_inflate_status;
+
+/* max_batch_bytes bounds both comp_bytes and the output span of one msnv_inflate() call, and a call takes at most
+ * msnv_inflater_max_members(max_batch_bytes) = max_batch_bytes / 64 + 1024 members (MSNV_E_LIMIT beyond; a BGZF member
+ * of real data is far larger than 64 bytes). Every buffer is allocated here, none later. */
+uint32_t    msnv_inflater_max_members(size_t max_batch_bytes);
+int         msnv_inflater_create(int device, size_t max_batch_bytes, msnv_inflater** out);
+/* Inflates n members into out[0, max(ooff + isize)) and returns when out is filled on the host. status[i] is the
+ * member's msnv_inflate_status; a malformed member affects no other member. Output bytes that no member covers are
+ * unspecified. Returns MSNV_E_ARG for a member outside comp or a batch above max_batch_bytes. */
+int         msnv_inflate(msnv_inflater* inf, const uint8_t* comp, size_t comp_bytes, const msnv_bgzf_member* m, uint32_t n,
+                         uint8_t* out, int32_t* status);
+void        msnv_inflater_destroy(msnv_inflater* inf);
+const char* msnv_inflater_last_error(const msnv_inflater* inf);
+/* Device time of the last msnv_inflate() call's kernel, milliseconds (CUDA events; copies excluded). */
+int         msnv_inflater_kernel_ms(const msnv_inflater* inf, float* ms);
+
 #ifdef __cplusplus
 }
 #endif

@@ -70,6 +70,14 @@ class SampleSizes(C.Structure):
                 ("n_segs", C.c_uint64), ("n_q4", C.c_uint64), ("n_aligned", C.c_uint64)]
 
 
+class BgzfMember(C.Structure):
+    _fields_ = [("coff", C.c_uint64), ("clen", C.c_uint32), ("isize", C.c_uint32), ("crc", C.c_uint32), ("reserved", C.c_uint32),
+                ("ooff", C.c_uint64)]
+
+
+# msnv_inflate_status
+INFLATE_OK, INFLATE_TRUNCATED, INFLATE_BAD_CODE, INFLATE_BAD_DISTANCE, INFLATE_TOO_LONG, INFLATE_TOO_SHORT, INFLATE_BAD_CRC = range(7)
+
 _lib = None
 
 
@@ -118,6 +126,15 @@ def load():
     lib.msnv_window_synth.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(SynthDesc), C.c_uint32, C.c_uint32]
     lib.msnv_shard_export_sample.argtypes = [C.c_void_p, C.c_uint32] + [C.c_void_p] * 8
     lib.msnv_shard_export_ref.argtypes = [C.c_void_p, C.c_void_p]
+    lib.msnv_inflater_create.argtypes = [C.c_int, C.c_size_t, C.POINTER(C.c_void_p)]
+    lib.msnv_inflate.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
+    lib.msnv_inflater_destroy.argtypes = [C.c_void_p]
+    lib.msnv_inflater_destroy.restype = None
+    lib.msnv_inflater_last_error.argtypes = [C.c_void_p]
+    lib.msnv_inflater_last_error.restype = C.c_char_p
+    lib.msnv_inflater_kernel_ms.argtypes = [C.c_void_p, C.POINTER(C.c_float)]
+    lib.msnv_inflater_max_members.argtypes = [C.c_size_t]
+    lib.msnv_inflater_max_members.restype = C.c_uint32
     _lib = lib
     return lib
 
@@ -402,3 +419,98 @@ def window_slice(arrays, pos_lo, pos_hi):
             "q4_off": (arrays["q4_off"][lo:hi + 1] - q0).astype(np.uint32), "mate": mate.astype(np.int32),
             "seg_pos": arrays["seg_pos"][s0:s1].copy(), "seg_len": arrays["seg_len"][s0:s1].copy(),
             "seq2": arrays["seq2"][q0:q1].copy(), "qual": arrays["qual"][4 * q0:4 * q1].copy()}
+
+
+class Inflater:
+    """msnv_inflater: BGZF members inflated on the device. One thread at a time per inflater; several inflaters may run
+    at once, next to a Context's calls."""
+
+    def __init__(self, device=0, max_batch_bytes=8 << 20):
+        self.lib = load()
+        self.max_batch_bytes = max_batch_bytes
+        h = C.c_void_p()
+        rc = self.lib.msnv_inflater_create(device, max_batch_bytes, C.byref(h))
+        if rc != 0:
+            msg = self.lib.msnv_inflater_last_error(h).decode()
+            self.lib.msnv_inflater_destroy(h)
+            raise MsnvError("msnv_inflater_create failed (%d): %s" % (rc, msg))
+        self.h = h
+
+    def close(self):
+        if self.h:
+            self.lib.msnv_inflater_destroy(self.h)
+            self.h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def inflate(self, comp, members):
+        """comp: uint8 array; members: numpy structured array with BgzfMember's fields (or a BgzfMember ctypes array).
+        Returns (out uint8 array of max(ooff + isize) bytes, int32 status per member)."""
+        import numpy as np
+        comp = np.ascontiguousarray(comp, dtype=np.uint8)
+        m = np.ascontiguousarray(members)
+        n = len(m)
+        out_bytes = int(max((int(x["ooff"]) + int(x["isize"]) for x in m), default=0))
+        out = np.zeros(max(out_bytes, 1), np.uint8)
+        status = np.full(max(n, 1), -1, np.int32)
+        rc = self.lib.msnv_inflate(self.h, _ptr(comp), comp.size, m.ctypes.data_as(C.c_void_p), n, _ptr(out), _ptr(status))
+        if rc != 0:
+            raise MsnvError("msnv_inflate failed (%d): %s" % (rc, self.lib.msnv_inflater_last_error(self.h).decode()))
+        return out[:out_bytes], status[:n]
+
+    def kernel_ms(self):
+        ms = C.c_float()
+        self.lib.msnv_inflater_kernel_ms(self.h, C.byref(ms))
+        return ms.value
+
+
+MEMBER_DTYPE = [("coff", "<u8"), ("clen", "<u4"), ("isize", "<u4"), ("crc", "<u4"), ("reserved", "<u4"), ("ooff", "<u8")]
+
+
+def bgzf_members(path_or_bytes):
+    """The BGZF members of a file, as msnv_inflate takes them: (compressed bytes, structured array of members whose
+    coff index the file and whose ooff lay the members out back to back). Parsed from the format (SAMv1 4.1)."""
+    import numpy as np
+    data = open(path_or_bytes, "rb").read() if isinstance(path_or_bytes, str) else bytes(path_or_bytes)
+    rows, pos, ooff = [], 0, 0
+    while pos < len(data):
+        xlen = int.from_bytes(data[pos + 10:pos + 12], "little")
+        bsize, off = None, 0
+        while off + 4 <= xlen:
+            x = pos + 12 + off
+            slen = int.from_bytes(data[x + 2:x + 4], "little")
+            if data[x:x + 2] == b"BC" and slen == 2:
+                bsize = int.from_bytes(data[x + 4:x + 6], "little")
+            off += 4 + slen
+        if bsize is None:
+            raise ValueError("BGZF member without BC subfield at %d" % pos)
+        end = pos + bsize + 1
+        crc = int.from_bytes(data[end - 8:end - 4], "little")
+        isize = int.from_bytes(data[end - 4:end], "little")
+        rows.append((pos + 12 + xlen, end - 8 - (pos + 12 + xlen), isize, crc, 0, ooff))
+        ooff += isize
+        pos = end
+    return np.frombuffer(data, np.uint8), np.array(rows, dtype=MEMBER_DTYPE)
+
+
+def bgzf_batches(comp, members, max_batch_bytes):
+    """Cut a file's members (bgzf_members) into msnv_inflate batches of at most max_batch_bytes on either side: a list of
+    (compressed bytes, members with coff and ooff relative to the batch)."""
+    out, i, n = [], 0, len(members)
+    while i < n:
+        j, c0, o0 = i, int(members[i]["coff"]), int(members[i]["ooff"])
+        while j < n and int(members[j]["ooff"]) + int(members[j]["isize"]) - o0 <= max_batch_bytes and \
+                int(members[j]["coff"]) + int(members[j]["clen"]) - c0 <= max_batch_bytes:
+            j += 1
+        if j == i:
+            raise ValueError("member %d does not fit a batch of %d bytes" % (i, max_batch_bytes))
+        sub = members[i:j].copy()
+        sub["coff"] -= c0
+        sub["ooff"] -= o0
+        out.append((comp[c0:int(sub[-1]["coff"]) + c0 + int(sub[-1]["clen"])], sub))
+        i = j
+    return out

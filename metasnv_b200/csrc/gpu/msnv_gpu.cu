@@ -18,6 +18,7 @@
 #include <string>
 #include <vector>
 
+#include "inflate_kernels.cuh"
 #include "kernels.cuh"
 #include "synth_kernels.cuh"
 
@@ -1279,3 +1280,125 @@ int msnv_cov_run(msnv_ctx* ctx, const msnv_cov_blocks* b, uint32_t max_cov, uint
 }
 
 }  // extern "C"
+
+// ---- BGZF inflate: an object of its own, so that every decoding thread can own one next to the context's thread
+struct msnv_inflater {
+    int device = 0;
+    size_t max_bytes = 0;
+    cudaStream_t stream = nullptr;
+    std::string err;
+    uint8_t *h_comp = nullptr, *h_out = nullptr;                // page-locked staging, max_bytes each
+    uint8_t *d_comp = nullptr, *d_out = nullptr;
+    msnv_bgzf_member *h_m = nullptr, *d_m = nullptr;
+    int32_t *h_status = nullptr, *d_status = nullptr;
+    uint32_t cap_m = 0;
+    cudaEvent_t ev[2] = {};
+    float kernel_ms = 0;
+};
+
+namespace {
+int inf_fail(msnv_inflater* f, int code, const char* fmt, ...)
+{
+    char buf[512];
+    va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
+    if (f) f->err = buf;
+    return code;
+}
+#define CUI(call)                                                                                        \
+    do {                                                                                                 \
+        cudaError_t e_ = (call);                                                                         \
+        if (e_ != cudaSuccess) return inf_fail(inf, MSNV_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
+    } while (0)
+}  // namespace
+
+extern "C" {
+
+uint32_t msnv_inflater_max_members(size_t max_batch_bytes) { return (uint32_t)std::min<uint64_t>(max_batch_bytes / 64 + 1024, 0xffffffffu); }
+
+int msnv_inflater_create(int device, size_t max_batch_bytes, msnv_inflater** out)
+{
+    if (!out) return MSNV_E_ARG;
+    *out = nullptr;
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0 || device < 0 || device >= n) return MSNV_E_CUDA;
+    if (max_batch_bytes == 0) return MSNV_E_ARG;
+    msnv_inflater* inf = new msnv_inflater();
+    inf->device = device;
+    inf->max_bytes = max_batch_bytes;
+    *out = inf;                                   // returned even on failure so the caller can read the error
+    CUI(cudaSetDevice(device));
+    CUI(cudaStreamCreateWithFlags(&inf->stream, cudaStreamNonBlocking));
+    for (auto& e : inf->ev) CUI(cudaEventCreate(&e));
+    CUI(cudaMallocHost((void**)&inf->h_comp, max_batch_bytes));
+    CUI(cudaMallocHost((void**)&inf->h_out, max_batch_bytes));
+    CUI(cudaMalloc((void**)&inf->d_comp, max_batch_bytes));
+    CUI(cudaMalloc((void**)&inf->d_out, max_batch_bytes));
+    // member arrays sized once for the largest batch: growing them later would free memory, which waits for the whole
+    // device, including a context's work on another thread
+    const uint64_t cap = msnv_inflater_max_members(max_batch_bytes);
+    CUI(cudaMallocHost((void**)&inf->h_m, cap * sizeof(msnv_bgzf_member)));
+    CUI(cudaMallocHost((void**)&inf->h_status, cap * 4));
+    CUI(cudaMalloc((void**)&inf->d_m, cap * sizeof(msnv_bgzf_member)));
+    CUI(cudaMalloc((void**)&inf->d_status, cap * 4));
+    inf->cap_m = (uint32_t)cap;
+    return MSNV_OK;
+}
+
+void msnv_inflater_destroy(msnv_inflater* inf)
+{
+    if (!inf) return;
+    cudaSetDevice(inf->device);
+    if (inf->stream) cudaStreamSynchronize(inf->stream);
+    cudaFreeHost(inf->h_comp); cudaFreeHost(inf->h_out); cudaFreeHost(inf->h_m); cudaFreeHost(inf->h_status);
+    cudaFree(inf->d_comp); cudaFree(inf->d_out); cudaFree(inf->d_m); cudaFree(inf->d_status);
+    for (auto& e : inf->ev) if (e) cudaEventDestroy(e);
+    if (inf->stream) cudaStreamDestroy(inf->stream);
+    delete inf;
+}
+
+const char* msnv_inflater_last_error(const msnv_inflater* inf) { return inf ? inf->err.c_str() : "no inflater (no CUDA device?)"; }
+
+int msnv_inflater_kernel_ms(const msnv_inflater* inf, float* ms)
+{
+    if (!inf || !ms) return MSNV_E_ARG;
+    *ms = inf->kernel_ms;
+    return MSNV_OK;
+}
+
+int msnv_inflate(msnv_inflater* inf, const uint8_t* comp, size_t comp_bytes, const msnv_bgzf_member* m, uint32_t n,
+                 uint8_t* out, int32_t* status)
+{
+    if (!inf || (n && (!comp || !m || !out || !status))) return MSNV_E_ARG;
+    inf->kernel_ms = 0;
+    if (n == 0) return MSNV_OK;
+    if (n > inf->cap_m) return inf_fail(inf, MSNV_E_LIMIT, "msnv_inflate: %u members exceed the inflater's %u", n, inf->cap_m);
+    if (comp_bytes > inf->max_bytes) return inf_fail(inf, MSNV_E_ARG, "msnv_inflate: %zu compressed bytes exceed the inflater's batch of %zu", comp_bytes, inf->max_bytes);
+    uint64_t out_bytes = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (m[i].coff > comp_bytes || m[i].clen > comp_bytes - m[i].coff)
+            return inf_fail(inf, MSNV_E_ARG, "msnv_inflate: member %u lies outside the %zu compressed bytes", i, comp_bytes);
+        if (m[i].ooff > inf->max_bytes || m[i].isize > inf->max_bytes - m[i].ooff)
+            return inf_fail(inf, MSNV_E_ARG, "msnv_inflate: member %u's output exceeds the inflater's batch of %zu bytes", i, inf->max_bytes);
+        out_bytes = std::max<uint64_t>(out_bytes, m[i].ooff + m[i].isize);
+    }
+    CUI(cudaSetDevice(inf->device));
+    cudaStream_t st = inf->stream;
+    memcpy(inf->h_comp, comp, comp_bytes);
+    memcpy(inf->h_m, m, (size_t)n * sizeof(msnv_bgzf_member));
+    CUI(cudaMemcpyAsync(inf->d_comp, inf->h_comp, comp_bytes, cudaMemcpyHostToDevice, st));
+    CUI(cudaMemcpyAsync(inf->d_m, inf->h_m, (size_t)n * sizeof(msnv_bgzf_member), cudaMemcpyHostToDevice, st));
+    CUI(cudaEventRecord(inf->ev[0], st));
+    inflate_kernel<<<(n + INFLATE_WARPS - 1) / INFLATE_WARPS, INFLATE_WARPS * 32, 0, st>>>(inf->d_comp, inf->d_m, n, inf->d_out, inf->d_status);
+    CUI(cudaGetLastError());
+    CUI(cudaEventRecord(inf->ev[1], st));
+    CUI(cudaMemcpyAsync(inf->h_out, inf->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+    CUI(cudaMemcpyAsync(inf->h_status, inf->d_status, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+    CUI(cudaStreamSynchronize(st));
+    cudaEventElapsedTime(&inf->kernel_ms, inf->ev[0], inf->ev[1]);
+    memcpy(out, inf->h_out, out_bytes);
+    memcpy(status, inf->h_status, (size_t)n * 4);
+    return MSNV_OK;
+}
+
+}  // extern "C"
+#undef CUI
