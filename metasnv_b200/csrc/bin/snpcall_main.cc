@@ -70,7 +70,7 @@ static int pick_device(const std::string& indiv_path)
 struct Job { std::string ref, bed, list; };
 
 // Pinned bounce buffers between the decoding threads and the device. Page-locking memory costs about a second per
-// gigabyte, so the pool is small (a few chunks, locked in the background while the reference is being read) and
+// gigabyte, so the pool is small (a few chunks, locked in the background while the first window decodes) and
 // recycled: a decoding thread copies its finished batch into the chunk that is being filled (several batches share a
 // chunk), the main thread queues the upload from there (DMA at the host link's rate, it overlaps the decoding) and a
 // chunk goes back to the pool once it is full and the copies of all its batches have run.
@@ -83,19 +83,19 @@ struct BouncePool {
     std::vector<int> free_ids;
     int cur = -1;                                          // the chunk being filled
     bool closed = false;                                   // no more chunks will come (allocation failed or stopped)
-    bool started = false;                                  // chunks are being page-locked (needs the CUDA context); batches decoded before that are staged afterwards
-    void start() { { std::lock_guard<std::mutex> lk(mu); started = true; } cv.notify_all(); }
-    bool is_started() { std::lock_guard<std::mutex> lk(mu); return started; }
-    void wait_started() { std::unique_lock<std::mutex> lk(mu); cv.wait(lk, [&] { return started || closed; }); }
+    bool aborted = false;                                  // the run failed: no chunk will be handed back, so none is handed out
     void add(uint8_t* p) { { std::lock_guard<std::mutex> lk(mu); chunks.push_back(Chunk{p, 0, 0, false}); free_ids.push_back((int)chunks.size() - 1); } cv.notify_all(); }
     void close() { { std::lock_guard<std::mutex> lk(mu); closed = true; } cv.notify_all(); }
-    // room for one batch: (pointer, chunk id), or (nullptr, -1) when the batch is larger than a chunk or there is no pool
+    void abort() { { std::lock_guard<std::mutex> lk(mu); aborted = true; } cv.notify_all(); }
+    // room for one batch: (pointer, chunk id), or (nullptr, -1) when the batch is larger than a chunk, there is no pool or
+    // the run failed
     uint8_t* acquire(size_t bytes, int& id) {
         const size_t need = (bytes + 255) & ~(size_t)255;
         id = -1;
         if (need > CHUNK) return nullptr;
         std::unique_lock<std::mutex> lk(mu);
         for (;;) {
+            if (aborted) return nullptr;
             if (cur >= 0 && chunks[cur].used + need <= CHUNK) break;
             if (cur >= 0) { chunks[cur].sealed = true; maybe_free(cur); cur = -1; }
             if (!free_ids.empty()) { cur = free_ids.back(); free_ids.pop_back(); chunks[cur].used = 0; chunks[cur].sealed = false; break; }
@@ -122,30 +122,6 @@ private:
 static size_t pack_step(size_t& off, size_t bytes) { const size_t o = off; off = (off + bytes + 32 + 255) & ~(size_t)255; return o; }
 
 // one sample's batch as the library wants it: copied into a bounce chunk when it fits one (else the decoder's own arrays)
-static msnv_sample_reads stage_batch(const SampleReads& r, BouncePool& pool, int& chunk)
-{
-    msnv_sample_reads v = r.view();
-    chunk = -1;
-    if (v.n_reads == 0) return v;
-    size_t off = 0;
-    const size_t o_pos = pack_step(off, r.pos.size() * 4), o_sgo = pack_step(off, r.seg_off.size() * 4), o_q4 = pack_step(off, r.q4_off.size() * 4),
-                 o_mate = pack_step(off, r.mate.size() * 4), o_sp = pack_step(off, r.seg_pos.size() * 4), o_sl = pack_step(off, r.seg_len.size() * 2),
-                 o_seq = pack_step(off, r.seq2.size()), o_qual = pack_step(off, r.qual.size());
-    uint8_t* p = pool.acquire(off, chunk);
-    if (!p) return v;
-    auto put = [&](size_t o, const void* src, size_t bytes) { memcpy(p + o, src, bytes); return p + o; };
-    v.pos = (const int32_t*)put(o_pos, r.pos.data(), r.pos.size() * 4);
-    v.seg_off = (const uint32_t*)put(o_sgo, r.seg_off.data(), r.seg_off.size() * 4);
-    v.q4_off = (const uint32_t*)put(o_q4, r.q4_off.data(), r.q4_off.size() * 4);
-    v.mate = (const int32_t*)put(o_mate, r.mate.data(), r.mate.size() * 4);
-    v.seg_pos = (const int32_t*)put(o_sp, r.seg_pos.data(), r.seg_pos.size() * 4);
-    v.seg_len = (const uint16_t*)put(o_sl, r.seg_len.data(), r.seg_len.size() * 2);
-    v.seq2 = put(o_seq, r.seq2.data(), r.seq2.size());
-    v.qual = put(o_qual, r.qual.data(), r.qual.size());
-    return v;
-}
-
-// the same for a BAM-shaped batch (the device expands it)
 static msnv_raw_reads stage_raw(const RawReads& r, BouncePool& pool, int& chunk)
 {
     msnv_raw_reads v = r.view();
@@ -240,11 +216,11 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
     const uint32_t tiles_per_window = (n_tiles + n_windows - 1) / n_windows;
     n_windows = (n_tiles + tiles_per_window - 1) / tiles_per_window;
 
-    // MSNV_EARLY_DECODE=1: decode the first window while the CUDA context comes up (batches are staged into bounce chunks once they
-    // can be page-locked). Default: wait for the context first - 21 interleaved runs on four boxes show no difference in the mean
-    // (4.1 s against 4.0 s on 2 GB of BAM): the early decode hides a slow context (1 - 3 s) but decodes slower while the driver maps
+    // wait for the context before decoding: decoding while it comes up gains nothing on average (21 interleaved runs on four
+    // boxes, 2 GB of BAM: 4.1 s against 4.0 s) - it hides a slow context (1 - 3 s) but decodes slower while the driver maps
     // memory (the decoders' page faults and the driver's mappings contend for the address-space lock); BASELINE.md section 4.
-    if (!(getenv("MSNV_EARLY_DECODE") && atoi(getenv("MSNV_EARLY_DECODE")) != 0) && ctx_thread.joinable()) ctx_thread.join();
+    ctx_thread.join();
+    stage("CUDA context created");
 
     // ---- decoders (one per BAM, resumable) and the thread pool
     int n_threads = (int)std::thread::hardware_concurrency();
@@ -274,82 +250,19 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
                 }
             });
         for (auto& th : pool) th.join();
-        if (bad) { fprintf(stderr, "snpCall: %s\n", first_err.c_str()); if (ctx_thread.joinable()) ctx_thread.join(); msnv_destroy(ctx); return 1; }
+        if (bad) { fprintf(stderr, "snpCall: %s\n", first_err.c_str()); msnv_destroy(ctx); return 1; }
     }
-    BouncePool pool;
     stage("decoders open");
-
-    // MSNV_RAW=0: build the position-aligned layout on the host (the C ABI's other input form) instead of on the device
-    const bool raw_mode = !(getenv("MSNV_RAW") && atoi(getenv("MSNV_RAW")) == 0);
-    std::vector<SampleReads> batch[2];
-    std::vector<RawReads> rbatch[2];
-    if (raw_mode) { rbatch[0].resize(S); rbatch[1].resize(S); } else { batch[0].resize(S); batch[1].resize(S); }
-    struct WindowJob {
-        std::vector<std::thread> pool; std::atomic<uint32_t> next{0}; std::atomic<bool> failed{false};
-        std::mutex mu; std::vector<uint32_t> ready; std::string err; uint32_t n_done = 0;
-        std::vector<msnv_sample_reads> view; std::vector<msnv_raw_reads> rview; std::vector<int> chunk;       // per sample: the staged batch
-    };
-    auto start_window = [&](WindowJob& J, uint32_t k) {
-        const uint32_t lo = k * tiles_per_window * MSNV_TILE, hi = std::min<uint64_t>((uint64_t)(k + 1) * tiles_per_window * MSNV_TILE, layout.n_positions);
-        J.next = 0; J.failed = false; J.ready.clear(); J.err.clear(); J.n_done = 0;
-        J.view.assign(raw_mode ? 0 : S, msnv_sample_reads{}); J.rview.assign(raw_mode ? S : 0, msnv_raw_reads{}); J.chunk.assign(S, -1);
-        for (int t = 0; t < n_threads; ++t)
-            J.pool.emplace_back([&J, &dec, &batch, &rbatch, &pool, raw_mode, k, lo, hi, S]() {
-                auto stage_one = [&](uint32_t s) {
-                    if (raw_mode) J.rview[s] = stage_raw(rbatch[k & 1][s], pool, J.chunk[s]);
-                    else J.view[s] = stage_batch(batch[k & 1][s], pool, J.chunk[s]);
-                };
-                std::vector<uint32_t> deferred;           // decoded while the CUDA context was still coming up: no bounce chunk to copy into yet
-                for (;;) {
-                    const uint32_t s = J.next.fetch_add(1);
-                    if (s >= S) break;
-                    std::string e;
-                    bool good = true;
-                    if (!J.failed) {
-                        if (raw_mode) good = dec[s]->window_raw(lo, (uint32_t)hi, k ? &rbatch[(k - 1) & 1][s] : nullptr, rbatch[k & 1][s], e);
-                        else good = dec[s]->window(lo, (uint32_t)hi, k ? &batch[(k - 1) & 1][s] : nullptr, batch[k & 1][s], e);
-                    }
-                    if (good && !J.failed) {
-                        if (!pool.is_started()) { deferred.push_back(s); continue; }
-                        stage_one(s);
-                    }
-                    std::lock_guard<std::mutex> lk(J.mu);
-                    if (!good) { if (J.err.empty()) J.err = e; J.failed = true; }
-                    J.ready.push_back(s);
-                }
-                for (uint32_t s : deferred) {
-                    pool.wait_started();                  // (or closed: then the batch goes up from the decoder's own arrays)
-                    if (!J.failed) stage_one(s);
-                    std::lock_guard<std::mutex> lk(J.mu);
-                    J.ready.push_back(s);
-                }
-            });
-    };
-
-    // (MSNV_EARLY_DECODE=1: the context may still be coming up here; what is decoded before bounce chunks can be page-locked is
-    // copied into them afterwards)
-    stage("first window starts");
-    const double t_dec0 = now_s();
-    std::unique_ptr<WindowJob> cur(new WindowJob()), nxt;
-    start_window(*cur, 0);
-    if (ctx_thread.joinable()) ctx_thread.join();
     if (dev < 0 || ctx_rc != MSNV_OK) {
         fprintf(stderr, "snpCall: no usable CUDA device (%s); this build has no CPU calling path\n", msnv_last_error(ctx));
-        cur->failed = true; pool.close();
-        for (auto& th : cur->pool) th.join();
         msnv_destroy(ctx);
         return 1;
     }
-    stage("CUDA context created");
-    if (msnv_shard_begin(ctx, S, layout.n_positions, ref.data()) != MSNV_OK) {
-        fprintf(stderr, "snpCall: %s\n", msnv_last_error(ctx));
-        cur->failed = true; pool.close();
-        for (auto& th : cur->pool) th.join();
-        msnv_destroy(ctx); return 1;
-    }
 
+    // bounce chunks are page-locked (that needs only the context) while the first window decodes; a decoding thread whose batch
+    // is ready waits in acquire() for one
+    BouncePool pool;
     std::atomic<bool> stop_pinning(false);
-    pool.start();
     std::thread pinner([&]() {
         size_t n = (size_t)std::min(8.0, std::max(2.0, est_bytes / (double)BouncePool::CHUNK));
         if (const char* e = getenv("MSNV_BOUNCE_CHUNKS")) n = (size_t)std::max(0, atoi(e));
@@ -361,6 +274,44 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
         pool.close();
     });
     struct PinJoin { std::atomic<bool>& stop; std::thread& t; ~PinJoin() { stop = true; if (t.joinable()) t.join(); } } pin_join{stop_pinning, pinner};
+
+    std::vector<RawReads> batch[2];
+    batch[0].resize(S); batch[1].resize(S);
+    struct WindowJob {
+        std::vector<std::thread> pool; std::atomic<uint32_t> next{0}; std::atomic<bool> failed{false};
+        std::mutex mu; std::vector<uint32_t> ready; std::string err; uint32_t n_done = 0;
+        std::vector<msnv_raw_reads> view; std::vector<int> chunk;       // per sample: the staged batch
+    };
+    auto start_window = [&](WindowJob& J, uint32_t k) {
+        const uint32_t lo = k * tiles_per_window * MSNV_TILE, hi = std::min<uint64_t>((uint64_t)(k + 1) * tiles_per_window * MSNV_TILE, layout.n_positions);
+        J.next = 0; J.failed = false; J.ready.clear(); J.err.clear(); J.n_done = 0;
+        J.view.assign(S, msnv_raw_reads{}); J.chunk.assign(S, -1);
+        for (int t = 0; t < n_threads; ++t)
+            J.pool.emplace_back([&J, &dec, &batch, &pool, k, lo, hi, S]() {
+                for (;;) {
+                    const uint32_t s = J.next.fetch_add(1);
+                    if (s >= S) break;
+                    std::string e;
+                    bool good = true;
+                    if (!J.failed) good = dec[s]->window(lo, (uint32_t)hi, k ? &batch[(k - 1) & 1][s] : nullptr, batch[k & 1][s], e);
+                    if (good && !J.failed) J.view[s] = stage_raw(batch[k & 1][s], pool, J.chunk[s]);
+                    std::lock_guard<std::mutex> lk(J.mu);
+                    if (!good) { if (J.err.empty()) J.err = e; J.failed = true; }
+                    J.ready.push_back(s);
+                }
+            });
+    };
+
+    stage("first window starts");
+    const double t_dec0 = now_s();
+    std::unique_ptr<WindowJob> cur(new WindowJob()), nxt;
+    start_window(*cur, 0);
+    if (msnv_shard_begin(ctx, S, layout.n_positions, ref.data()) != MSNV_OK) {
+        fprintf(stderr, "snpCall: %s\n", msnv_last_error(ctx));
+        cur->failed = true; pool.abort();
+        for (auto& th : cur->pool) th.join();
+        msnv_destroy(ctx); return 1;
+    }
     HitWriter w;
     w.pop_out = stdout; w.indiv_out = indiv; w.ann = ann.active() ? &ann : nullptr;
     std::vector<HitWriter::Contig> ctgs;
@@ -401,16 +352,15 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
             for (uint32_t s : got) {
                 const double a = now_s();
                 const uint32_t lib_slot = n_windows > 1 ? slot : 0u;          // (one window: the whole shard, opened by msnv_shard_begin in slot 0)
-                const int arc = raw_mode ? msnv_window_add_sample_raw(ctx, lib_slot, s, &cur->rview[s]) : msnv_window_add_sample(ctx, lib_slot, s, &cur->view[s]);
-                if (arc != MSNV_OK) { fprintf(stderr, "snpCall: %s\n", msnv_last_error(ctx)); rc = 1; break; }
+                if (msnv_window_add_sample_raw(ctx, lib_slot, s, &cur->view[s]) != MSNV_OK) { fprintf(stderr, "snpCall: %s\n", msnv_last_error(ctx)); rc = 1; break; }
                 if (cur->chunk[s] >= 0) in_flight.push_back(cur->chunk[s]);
-                (cur->chunk[s] >= 0 ? h2d_bytes : pageable_bytes) += raw_mode ? rbatch[slot][s].bytes() : batch[slot][s].bytes();
+                (cur->chunk[s] >= 0 ? h2d_bytes : pageable_bytes) += batch[slot][s].bytes();
                 t_add += now_s() - a;
             }
             if (in_flight.size() >= 48 && !recycle()) { rc = 1; break; }
         }
         if (!recycle()) rc = 1;
-        if (rc) { cur->failed = true; pool.close(); }
+        if (rc) { cur->failed = true; pool.abort(); }
         for (auto& th : cur->pool) th.join();
         cur->pool.clear();
         if (cur->failed) { fprintf(stderr, "snpCall: %s\n", cur->err.c_str()); rc = 1; }
@@ -469,11 +419,9 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
     const double t_end = now_s();
     stage("kernels done, output written");
 
-    if (raw_mode) {
-        uint64_t iupac = 0;
-        if (msnv_expand_stats(ctx, &iupac) == MSNV_OK && iupac)
-            fprintf(stderr, "[msnv] %llu read bases are neither A/C/G/T nor N; such bases are not counted\n", (unsigned long long)iupac);
-    }
+    uint64_t iupac = 0;
+    if (msnv_expand_stats(ctx, &iupac) == MSNV_OK && iupac)
+        fprintf(stderr, "[msnv] %llu read bases are neither A/C/G/T nor N; such bases are not counted\n", (unsigned long long)iupac);
     DecodeStats tot;
     uint32_t n_indexed = 0;
     for (uint32_t s = 0; s < S; ++s) {
@@ -490,7 +438,7 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
                     "{\"tool\": \"snpCall\", \"device\": %d, \"samples\": %u, \"positions\": %u, \"windows\": %u, \"bams_read_through_index\": %u, "
                     "\"records\": %llu, \"reads\": %llu, \"aligned_bases\": %llu, \"pairs\": %llu, \"dropped_by_cap\": %llu, "
                     "\"bam_bytes\": %llu, \"bam_bytes_inflated\": %llu, \"h2d_bytes\": %llu, \"h2d_pageable_bytes\": %llu, \"hits\": %llu, "
-                    "\"records_expanded_on_device\": %d, \"decode_threads\": %d, \"decode_wall_s\": %.6f, \"decode_cpu_s\": %.6f, \"inflate_cpu_s\": %.6f, "
+                    "\"decode_threads\": %d, \"decode_wall_s\": %.6f, \"decode_cpu_s\": %.6f, \"inflate_cpu_s\": %.6f, "
                     "\"h2d_s\": %.6f, \"h2d_not_hidden_s\": %.6f, \"waiting_for_decode_s\": %.6f, "
                     "\"gpu_run_wall_s\": %.6f, \"format_s\": %.6f, \"total_s\": %.6f, "
                     "\"ms_index\": %.4f, \"ms_pileup\": %.4f, \"ms_call\": %.4f, \"ms_compact\": %.4f, \"ms_gather\": %.4f, "
@@ -498,7 +446,7 @@ static int run_direct(const Job& job, const msnv_call_params& prm, const std::st
                     dev, S, layout.n_positions, n_windows, n_indexed, (unsigned long long)tot.records, (unsigned long long)tot.accepted,
                     (unsigned long long)tot.aligned_bases, (unsigned long long)tot.pairs, (unsigned long long)tot.dropped_by_cap,
                     (unsigned long long)bam_bytes_total, (unsigned long long)tot.compressed_bytes, (unsigned long long)h2d_bytes,
-                    (unsigned long long)pageable_bytes, (unsigned long long)n_hits_total, raw_mode ? 1 : 0, n_threads * inflate_threads,
+                    (unsigned long long)pageable_bytes, (unsigned long long)n_hits_total, n_threads * inflate_threads,
                     t_dec1 - t_dec0, tot.seconds, tot.inflate_seconds, t_add, t_wait_upload, t_decode_wait, t_run, t_format, t_end - t_start,
                     tm_sum.ms_index, tm_sum.ms_pileup, tm_sum.ms_call, tm_sum.ms_compact, tm_sum.ms_gather, (unsigned long long)items_total,
                     tm_sum.kernel_launches, (unsigned long long)ranges_total);

@@ -121,17 +121,6 @@ std::vector<uint8_t> shard_reference(const ShardLayout& layout, const BamHeader&
 }
 
 // ------------------------------------------------------------------ SoA helpers
-msnv_sample_reads SampleReads::view() const
-{
-    msnv_sample_reads v;
-    memset(&v, 0, sizeof v);
-    v.n_reads = (uint32_t)pos.size();
-    v.max_span = max_span;
-    v.pos = pos.data(); v.seg_off = seg_off.data(); v.q4_off = q4_off.data(); v.mate = mate.data();
-    v.seg_pos = seg_pos.data(); v.seg_len = seg_len.data(); v.seq2 = seq2.data(); v.qual = qual.data();
-    return v;
-}
-
 msnv_raw_reads RawReads::view() const
 {
     msnv_raw_reads v;
@@ -148,16 +137,7 @@ size_t RawReads::bytes() const
     return pos.size() * 8 + seg_off.size() * 4 + q4_off.size() * 4 + raw_off.size() * 4 + n_cigar.size() * 2 + l_seq.size() * 2 + raw.size() * 4;
 }
 
-size_t SampleReads::bytes() const
-{
-    return pos.size() * 4 + seg_off.size() * 4 + q4_off.size() * 4 + mate.size() * 4 + seg_pos.size() * 4 +
-           seg_len.size() * 2 + seq2.size() + qual.size();
-}
-
 namespace {
-
-// BAM 4-bit base code -> 2-bit code (A,C,G,T), or 0x80 (flag, code bits 0) for everything else
-const uint8_t kCode4to2f[16] = {0x80, 0, 1, 0x80, 2, 0x80, 0x80, 0x80, 3, 0x80, 0x80, 0x80, 0x80, 0x80, 0x80, 0x80};
 
 inline uint64_t hash_qname(const char* s)
 {
@@ -188,7 +168,7 @@ struct SampleDecoderState {
     int cur_tid = -1; int32_t last_pos = -1;
     std::priority_queue<Buffered, std::vector<Buffered>, ByEnd> buffered;    // reads the iterator still holds
     std::unordered_map<uint64_t, Stored> olap;                               // qname -> earlier mate waiting for its partner (index = ordinal)
-    bool warned_overhang = false, warned_iupac = false;
+    bool warned_overhang = false;
     uint64_t n_emitted = 0;                      // ordinal of the next accepted read over the whole file
     uint64_t base = 0;                           // ordinal of the first read of the window batch being built
     // index-driven reading: runs of consecutive tids of the shard, visited in order
@@ -248,22 +228,9 @@ static int next_record(SampleDecoderState& S, BamRecord& r)
     }
 }
 
-bool SampleDecoder::window(uint32_t pos_lo, uint32_t pos_hi, const SampleReads* prev, SampleReads& out, std::string& err)
-{
-    return window_impl(pos_lo, pos_hi, prev, &out, nullptr, nullptr, err);
-}
-
-bool SampleDecoder::window_raw(uint32_t pos_lo, uint32_t pos_hi, const RawReads* prev, RawReads& out, std::string& err)
-{
-    return window_impl(pos_lo, pos_hi, nullptr, nullptr, prev, &out, err);
-}
-
-bool SampleDecoder::window_impl(uint32_t pos_lo, uint32_t pos_hi, const SampleReads* prev, SampleReads* out_p, const RawReads* prev_raw, RawReads* out_raw,
-                                std::string& err)
+bool SampleDecoder::window(uint32_t pos_lo, uint32_t pos_hi, const RawReads* prev, RawReads& o, std::string& err)
 {
     SampleDecoderState& S = *st_;
-    SampleReads dummy;
-    SampleReads& out = out_p ? *out_p : dummy;
     const ShardLayout& layout = *S.layout;
     const std::vector<int64_t>& ref_len_of_tid = *S.ref_len;
     DecodeStats& st = S.st;
@@ -272,59 +239,30 @@ bool SampleDecoder::window_impl(uint32_t pos_lo, uint32_t pos_hi, const SampleRe
     const int MAXCNT = 8000;                         // samtools mpileup -d default (>= 1.9), per file
 
     // ---- the previous window's reads that reach this one: a contiguous tail of its batch
-    out = SampleReads();
+    o = RawReads();
     if (prev && !prev->pos.empty()) {
-        const size_t n = prev->pos.size();
+        const RawReads& p = *prev;
+        const size_t n = p.pos.size();
         size_t first = n;
         for (size_t i = n; i-- > 0;) {
-            if ((int64_t)prev->pos[i] + (int64_t)prev->max_span <= (int64_t)pos_lo) break;      // no earlier read can reach the window either
-            const uint32_t k = prev->seg_off[i + 1] - 1;                                         // its last segment
-            if ((int64_t)prev->seg_pos[k] + prev->seg_len[k] > (int64_t)pos_lo) first = i;
+            if ((int64_t)p.pos[i] + (int64_t)p.max_span <= (int64_t)pos_lo) break;          // no earlier read can reach the window either
+            if ((int64_t)p.end[i] > (int64_t)pos_lo) first = i;
         }
         if (first < n) {
-            const uint32_t s0 = prev->seg_off[first], q0 = prev->q4_off[first];
-            out.pos.assign(prev->pos.begin() + first, prev->pos.end());
-            out.seg_off.resize(n - first + 1); out.q4_off.resize(n - first + 1); out.mate.resize(n - first);
-            for (size_t i = first; i <= n; ++i) { out.seg_off[i - first] = prev->seg_off[i] - s0; out.q4_off[i - first] = prev->q4_off[i] - q0; }
-            for (size_t i = first; i < n; ++i) { const int64_t m = (int64_t)prev->mate[i] - (int64_t)first; out.mate[i - first] = m >= 0 ? (int32_t)m : -1; }
-            out.seg_pos.assign(prev->seg_pos.begin() + s0, prev->seg_pos.end());
-            out.seg_len.assign(prev->seg_len.begin() + s0, prev->seg_len.end());
-            out.seq2.assign(prev->seq2.begin() + q0, prev->seq2.end());
-            out.qual.assign(prev->qual.begin() + 4 * (size_t)q0, prev->qual.end());
-            out.max_span = prev->max_span;
+            const uint32_t s0 = p.seg_off[first], q0 = p.q4_off[first], r0 = p.raw_off[first];
+            o.pos.assign(p.pos.begin() + first, p.pos.end());
+            o.end.assign(p.end.begin() + first, p.end.end());
+            o.n_cigar.assign(p.n_cigar.begin() + first, p.n_cigar.end());
+            o.l_seq.assign(p.l_seq.begin() + first, p.l_seq.end());
+            o.seg_off.resize(n - first + 1); o.q4_off.resize(n - first + 1); o.raw_off.resize(n - first + 1); o.mate.resize(n - first);
+            for (size_t i = first; i <= n; ++i) { o.seg_off[i - first] = p.seg_off[i] - s0; o.q4_off[i - first] = p.q4_off[i] - q0; o.raw_off[i - first] = p.raw_off[i] - r0; }
+            for (size_t i = first; i < n; ++i) { const int64_t m = (int64_t)p.mate[i] - (int64_t)first; o.mate[i - first] = m >= 0 ? (int32_t)m : -1; }
+            o.raw.assign(p.raw.begin() + r0, p.raw.end());
+            o.max_span = p.max_span;
         }
         S.base = S.n_emitted - (n - first);
     } else {
         S.base = S.n_emitted;
-    }
-
-    if (out_raw) {
-        RawReads& o = *out_raw;
-        o = RawReads();
-        if (prev_raw && !prev_raw->pos.empty()) {
-            const RawReads& p = *prev_raw;
-            const size_t n = p.pos.size();
-            size_t first = n;
-            for (size_t i = n; i-- > 0;) {
-                if ((int64_t)p.pos[i] + (int64_t)p.max_span <= (int64_t)pos_lo) break;          // no earlier read can reach the window either
-                if ((int64_t)p.end[i] > (int64_t)pos_lo) first = i;
-            }
-            if (first < n) {
-                const uint32_t s0 = p.seg_off[first], q0 = p.q4_off[first], r0 = p.raw_off[first];
-                o.pos.assign(p.pos.begin() + first, p.pos.end());
-                o.end.assign(p.end.begin() + first, p.end.end());
-                o.n_cigar.assign(p.n_cigar.begin() + first, p.n_cigar.end());
-                o.l_seq.assign(p.l_seq.begin() + first, p.l_seq.end());
-                o.seg_off.resize(n - first + 1); o.q4_off.resize(n - first + 1); o.raw_off.resize(n - first + 1); o.mate.resize(n - first);
-                for (size_t i = first; i <= n; ++i) { o.seg_off[i - first] = p.seg_off[i] - s0; o.q4_off[i - first] = p.q4_off[i] - q0; o.raw_off[i - first] = p.raw_off[i] - r0; }
-                for (size_t i = first; i < n; ++i) { const int64_t m = (int64_t)p.mate[i] - (int64_t)first; o.mate[i - first] = m >= 0 ? (int32_t)m : -1; }
-                o.raw.assign(p.raw.begin() + r0, p.raw.end());
-                o.max_span = p.max_span;
-            }
-            S.base = S.n_emitted - (n - first);
-        } else {
-            S.base = S.n_emitted;
-        }
     }
 
     BamRecord r;
@@ -435,110 +373,33 @@ bool SampleDecoder::window_impl(uint32_t pos_lo, uint32_t pos_hi, const SampleRe
                 S.olap.erase(it);
             }
         }
-        if (out_raw) {
-            // ---- BAM-shaped batch: offsets of the aligned layout (the device fills it) and the record's own bytes
-            RawReads& o = *out_raw;
-            size_t quads = 0, q_len = 0;
-            {
-                uint32_t rx = ctg.offset + (uint32_t)c.pos;
-                for (int i = 0; i < c.n_cigar; ++i) {
-                    const uint32_t w = r.cigar_at(i), op = w & 0xf, len = w >> 4;
-                    if (op == CIG_M || op == CIG_EQ || op == CIG_X) { if (len) { quads += ((rx & 3u) + len + 3u) >> 2; st.aligned_bases += len; } rx += len; q_len += len; }
-                    else if (op == CIG_D || op == CIG_N) rx += len;
-                    else if (op == CIG_I || op == CIG_S) q_len += len;
-                }
-            }
-            if (q_len > (size_t)c.l_seq) { err = bam_path + ": read " + r.qname + ": CIGAR longer than the sequence"; return false; }
-            if (o.q4_off.back() + quads > 0xffffffffull) { err = bam_path + ": more than 2^34 bases in one shard of one sample"; return false; }
-            o.pos.push_back((int32_t)(ctg.offset + (uint32_t)c.pos));
-            o.end.push_back((int32_t)(ctg.offset + (uint32_t)end));
-            o.mate.push_back(mate_idx);
-            if (mate_idx >= 0) { o.mate[(size_t)mate_idx] = (int32_t)idx; ++st.pairs; }
-            o.seg_off.push_back(o.seg_off.back() + n_seg);
-            o.q4_off.push_back((uint32_t)(o.q4_off.back() + quads));
-            o.n_cigar.push_back((uint16_t)c.n_cigar);
-            o.l_seq.push_back((uint16_t)c.l_seq);
-            const size_t nb = 4 * (size_t)c.n_cigar + (size_t)((c.l_seq + 1) / 2) + (size_t)c.l_seq, nw = (nb + 3) / 4;
-            const size_t w0 = o.raw.size();
-            o.raw.resize(w0 + nw, 0);
-            memcpy(o.raw.data() + w0, r.cigar, nb);                      // CIGAR, bases and qualities are contiguous in the record
-            o.raw_off.push_back((uint32_t)(w0 + nw));
-            if ((uint32_t)rlen > o.max_span) o.max_span = (uint32_t)rlen;
-            if (st.first_column < 0) {
-                int64_t p = layout.first_inside(slot, c.pos, end);
-                if (p >= 0) st.first_column = (int64_t)ctg.offset + p;
-            }
-            ++st.accepted;
-            continue;
-        }
-        // ---- append to the structure of arrays
-        out.pos.push_back((int32_t)(ctg.offset + (uint32_t)c.pos));
-        out.mate.push_back(mate_idx);
-        if (mate_idx >= 0) { out.mate[(size_t)mate_idx] = (int32_t)idx; ++st.pairs; }
-        out.seg_off.push_back(out.seg_off.back() + n_seg);
-        // every M/=/X operation becomes a segment stored position-aligned (include/msnv.h): byte i of its
-        // quads belongs to shard coordinate (first & ~3) + i; inserted and clipped bases are dropped
-        size_t quads = 0;
+        // ---- offsets of the aligned layout (the device fills it) and the record's own bytes
+        size_t quads = 0, q_len = 0;
         {
-            uint32_t rx = ctg.offset + (uint32_t)c.pos;           // shard coordinate
-            size_t qy = 0;                                        // query index
+            uint32_t rx = ctg.offset + (uint32_t)c.pos;
             for (int i = 0; i < c.n_cigar; ++i) {
                 const uint32_t w = r.cigar_at(i), op = w & 0xf, len = w >> 4;
-                if (op == CIG_M || op == CIG_EQ || op == CIG_X) {
-                    if (len) {
-                        if (qy + len > (size_t)c.l_seq) { err = bam_path + ": read " + r.qname + ": CIGAR longer than the sequence"; return false; }
-                        const uint32_t a = rx & 3u; const size_t nq = (a + len + 3u) >> 2;
-                        const size_t s0 = out.seq2.size(), q0 = out.qual.size();
-                        out.seq2.resize(s0 + nq, 0);
-                        out.qual.resize(q0 + 4 * nq, 0);
-                        uint8_t* sq = out.seq2.data() + s0; uint8_t* ql = out.qual.data() + q0;
-                        // three plain passes instead of one branchy loop: (1) nibbles -> 2-bit code or the "other base"
-                        // flag 0x80, two per sequence byte; (2) qualities capped at 127 plus the flag; (3) four codes per byte
-                        uint8_t cf[MSNV_MAX_READ_BASES + 2];
-                        {
-                            uint32_t k = 0; size_t i2 = qy;
-                            if (i2 & 1) { cf[k++] = kCode4to2f[r.seq[i2 >> 1] & 0xf]; ++i2; }
-                            for (; k + 2 <= len; k += 2, i2 += 2) { const uint8_t b = r.seq[i2 >> 1]; cf[k] = kCode4to2f[b >> 4]; cf[k + 1] = kCode4to2f[b & 0xf]; }
-                            if (k < len) cf[k] = kCode4to2f[r.seq[i2 >> 1] >> 4];
-                        }
-                        const uint8_t* qin = r.qual + qy;
-                        uint8_t any = 0;
-                        for (uint32_t k = 0; k < len; ++k) {
-                            const uint8_t q = qin[k] < 127 ? qin[k] : 127;
-                            ql[a + k] = (uint8_t)(q | (cf[k] & 0x80));
-                            any |= cf[k];
-                        }
-                        {
-                            uint32_t k = 0, o = a;
-                            for (; (o & 3) && k < len; ++k, ++o) sq[o >> 2] |= (uint8_t)((cf[k] & 3) << ((o & 3) * 2));
-                            for (; k + 4 <= len; k += 4, o += 4)
-                                sq[o >> 2] = (uint8_t)((cf[k] & 3) | (cf[k + 1] & 3) << 2 | (cf[k + 2] & 3) << 4 | (cf[k + 3] & 3) << 6);
-                            for (; k < len; ++k, ++o) sq[o >> 2] |= (uint8_t)((cf[k] & 3) << ((o & 3) * 2));
-                        }
-                        if ((any & 0x80) && !S.warned_iupac) {           // rare: is one of the flagged bases something other than N?
-                            for (uint32_t k = 0; k < len; ++k) {
-                                const size_t i2 = qy + k;
-                                const uint8_t c4 = (r.seq[i2 >> 1] >> ((~i2 & 1) << 2)) & 0xf;
-                                if ((cf[k] & 0x80) && c4 != 15) {
-                                    fprintf(stderr, "[msnv] %s: read %s has a base other than A/C/G/T/N; such bases are not counted\n", bam_path.c_str(), r.qname);
-                                    S.warned_iupac = true;
-                                    break;
-                                }
-                            }
-                        }
-                        out.seg_pos.push_back((int32_t)rx);
-                        out.seg_len.push_back((uint16_t)len);
-                        quads += nq;
-                        st.aligned_bases += len;
-                    }
-                    rx += len; qy += len;
-                } else if (op == CIG_D || op == CIG_N) rx += len;
-                else if (op == CIG_I || op == CIG_S) qy += len;
+                if (op == CIG_M || op == CIG_EQ || op == CIG_X) { if (len) { quads += ((rx & 3u) + len + 3u) >> 2; st.aligned_bases += len; } rx += len; q_len += len; }
+                else if (op == CIG_D || op == CIG_N) rx += len;
+                else if (op == CIG_I || op == CIG_S) q_len += len;
             }
         }
-        if (out.q4_off.back() + quads > 0xffffffffull) { err = bam_path + ": more than 2^34 bases in one shard of one sample"; return false; }
-        out.q4_off.push_back((uint32_t)(out.q4_off.back() + quads));
-        if ((uint32_t)rlen > out.max_span) out.max_span = (uint32_t)rlen;
+        if (q_len > (size_t)c.l_seq) { err = bam_path + ": read " + r.qname + ": CIGAR longer than the sequence"; return false; }
+        if (o.q4_off.back() + quads > 0xffffffffull) { err = bam_path + ": more than 2^34 bases in one shard of one sample"; return false; }
+        o.pos.push_back((int32_t)(ctg.offset + (uint32_t)c.pos));
+        o.end.push_back((int32_t)(ctg.offset + (uint32_t)end));
+        o.mate.push_back(mate_idx);
+        if (mate_idx >= 0) { o.mate[(size_t)mate_idx] = (int32_t)idx; ++st.pairs; }
+        o.seg_off.push_back(o.seg_off.back() + n_seg);
+        o.q4_off.push_back((uint32_t)(o.q4_off.back() + quads));
+        o.n_cigar.push_back((uint16_t)c.n_cigar);
+        o.l_seq.push_back((uint16_t)c.l_seq);
+        const size_t nb = 4 * (size_t)c.n_cigar + (size_t)((c.l_seq + 1) / 2) + (size_t)c.l_seq, nw = (nb + 3) / 4;
+        const size_t w0 = o.raw.size();
+        o.raw.resize(w0 + nw, 0);
+        memcpy(o.raw.data() + w0, r.cigar, nb);                      // CIGAR, bases and qualities are contiguous in the record
+        o.raw_off.push_back((uint32_t)(w0 + nw));
+        if ((uint32_t)rlen > o.max_span) o.max_span = (uint32_t)rlen;
         if (st.first_column < 0) {
             int64_t p = layout.first_inside(slot, c.pos, end);
             if (p >= 0) st.first_column = (int64_t)ctg.offset + p;
@@ -549,16 +410,6 @@ bool SampleDecoder::window_impl(uint32_t pos_lo, uint32_t pos_hi, const SampleRe
     st.compressed_bytes = S.rd.compressed_bytes_read();
     st.inflate_seconds = S.rd.inflate_seconds();
     st.seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-    return true;
-}
-
-bool decode_sample_for_pileup(const std::string& bam_path, const ShardLayout& layout, const std::vector<int64_t>& ref_len_of_tid,
-                              int inflate_threads, SampleReads& out, DecodeStats& st, std::string& err)
-{
-    SampleDecoder d;
-    if (!d.open(bam_path, layout, ref_len_of_tid, inflate_threads, std::string(), err)) return false;
-    if (!d.window(0, layout.n_positions, nullptr, out, err)) return false;
-    st = d.stats();
     return true;
 }
 

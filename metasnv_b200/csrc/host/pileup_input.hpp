@@ -46,22 +46,9 @@ struct ShardLayout {
     int64_t first_inside(int slot, int64_t beg, int64_t end) const;
 };
 
-// Growable host-side arrays of one sample, in the layout of msnv_sample_reads.
-struct SampleReads {
-    std::vector<int32_t>  pos;
-    std::vector<uint32_t> seg_off{0}, q4_off{0};
-    std::vector<int32_t>  mate;
-    std::vector<int32_t>  seg_pos;
-    std::vector<uint16_t> seg_len;
-    std::vector<uint8_t>  seq2, qual;
-    uint32_t max_span = 0;
-    msnv_sample_reads view() const;
-    size_t bytes() const;
-};
-
-// The same batch as BAM stores it (msnv_raw_reads): the device walks the CIGARs and packs the bases (expand_kernel), the
-// decoding thread only copies the record's own bytes. `end` (one past the last reference base, shard coordinate) is the
-// host's: it decides which reads a later window still needs.
+// One sample's batch as BAM stores it (msnv_raw_reads): the device walks the CIGARs and packs the bases (expand_kernel),
+// the decoding thread only copies the record's own bytes. `end` (one past the last reference base, shard coordinate) is
+// the host's: it decides which reads a later window still needs.
 struct RawReads {
     std::vector<int32_t>  pos, end, mate;
     std::vector<uint32_t> seg_off{0}, q4_off{0}, raw_off{0};
@@ -87,10 +74,11 @@ struct DecodeStats {
 // coordinates), so neither the host nor the device has to hold a whole shard - the reference's pipe streams the same
 // way (call_vC.cpp:466-479 reads one pileup line at a time). Everything mpileup decides per read in file order
 // (filters, depth cap, mate pairing) carries over from window to window.
-//   window(lo, hi, prev, out): `out` = every accepted read that starts before `hi` and was not finished before `lo`:
-//   first the tail of the previous window's batch `prev` (from its first read that reaches `lo` on; pass nullptr for
-//   the first window), then the reads decoded now. Mate links are indices into `out`; a link whose partner is not in
-//   `out` is dropped (the two then share no position inside the window).
+//   window(lo, hi, prev, out): `out` = every accepted read that starts before `hi` and ends after `lo`: first the tail
+//   of the previous window's batch `prev` (from its first read whose `end` is past `lo` on; pass nullptr for the first
+//   window), then the reads decoded now. Mate links are indices into `out`; a link whose partner is not in `out` is
+//   dropped (the two then share no position inside the window).
+// `ref_len_of_tid[tid]` is the FASTA length of the contig or -1 when the FASTA lacks it (mpileup then keeps every read).
 // With a TidIndex and a -l split the decoder seeks to the runs of contigs the split names instead of inflating the
 // whole file.
 class SampleDecoder {
@@ -101,22 +89,12 @@ public:
     SampleDecoder& operator=(const SampleDecoder&) = delete;
     bool open(const std::string& bam_path, const ShardLayout& layout, const std::vector<int64_t>& ref_len_of_tid, int inflate_threads,
               const std::string& index_hint, std::string& err);
-    bool window(uint32_t pos_lo, uint32_t pos_hi, const SampleReads* prev, SampleReads& out, std::string& err);
-    // the same window as BAM-shaped records (the aligned layout is then built on the device)
-    bool window_raw(uint32_t pos_lo, uint32_t pos_hi, const RawReads* prev, RawReads& out, std::string& err);
+    bool window(uint32_t pos_lo, uint32_t pos_hi, const RawReads* prev, RawReads& out, std::string& err);
     const DecodeStats& stats() const;
     bool used_index() const;
 private:
-    bool window_impl(uint32_t pos_lo, uint32_t pos_hi, const SampleReads* prev, SampleReads* out, const RawReads* prev_raw, RawReads* out_raw, std::string& err);
     SampleDecoderState* st_;
 };
-
-// Decode one BAM into `out` for the contigs of `layout` (one window over the whole shard). `ref_len_of_tid[tid]` is the FASTA length
-// of the contig or -1 when the FASTA lacks it (mpileup then keeps every read). The BAM's header
-// is not compared with the shard's: like mpileup, the first file's header rules.
-bool decode_sample_for_pileup(const std::string& bam_path, const ShardLayout& layout,
-                              const std::vector<int64_t>& ref_len_of_tid, int inflate_threads, SampleReads& out,
-                              DecodeStats& st, std::string& err);
 
 // Reference characters of the shard, one byte per shard coordinate: the FASTA character where the
 // contig has one and the position is inside the shard's intervals, 'N' inside the intervals but

@@ -8,7 +8,9 @@ numpy_counts()    recounts one sample from the structure-of-arrays batch of incl
                   both mates of a pair cover are corrected by htslib's tweak_overlap_quality (Annex A.2): equal bases ->
                   the earlier read gets min(qa+qb, 127... htslib: 200) and the later one 0; different bases -> the better one keeps
                   int(0.8*q), the other 0, ties go to the earlier read.
-decode_dump()     runs bin/msnv_decode_dump and loads the batches it writes.
+decode_dump()     runs bin/msnv_decode_dump and loads the batches it writes: the decoder's BAM-shaped records expanded
+                  on the host into that layout, and with raw=True the records themselves (expand_raw() restates the
+                  expansion in Python).
 """
 import json
 import os

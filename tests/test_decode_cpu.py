@@ -1,6 +1,7 @@
 """CPU tests of the host BAM decoder (csrc/host/pileup_input.cc) and of the data layout of include/msnv.h:
-`bin/msnv_decode_dump` writes the batches `snpCall` would upload; their structural invariants are checked and a
-numpy recount of every sample (tests/pileup_counts.py) must equal the counts of the oracle's mpileup text.
+`bin/msnv_decode_dump` writes the batches `snpCall` uploads, expanded on the host into the aligned layout; their structural
+invariants are checked and a numpy recount of every sample (tests/pileup_counts.py) must equal the counts of the oracle's
+mpileup text.
 This covers, without a GPU, everything upstream of the kernels: mpileup's read filters, the depth cap, the overlap
 pairing, the position-aligned segments with their zero padding, the reads carried from one position window to the
 next, and the limits on read length and reference span."""
@@ -86,7 +87,8 @@ def test_decoder_batches_recount_to_the_oracle_text(preset, scale, samples, data
     """Synthetic sets, the edge set of tests/golden/edge_set.py (255 reads on one position in 270 samples, 250..260 reads
     on one tile, 1200x from one BAM, overlapping mates whose corrected qualities land on 12 and 13, reads of 4096 bases
     (one in 128 segments) at both ends of a contig whose length is not a multiple of 4), and the span set of
-    tests/golden/span_set.py (reads of up to 32768 reference positions, in both of the decoder's output forms)."""
+    tests/golden/span_set.py (reads of up to 32768 reference positions; there the BAM-shaped records are also expanded by the
+Python restatement of expand_kernel)."""
     if preset == "edge":
         data = write_edge_set(str(tmp_path / "edge"))
     elif preset == "span":
@@ -150,9 +152,9 @@ def test_decoder_hand_written_cases(sams, pile, built, tmp_path):
 
 
 def test_bam_shaped_batches_expand_to_the_aligned_layout(built, tmp_path):
-    """The decoder's other output form - reads as BAM stores them, expanded on the device by expand_kernel - against the
-    aligned layout the decoder builds itself, through a plain-Python restatement of the expansion: hand-written cases
-    (indels, clips, =/X/P/N/H operations, N bases, one-base segments) and a small synthetic set."""
+    """The decoder's batches - reads as BAM stores them, expanded on the device by expand_kernel - through two independent
+    restatements of that expansion, msnv_decode_dump's host expansion and a plain-Python one, which must agree byte for
+    byte: hand-written cases (indels, clips, =/X/P/N/H operations, N bases, one-base segments) and a small synthetic set."""
     tmp = str(tmp_path)
     bams = []
     for s in ("s1", "s2", "s4_ops", "s3_refskip", "s5_rules", "s6_leading_del"):
@@ -208,7 +210,7 @@ WINDOW_TILES = [1, 3, 7]
 
 @pytest.fixture(scope="module")
 def span_data(built, tmp_path_factory):
-    """The span set, the decoder's whole-shard batches of it (both forms) and the oracle's counts."""
+    """The span set, the decoder's whole-shard batches of it (expanded on the host) and the oracle's counts."""
     d = str(tmp_path_factory.mktemp("span"))
     data = span_set.write_span_set(os.path.join(d, "set"))
     lay, whole = decode_dump(os.path.join(data, "ref.fa"), os.path.join(data, "all_samples"), os.path.join(d, "dump"))
@@ -226,10 +228,10 @@ def _read_keys(e, idx):
 
 @pytest.mark.parametrize("win_tiles", WINDOW_TILES)
 def test_windowed_decoder_batches_recount_to_the_oracle(win_tiles, span_data, tmp_path):
-    """snpCall decodes a shard window by window, and SampleDecoder::window / window_raw carry the reads of the previous
-    window that reach the next one. On the span set cut into windows of 1, 3 and 7 tiles (a read of span 32768 crosses up
-    to 33 of them), each window's batch, in both forms, recounts to the oracle's counts over that window's positions, and
-    holds every read that abi.window_slice offers the window and that touches it."""
+    """snpCall decodes a shard window by window, and SampleDecoder::window carries the reads of the previous window that
+    reach the next one. On the span set cut into windows of 1, 3 and 7 tiles (a read of span 32768 crosses up to 33 of
+    them), each window's batch, expanded on the host and by the Python restatement, recounts to the oracle's counts over
+    that window's positions, and holds every read that abi.window_slice offers the window and that touches it."""
     from collections import Counter
     data, lay0, whole, want = span_data
     T, P = lay0["tile"], lay0["n_positions"]

@@ -289,7 +289,7 @@ def test_full_size_shard_counts_recount_with_numpy(built):
 
 def test_expand_kernel_builds_the_aligned_layout(built, tmp_path):
     """Reads handed over as BAM stores them (msnv_window_add_sample_raw): expand_kernel must build, byte for byte, the
-    position-aligned arrays the host decoder builds itself (and that tests/test_decode_cpu.py pins against the oracle):
+    position-aligned arrays of msnv_decode_dump's host expansion (which tests/test_decode_cpu.py pins against the oracle):
     hand-written CIGAR cases and a synthetic set with indels, clips and N bases. Then the calls must be the same too."""
     import json
     from metasnv_b200 import abi

@@ -63,11 +63,11 @@ def _same(a, b):
 
 
 # the library's choice; both pileup forms, also with the smallest stages (16 reads, one 4096-base read of quads); both
-# search paths of the index; the layout built on the host; 256 consumer threads
+# search paths of the index; 256 consumer threads
 COUNT_FORMS = [{}, {"MSNV_PILEUP": "scatter"}, {"MSNV_PILEUP": "gather"},
                {"MSNV_PILEUP": "scatter", "MSNV_MAX_READS": "16", "MSNV_CHUNK_Q4": "1280"},
                {"MSNV_PILEUP": "gather", "MSNV_MAX_READS": "16", "MSNV_CHUNK_Q4": "1280"},
-               {"MSNV_INDEX_BITMAP": "0"}, {"MSNV_INDEX_BITMAP": "1"}, {"MSNV_RAW": "0"}, {"MSNV_CONSUMERS": "256"}]
+               {"MSNV_INDEX_BITMAP": "0"}, {"MSNV_INDEX_BITMAP": "1"}, {"MSNV_CONSUMERS": "256"}]
 
 
 @pytest.mark.parametrize("env", COUNT_FORMS, ids=lambda e: "-".join("%s=%s" % kv for kv in e.items()) or "library")
