@@ -27,6 +27,7 @@
 
 #include "../../../include/msnv.h"
 #include "../host/pileup_input.hpp"
+#include "../host/sample_layout.hpp"
 #include "../host/snp_output.hpp"
 #include "../host/text_pileup.hpp"
 
@@ -117,34 +118,28 @@ private:
     void maybe_free(int id) { if (chunks[id].sealed && chunks[id].pending == 0) { chunks[id].sealed = false; chunks[id].used = 0; free_ids.push_back(id); } }
 };
 
-// offsets of consecutive arrays inside one block: the rule the library uses for its device blocks (msnv_gpu.cu), so that a batch
-// packed this way goes up in one or two copies instead of eight
-static size_t pack_step(size_t& off, size_t bytes) { const size_t o = off; off = (off + bytes + 32 + 255) & ~(size_t)255; return o; }
-
-// one sample's batch as the library wants it: copied into a bounce chunk when it fits one (else the decoder's own arrays)
+// one sample's batch as the library wants it: copied into a bounce chunk when it fits one (else the decoder's own arrays),
+// packed by the library's block layout so that each group goes up in one copy
 static msnv_raw_reads stage_raw(const RawReads& r, BouncePool& pool, int& chunk)
 {
     msnv_raw_reads v = r.view();
     chunk = -1;
     if (v.n_reads == 0) return v;
-    size_t off = 0;
-    const size_t o_pos = pack_step(off, r.pos.size() * 4), o_sgo = pack_step(off, r.seg_off.size() * 4), o_q4 = pack_step(off, r.q4_off.size() * 4),
-                 o_mate = pack_step(off, r.mate.size() * 4);
-    size_t off2 = 0;                                       // second group: what the library stages for expand_kernel
-    const size_t s_off = pack_step(off2, r.raw_off.size() * 4), s_raw = pack_step(off2, r.raw.size() * 4), s_nc = pack_step(off2, r.n_cigar.size() * 2),
-                 s_ls = pack_step(off2, r.l_seq.size() * 2);
-    uint8_t* p = pool.acquire(off + off2, chunk);
+    BlockLayout reads, records;
+    const ReadGroup g(reads, r.pos.size());
+    const RawGroup x(records, r.pos.size(), r.raw.size());
+    uint8_t* p = pool.acquire(reads.size + records.size, chunk);
     if (!p) return v;
-    uint8_t* p2 = p + off;
+    uint8_t* p2 = p + reads.size;
     auto put = [&](uint8_t* base, size_t o, const void* src, size_t bytes) { memcpy(base + o, src, bytes); return base + o; };
-    v.pos = (const int32_t*)put(p, o_pos, r.pos.data(), r.pos.size() * 4);
-    v.seg_off = (const uint32_t*)put(p, o_sgo, r.seg_off.data(), r.seg_off.size() * 4);
-    v.q4_off = (const uint32_t*)put(p, o_q4, r.q4_off.data(), r.q4_off.size() * 4);
-    v.mate = (const int32_t*)put(p, o_mate, r.mate.data(), r.mate.size() * 4);
-    v.raw_off = (const uint32_t*)put(p2, s_off, r.raw_off.data(), r.raw_off.size() * 4);
-    v.raw = put(p2, s_raw, r.raw.data(), r.raw.size() * 4);
-    v.n_cigar = (const uint16_t*)put(p2, s_nc, r.n_cigar.data(), r.n_cigar.size() * 2);
-    v.l_seq = (const uint16_t*)put(p2, s_ls, r.l_seq.data(), r.l_seq.size() * 2);
+    v.pos = (const int32_t*)put(p, g.pos, r.pos.data(), r.pos.size() * 4);
+    v.seg_off = (const uint32_t*)put(p, g.seg_off, r.seg_off.data(), r.seg_off.size() * 4);
+    v.q4_off = (const uint32_t*)put(p, g.q4_off, r.q4_off.data(), r.q4_off.size() * 4);
+    v.mate = (const int32_t*)put(p, g.mate, r.mate.data(), r.mate.size() * 4);
+    v.raw_off = (const uint32_t*)put(p2, x.raw_off, r.raw_off.data(), r.raw_off.size() * 4);
+    v.raw = put(p2, x.raw, r.raw.data(), r.raw.size() * 4);
+    v.n_cigar = (const uint16_t*)put(p2, x.n_cigar, r.n_cigar.data(), r.n_cigar.size() * 2);
+    v.l_seq = (const uint16_t*)put(p2, x.l_seq, r.l_seq.data(), r.l_seq.size() * 2);
     return v;
 }
 

@@ -21,8 +21,69 @@
 #include "inflate_kernels.cuh"
 #include "kernels.cuh"
 #include "synth_kernels.cuh"
+#include "../host/sample_layout.hpp"
 
 using namespace msnv_gpu;
+using msnv::BlockLayout; using msnv::ReadGroup; using msnv::SegmentGroup; using msnv::RawGroup;
+
+// A block of device (cudaMalloc) or pinned host (cudaMallocHost) memory that this object owns, with its capacity in
+// elements. ensure() frees the old block before it allocates the new one, so growing never holds both. A failed
+// allocation leaves the buffer empty and clears the runtime's last error: the caller reports it, and a later call that
+// needs the buffer allocates it again.
+template <class T, cudaError_t (*Alloc)(void**, size_t), cudaError_t (*Free)(void*)>
+struct Buf {
+    T* p = nullptr;
+    uint64_t cap = 0;
+    Buf() = default;
+    Buf(const Buf&) = delete;
+    Buf& operator=(const Buf&) = delete;
+    ~Buf() { reset(); }
+    operator T*() const { return p; }
+    void reset() { if (p) Free(p); p = nullptr; cap = 0; }
+    // room for n elements; `want` (>= n) of them when it has to grow. With `keep` the first keep elements survive: the
+    // new block is then allocated and filled before the old one is freed (pinned memory only).
+    cudaError_t ensure(uint64_t n, uint64_t want, uint64_t keep = 0)
+    {
+        if (n <= cap) return cudaSuccess;
+        if (!keep) reset();
+        T* q = nullptr;
+        const cudaError_t e = Alloc((void**)&q, (size_t)want * sizeof(T));
+        if (e != cudaSuccess) { cudaGetLastError(); reset(); return e; }
+        if (keep) memcpy(q, p, (size_t)keep * sizeof(T));
+        reset();
+        p = q; cap = want;
+        return cudaSuccess;
+    }
+    cudaError_t ensure(uint64_t n) { return ensure(n, n); }
+};
+template <class T> using DevBuf = Buf<T, cudaMalloc, cudaFree>;
+template <class T> using PinnedBuf = Buf<T, cudaMallocHost, cudaFreeHost>;
+
+// f(a.pos, b.pos, ..., w) for each of the six arrays of the hit sets a, b, ...; w is the array's elements per hit
+template <class F, class... H>
+void each_hit_array(uint64_t S, F f, H&... h)
+{
+    f(h.pos..., 1); f(h.total..., 5); f(h.pop..., 1); f(h.ind..., 1); f(h.cov..., S); f(h.allele..., 4 * S);
+}
+
+// The called positions as six parallel arrays: position, totals, population and individual masks, and per sample the
+// coverage and the allele counts. One set on the device holds the hits of a range, one pinned set those of a window.
+template <template <class> class B>
+struct HitArrays {
+    B<uint32_t> pos, total; B<uint8_t> pop, ind; B<uint16_t> cov, allele;
+    // room for n hits of S samples, `cap` hits when it grows; the first `keep` hits survive the growth (pinned sets).
+    // Without hits to keep every old block is freed before the first new one is allocated.
+    cudaError_t ensure(uint64_t n, uint64_t S, uint64_t cap, uint64_t keep = 0)
+    {
+        bool fits = true;
+        each_hit_array(S, [&](auto& b, uint64_t w) { fits = fits && n * w <= b.cap; }, *this);
+        if (fits) return cudaSuccess;
+        if (!keep) each_hit_array(S, [](auto& b, uint64_t) { b.reset(); }, *this);
+        cudaError_t e = cudaSuccess;
+        each_hit_array(S, [&](auto& b, uint64_t w) { if (e == cudaSuccess) e = b.ensure(n * w, cap * w, keep * w); }, *this);
+        return e;
+    }
+};
 
 constexpr int N_SLOTS = 2;
 
@@ -42,8 +103,8 @@ struct msnv_ctx {
         std::vector<msnv_sample_sizes> sizes;       // [S]
         std::vector<Block> allocs;                  // device blocks holding the samples
         uint64_t n_reads = 0, n_bases = 0, n_segs = 0;
-        SampleDev* d_samples = nullptr; uint32_t cap_samples = 0;
-        unsigned long long* d_aligned = nullptr; uint32_t cap_aligned = 0; bool has_raw = false;     // aligned bases per sample (samples expanded on the device)
+        DevBuf<SampleDev> d_samples;
+        DevBuf<unsigned long long> d_aligned; bool has_raw = false;     // aligned bases per sample (samples expanded on the device)
         cudaEvent_t uploaded = nullptr;
     };
 
@@ -54,67 +115,59 @@ struct msnv_ctx {
     std::vector<Block> pool;            // blocks of finished windows / shards, reused by later ones
     std::vector<Slab> slabs;            // small blocks are carved out of large allocations
     uint64_t gen = 0;                   // counts msnv_window_begin calls: pool entries unused for a while are freed
-    uint8_t* d_ref = nullptr;
-    uint8_t* d_expect = nullptr;        // expected letter per position (derived from d_ref)
+    DevBuf<uint8_t> d_ref;
+    DevBuf<uint8_t> d_expect;           // expected letter per position (derived from d_ref)
 
     // ---- work buffers (grown on demand, kept across windows and shards)
-    Item* d_items = nullptr;        uint64_t cap_items = 0;
-    uint8_t* d_tiles = nullptr;     uint64_t cap_tile_slots = 0;    // count planes, SLOT_BYTES per item of a range
-    uint64_t* d_text_acgt = nullptr; uint16_t* d_text_match = nullptr; uint64_t cap_text = 0;   // classic text mode staging
+    DevBuf<Item> d_items;
+    DevBuf<uint8_t> d_tiles;            // count planes, SLOT_BYTES per item of a range
+    DevBuf<uint64_t> d_text_acgt; DevBuf<uint16_t> d_text_match;   // classic text mode staging
     int sm_count = 0;
-    uint32_t* d_tile_begin = nullptr; uint32_t* d_tile_hits = nullptr; uint8_t* d_flags = nullptr; uint64_t cap_tiles = 0;
+    DevBuf<uint32_t> d_tile_begin, d_tile_hits; DevBuf<uint8_t> d_flags;
     std::vector<uint32_t> h_tile_begin;
-    uint32_t* d_block_sums = nullptr; uint64_t cap_blocks = 0;
-    uint2* d_range_cache = nullptr;   uint64_t cap_range = 0;
-    uint32_t* d_bitmap = nullptr;     uint64_t cap_bitmap = 0;
-    uint32_t* d_scalar = nullptr;   int* d_err = nullptr;
-    uint32_t* d_fix_list = nullptr;   uint64_t cap_fix_list = 0;        // samples with mate links
+    DevBuf<uint32_t> d_block_sums;
+    DevBuf<uint2> d_range_cache;
+    DevBuf<uint32_t> d_bitmap;
+    DevBuf<uint32_t> d_scalar; DevBuf<int> d_err;
+    DevBuf<uint32_t> d_fix_list;        // samples with mate links
     // raw (BAM-shaped) reads of the sample being expanded: one staging buffer, reused in stream order
-    uint8_t* d_raw = nullptr;         uint64_t cap_raw = 0;
-    unsigned long long* d_xstat = nullptr;       // [0] IUPAC bases seen by expand_kernel, [1] inconsistent record flag
+    DevBuf<uint8_t> d_raw;
+    DevBuf<unsigned long long> d_xstat;  // [0] IUPAC bases seen by expand_kernel, [1] inconsistent record flag
     // what msnv_shard_counts can still look at: the last range of the last run
     uint32_t last_slot = 0, last_item0 = 0, last_ta = 0, last_tb = 0;
 
     // ---- hits: device buffers for one range, pinned host arrays for the whole window
-    uint64_t cap_dhits = 0, cap_dhits_S = 0, cap_hhits = 0, cap_hhits_S = 0;
-    uint32_t *d_hit_pos = nullptr, *d_hit_total = nullptr; uint8_t *d_hit_pop = nullptr, *d_hit_ind = nullptr;
-    uint16_t *d_hit_cov = nullptr, *d_hit_allele = nullptr;
-    uint32_t *h_hit_pos = nullptr, *h_hit_total = nullptr; uint8_t *h_hit_pop = nullptr, *h_hit_ind = nullptr;
-    uint16_t *h_hit_cov = nullptr, *h_hit_allele = nullptr;
-    uint32_t* h_scalar = nullptr;   // pinned, 8 words
+    HitArrays<DevBuf> d_hits;
+    HitArrays<PinnedBuf> h_hits;
+    PinnedBuf<uint32_t> h_scalar;       // 8 words
 
     // coverage pass: work buffers grown on demand and kept (one call per BAM, hundreds of calls per job)
-    int32_t* d_cov_diff = nullptr; uint64_t cap_cov_diff = 0;
-    uint32_t* d_cov_beg = nullptr; uint32_t* d_cov_end = nullptr; uint64_t cap_cov_blocks = 0;
-    uint32_t* d_cov_meta = nullptr; uint64_t cap_cov_meta = 0;          // chunk0 | chunk_contig | contig_len | blk_off (as 2 words each)
-    unsigned long long* d_cov_out = nullptr; uint64_t cap_cov_out = 0;  // cov_sum | hist
+    DevBuf<int32_t> d_cov_diff;
+    DevBuf<uint32_t> d_cov_beg, d_cov_end;
+    DevBuf<uint32_t> d_cov_meta;        // chunk0 | chunk_contig | contig_len | blk_off (as 2 words each)
+    DevBuf<unsigned long long> d_cov_out;  // cov_sum | hist
     cudaEvent_t ev[8] = {};
     msnv_timings tm = {};
 };
 
 namespace {
 
-int fail(msnv_ctx* c, int code, const char* fmt, ...)
+// records the error on a context or an inflater and returns `code`
+template <class Obj>
+int fail(Obj* o, int code, const char* fmt, ...)
 {
     char buf[512];
     va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
-    if (c) c->err = buf;
+    if (o) o->err = buf;
     return code;
 }
 
+// (the object the error is recorded on is `ctx`, a context or an inflater)
 #define CU(call)                                                                                         \
     do {                                                                                                 \
         cudaError_t e_ = (call);                                                                         \
         if (e_ != cudaSuccess) return fail(ctx, MSNV_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
-
-template <class T>
-int grow(msnv_ctx* ctx, T*& p, uint64_t n)
-{
-    if (p) { CU(cudaFree(p)); p = nullptr; }
-    CU(cudaMalloc((void**)&p, (size_t)(n ? n : 1) * sizeof(T)));
-    return 0;
-}
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -185,51 +238,6 @@ void* take_block(msnv_ctx* ctx, msnv_ctx::Window& w, size_t bytes)
     return p;
 }
 
-// device buffers for the hits of one range
-int ensure_dev_hits(msnv_ctx* ctx, uint64_t n_hits)
-{
-    const uint64_t S = ctx->S;
-    if (n_hits <= ctx->cap_dhits && n_hits * S <= ctx->cap_dhits_S) return 0;
-    const uint64_t cap = n_hits + n_hits / 4 + 1024;
-    cudaFree(ctx->d_hit_pos); cudaFree(ctx->d_hit_total); cudaFree(ctx->d_hit_pop); cudaFree(ctx->d_hit_ind);
-    cudaFree(ctx->d_hit_cov); cudaFree(ctx->d_hit_allele);
-    ctx->d_hit_pos = ctx->d_hit_total = nullptr; ctx->d_hit_pop = ctx->d_hit_ind = nullptr; ctx->d_hit_cov = ctx->d_hit_allele = nullptr;
-    ctx->cap_dhits = ctx->cap_dhits_S = 0;
-    CU(cudaMalloc((void**)&ctx->d_hit_pos, cap * 4));
-    CU(cudaMalloc((void**)&ctx->d_hit_total, cap * 20));
-    CU(cudaMalloc((void**)&ctx->d_hit_pop, cap));
-    CU(cudaMalloc((void**)&ctx->d_hit_ind, cap));
-    CU(cudaMalloc((void**)&ctx->d_hit_cov, cap * S * 2));
-    CU(cudaMalloc((void**)&ctx->d_hit_allele, cap * S * 8));
-    ctx->cap_dhits = cap; ctx->cap_dhits_S = cap * S;
-    return 0;
-}
-
-// pinned host arrays for the hits of the whole window; `keep` hits already stored survive the growth
-int ensure_host_hits(msnv_ctx* ctx, uint64_t n_hits, uint64_t keep)
-{
-    const uint64_t S = ctx->S;
-    if (n_hits <= ctx->cap_hhits && n_hits * S <= ctx->cap_hhits_S) return 0;
-    const uint64_t cap = n_hits + n_hits / 2 + 1024;
-    uint32_t *pos = nullptr, *total = nullptr; uint8_t *pop = nullptr, *ind = nullptr; uint16_t *cov = nullptr, *allele = nullptr;
-    CU(cudaMallocHost((void**)&pos, cap * 4));
-    CU(cudaMallocHost((void**)&total, cap * 20));
-    CU(cudaMallocHost((void**)&pop, cap));
-    CU(cudaMallocHost((void**)&ind, cap));
-    CU(cudaMallocHost((void**)&cov, cap * S * 2));
-    CU(cudaMallocHost((void**)&allele, cap * S * 8));
-    if (keep) {
-        memcpy(pos, ctx->h_hit_pos, keep * 4); memcpy(total, ctx->h_hit_total, keep * 20);
-        memcpy(pop, ctx->h_hit_pop, keep); memcpy(ind, ctx->h_hit_ind, keep);
-        memcpy(cov, ctx->h_hit_cov, keep * S * 2); memcpy(allele, ctx->h_hit_allele, keep * S * 8);
-    }
-    cudaFreeHost(ctx->h_hit_pos); cudaFreeHost(ctx->h_hit_total); cudaFreeHost(ctx->h_hit_pop); cudaFreeHost(ctx->h_hit_ind);
-    cudaFreeHost(ctx->h_hit_cov); cudaFreeHost(ctx->h_hit_allele);
-    ctx->h_hit_pos = pos; ctx->h_hit_total = total; ctx->h_hit_pop = pop; ctx->h_hit_ind = ind; ctx->h_hit_cov = cov; ctx->h_hit_allele = allele;
-    ctx->cap_hhits = cap; ctx->cap_hhits_S = cap * S;
-    return 0;
-}
-
 // count-plane slots one range may use: what the device has free (less a reserve), or MSNV_TILE_BUDGET_MB
 uint64_t tile_budget_slots(msnv_ctx* ctx)
 {
@@ -238,7 +246,7 @@ uint64_t tile_budget_slots(msnv_ctx* ctx)
     else {
         size_t fr = 0, tot = 0;
         if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { cudaGetLastError(); fr = (size_t)8 << 30; }
-        fr += (size_t)ctx->cap_tile_slots * SLOT_BYTES;        // what the buffer holds already is ours to use
+        fr += ctx->d_tiles.cap;                                 // what the buffer holds already is ours to use
         // the called positions of a range need buffers too (10 bytes per hit and sample): a third of what is free stays for them
         const size_t reserve = (size_t)2 << 30;
         budget = fr > 3 * reserve ? (fr - reserve) / 3 * 2 : fr / 2;
@@ -248,29 +256,17 @@ uint64_t tile_budget_slots(msnv_ctx* ctx)
 
 int ensure_tile_slots(msnv_ctx* ctx, uint64_t n)
 {
-    if (n <= ctx->cap_tile_slots) return 0;
-    cudaFree(ctx->d_tiles); ctx->d_tiles = nullptr; ctx->cap_tile_slots = 0;
-    uint64_t cap = n + n / 16 + 16;
-    if (cudaMalloc((void**)&ctx->d_tiles, cap * SLOT_BYTES) != cudaSuccess) {
-        cudaGetLastError();
-        cap = n;
-        if (cudaMalloc((void**)&ctx->d_tiles, cap * SLOT_BYTES) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(ctx, MSNV_E_NOMEM, "count planes for %llu (sample, tile) items do not fit device memory", (unsigned long long)n);
-        }
-    }
-    ctx->cap_tile_slots = cap;
-    return 0;
+    if (ctx->d_tiles.ensure(n * SLOT_BYTES, (n + n / 16 + 16) * SLOT_BYTES) != cudaSuccess && ctx->d_tiles.ensure(n * SLOT_BYTES) != cudaSuccess)
+        return fail(ctx, MSNV_E_NOMEM, "count planes for %llu (sample, tile) items do not fit device memory", (unsigned long long)n);
+    return MSNV_OK;
 }
 
 int ensure_window_buffers(msnv_ctx* ctx, uint32_t n_tiles_w)
 {
-    if ((uint64_t)n_tiles_w + 1 <= ctx->cap_tiles) return 0;
-    if (grow(ctx, ctx->d_tile_begin, (uint64_t)n_tiles_w + 1)) return MSNV_E_CUDA;
-    if (grow(ctx, ctx->d_tile_hits, (uint64_t)n_tiles_w + 1)) return MSNV_E_CUDA;
-    if (grow(ctx, ctx->d_flags, (uint64_t)n_tiles_w * TILE)) return MSNV_E_CUDA;
-    ctx->cap_tiles = (uint64_t)n_tiles_w + 1;
-    return 0;
+    CU(ctx->d_tile_begin.ensure((uint64_t)n_tiles_w + 1));
+    CU(ctx->d_tile_hits.ensure((uint64_t)n_tiles_w + 1));
+    CU(ctx->d_flags.ensure((uint64_t)n_tiles_w * TILE));
+    return MSNV_OK;
 }
 
 }  // namespace
@@ -380,31 +376,31 @@ static int call_range(msnv_ctx* ctx, const msnv_ctx::Window& w, uint32_t a, uint
     if (ctx->h_scalar[6]) return fail(ctx, MSNV_E_LIMIT, "a read exceeds MSNV_MAX_READ_BASES / MSNV_MAX_READ_SEGMENTS, or its offsets and segments disagree");
     const uint32_t n_hits = ctx->h_scalar[1];
     n_range = n_hits;
-    if (ensure_dev_hits(ctx, n_hits)) return MSNV_E_CUDA;
-    if (ensure_host_hits(ctx, (uint64_t)n_before + n_hits, n_before)) return MSNV_E_CUDA;
+    const uint64_t n_window = (uint64_t)n_before + n_hits;
+    CU(ctx->d_hits.ensure(n_hits, S, (uint64_t)n_hits + n_hits / 4 + 1024));
+    CU(ctx->h_hits.ensure(n_window, S, n_window + n_window / 2 + 1024, n_before));
+    HitArrays<DevBuf>& d = ctx->d_hits;
     if (n_hits) {
-        compact_kernel<<<nt, TILE, 0, st>>>(ctx->d_flags + (size_t)ta * TILE, ctx->d_tile_hits + ta, w.t0 + ta, ctx->d_hit_pos, ctx->d_hit_pop, ctx->d_hit_ind);
+        compact_kernel<<<nt, TILE, 0, st>>>(ctx->d_flags + (size_t)ta * TILE, ctx->d_tile_hits + ta, w.t0 + ta, d.pos, d.pop, d.ind);
         ++launches;
     }
     CU(cudaEventRecord(ctx->ev[5], st));
 
     // ---- per-hit, per-sample numbers for the formatter
     if (n_hits) {
-        CU(cudaMemsetAsync(ctx->d_hit_cov, 0, (size_t)n_hits * S * 2, st));
-        CU(cudaMemsetAsync(ctx->d_hit_allele, 0, (size_t)n_hits * S * 8, st));
-        gather_kernel<<<n_hits, 128, 0, st>>>(ctx->d_tiles, ctx->d_items, a, ctx->d_tile_begin, w.t0, ctx->d_ref, ctx->d_expect, ctx->d_hit_pos, S,
-                                               text_mode, ctx->d_hit_cov, ctx->d_hit_allele, ctx->d_hit_total);
+        CU(cudaMemsetAsync(d.cov, 0, (size_t)n_hits * S * 2, st));
+        CU(cudaMemsetAsync(d.allele, 0, (size_t)n_hits * S * 8, st));
+        gather_kernel<<<n_hits, 128, 0, st>>>(ctx->d_tiles, ctx->d_items, a, ctx->d_tile_begin, w.t0, ctx->d_ref, ctx->d_expect, d.pos, S,
+                                               text_mode, d.cov, d.allele, d.total);
         ++launches;
     }
     CU(cudaEventRecord(ctx->ev[6], st));
     if (n_hits) {
-        const size_t o = n_before;
-        CU(cudaMemcpyAsync(ctx->h_hit_pos + o, ctx->d_hit_pos, (size_t)n_hits * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(ctx->h_hit_total + o * 5, ctx->d_hit_total, (size_t)n_hits * 20, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(ctx->h_hit_pop + o, ctx->d_hit_pop, n_hits, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(ctx->h_hit_ind + o, ctx->d_hit_ind, n_hits, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(ctx->h_hit_cov + o * S, ctx->d_hit_cov, (size_t)n_hits * S * 2, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(ctx->h_hit_allele + o * S * 4, ctx->d_hit_allele, (size_t)n_hits * S * 8, cudaMemcpyDeviceToHost, st));
+        cudaError_t e = cudaSuccess;
+        each_hit_array(S, [&](auto& h, auto& dv, uint64_t k) {
+            if (e == cudaSuccess) e = cudaMemcpyAsync(h.p + n_before * k, dv.p, n_hits * k * sizeof *dv.p, cudaMemcpyDeviceToHost, st);
+        }, ctx->h_hits, d);
+        if (e != cudaSuccess) return fail(ctx, MSNV_E_CUDA, "copy of the hits to the host failed: %s", cudaGetErrorString(e));
     }
     CU(cudaEventRecord(ctx->ev[7], st));
     CU(cudaStreamSynchronize(st));
@@ -421,8 +417,8 @@ static void publish_hits(msnv_ctx* ctx, uint32_t n_hits, msnv_hits* hits)
 {
     hits->n_hits = n_hits;
     hits->n_samples = ctx->S;
-    hits->pos = ctx->h_hit_pos; hits->pop_mask = ctx->h_hit_pop; hits->ind_mask = ctx->h_hit_ind;
-    hits->cov = ctx->h_hit_cov; hits->allele = ctx->h_hit_allele; hits->total = ctx->h_hit_total;
+    const HitArrays<PinnedBuf>& h = ctx->h_hits;
+    hits->pos = h.pos; hits->pop_mask = h.pop; hits->ind_mask = h.ind; hits->cov = h.cov; hits->allele = h.allele; hits->total = h.total;
 }
 
 // the pileup kernel over items [a, a + n) of the window, count planes to d_tiles (slot 0 = item a)
@@ -470,15 +466,11 @@ static int run_window(msnv_ctx* ctx, uint32_t slot, const msnv_call_params* prm,
     // the window's reads are on the device once the copy stream reaches this point
     CU(cudaEventRecord(w.uploaded, ctx->copy_stream));
     CU(cudaStreamWaitEvent(st, w.uploaded, 0));
-    if (w.cap_samples < S) {
-        cudaFree(w.d_samples); w.d_samples = nullptr; w.cap_samples = 0;
-        CU(cudaMalloc((void**)&w.d_samples, sizeof(SampleDev) * S));
-        w.cap_samples = S;
-    }
+    CU(w.d_samples.ensure(S));
     CU(cudaMemcpyAsync(w.d_samples, w.h_samples.data(), sizeof(SampleDev) * S, cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync(ctx->d_err, 0, 4, st));
     CU(cudaMemsetAsync(ctx->d_scalar, 0, 32, st));
-    if (ensure_window_buffers(ctx, nt)) return MSNV_E_CUDA;
+    if (int rc = ensure_window_buffers(ctx, nt)) return rc;
 
     // ---- mate overlap: verdicts per quad for the samples that have pairs (read by the pileup kernel)
     uint64_t max_reads = 0, max_fix_reads = 0;
@@ -491,10 +483,7 @@ static int run_window(msnv_ctx* ctx, uint32_t slot, const msnv_call_params* prm,
     cudaEvent_t ev_m0 = ctx->ev[2], ev_m1 = ctx->ev[3];
     CU(cudaEventRecord(ev_m0, st));
     if (!fix_samples.empty()) {
-        if (fix_samples.size() > ctx->cap_fix_list) {
-            if (grow(ctx, ctx->d_fix_list, fix_samples.size() + 64)) return MSNV_E_CUDA;
-            ctx->cap_fix_list = fix_samples.size() + 64;
-        }
+        CU(ctx->d_fix_list.ensure(fix_samples.size(), fix_samples.size() + 64));
         // (pageable source: the copy is staged before the call returns)
         CU(cudaMemcpyAsync(ctx->d_fix_list, fix_samples.data(), fix_samples.size() * 4, cudaMemcpyHostToDevice, st));
         unsigned gc = (unsigned)((max_fix_reads * 2 + 255) / 256); if (gc < 1) gc = 1; if (gc > 1024) gc = 1024;          // ~27 bytes per read, 16 per thread
@@ -513,11 +502,11 @@ static int run_window(msnv_ctx* ctx, uint32_t slot, const msnv_call_params* prm,
     const uint64_t n_pairs_idx = (uint64_t)nt * S;
     const uint64_t n_blocks = (n_pairs_idx + 255) / 256;
     if (n_blocks > 0x7fffffffull) return fail(ctx, MSNV_E_LIMIT, "window too large: %u tiles x %u samples", nt, S);
-    if (n_blocks > ctx->cap_blocks) { if (grow(ctx, ctx->d_block_sums, n_blocks)) return MSNV_E_CUDA; ctx->cap_blocks = n_blocks; }
+    CU(ctx->d_block_sums.ensure(n_blocks));
     // the (r_lo, r_hi) of every pair found by the counting pass is kept for the emitting pass when it fits 1 GiB
     uint2* cache = nullptr;
     if (n_pairs_idx * 8 <= (1ull << 30)) {
-        if (n_pairs_idx > ctx->cap_range) { if (grow(ctx, ctx->d_range_cache, n_pairs_idx)) return MSNV_E_CUDA; ctx->cap_range = n_pairs_idx; }
+        CU(ctx->d_range_cache.ensure(n_pairs_idx));
         cache = ctx->d_range_cache;
     }
     // the index and the pileup rely on coordinate order within a sample; checked on the device (0.3 ms for 5e8 reads)
@@ -530,7 +519,7 @@ static int run_window(msnv_ctx* ctx, uint32_t slot, const msnv_call_params* prm,
                                                      : w.n_reads / 20 < n_pairs_idx;     // < 20 reads per (tile, sample) pair on average
     if (sparse) {
         const uint64_t words = (uint64_t)words_per_sample * S;
-        if (words > ctx->cap_bitmap) { if (grow(ctx, ctx->d_bitmap, words)) return MSNV_E_CUDA; ctx->cap_bitmap = words; }
+        CU(ctx->d_bitmap.ensure(words));
         CU(cudaMemsetAsync(ctx->d_bitmap, 0, words * 4, st));
         mark_kernel<<<dim3(gx, S), 256, 0, st>>>(w.d_samples, words_per_sample, w.t0, nt, ctx->d_bitmap);
         ++launches;
@@ -552,11 +541,7 @@ static int run_window(msnv_ctx* ctx, uint32_t slot, const msnv_call_params* prm,
     const uint32_t n_items = ctx->h_scalar[0];
     const uint64_t item_reads = (uint64_t)ctx->h_scalar[2] | (uint64_t)ctx->h_scalar[3] << 32;
     const uint32_t item_reads_max = ctx->h_scalar[4];
-    if (n_items > ctx->cap_items) {
-        const uint64_t cap = (uint64_t)n_items + n_items / 8 + 64;
-        if (grow(ctx, ctx->d_items, cap)) return MSNV_E_CUDA;
-        ctx->cap_items = cap;
-    }
+    CU(ctx->d_items.ensure(n_items, (uint64_t)n_items + n_items / 8 + 64));
     index_kernel<true><<<(unsigned)n_blocks, 256, 0, st>>>(w.d_samples, S, w.t0, nt, ctx->d_block_sums, ctx->d_items, ctx->d_tile_begin, cache, bitmap,
                                                            words_per_sample, nullptr);
     ++launches;
@@ -616,6 +601,37 @@ static int run_window(msnv_ctx* ctx, uint32_t slot, const msnv_call_params* prm,
     return MSNV_OK;
 }
 
+// the checks of msnv_window_add_sample / _raw: an open window in `slot`, a sample in range that was not added yet,
+// and a reference span within the limit
+static int check_add(msnv_ctx* ctx, uint32_t slot, uint32_t sample, uint32_t n_reads, uint32_t max_span, const char* fn)
+{
+    if (!ctx->open || slot >= (uint32_t)N_SLOTS || !ctx->win[slot].open) return fail(ctx, MSNV_E_STATE, "%s: no open window in this slot", fn);
+    if (sample >= ctx->S) return fail(ctx, MSNV_E_ARG, "%s: sample %u out of range", fn, sample);
+    if (ctx->win[slot].h_samples[sample].n_reads) return fail(ctx, MSNV_E_STATE, "%s: sample %u added twice", fn, sample);
+    if (n_reads && max_span > (uint32_t)MSNV_MAX_READ_SPAN)
+        return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit of %u", sample, max_span, (uint32_t)MSNV_MAX_READ_SPAN);
+    return MSNV_OK;
+}
+
+// whether a caller's array p sits at offset o of its batch starting at b (then a group goes up in one copy)
+static bool at(const void* p, const void* b, size_t o) { return static_cast<const uint8_t*>(p) == static_cast<const uint8_t*>(b) + o; }
+
+// a sample whose read group is in block rb and segment group in block sb joins the window
+static void attach_sample(msnv_ctx::Window& w, uint32_t sample, uint8_t* rb, const ReadGroup& g, uint8_t* sb, const SegmentGroup& sg,
+                          const msnv_sample_sizes& z)
+{
+    SampleDev& d = w.h_samples[sample];
+    d.pos = (const int32_t*)(rb + g.pos);
+    d.seg_off = (const uint32_t*)(rb + g.seg_off); d.q4_off = (const uint32_t*)(rb + g.q4_off);
+    d.mate = (const int32_t*)(rb + g.mate);
+    d.seg_pos = (const int32_t*)(sb + sg.seg_pos);  d.seg_len = (const uint16_t*)(sb + sg.seg_len);
+    d.seq2 = sb + sg.seq2;                         d.qual = sb + sg.qual;
+    d.fix = sg.fix ? sb + sg.fix : nullptr;
+    d.n_reads = z.n_reads; d.max_span = z.max_span;
+    w.n_reads += z.n_reads; w.n_bases += 4 * z.n_q4; w.n_segs += z.n_segs;
+    w.sizes[sample] = z;
+}
+
 extern "C" {
 
 int msnv_abi_version(void) { return MSNV_ABI_VERSION; }
@@ -642,11 +658,11 @@ int msnv_create(int device, msnv_ctx** out)
     CU(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
     for (auto& e : ctx->ev) CU(cudaEventCreate(&e));
     for (auto& w : ctx->win) CU(cudaEventCreateWithFlags(&w.uploaded, cudaEventDisableTiming));
-    CU(cudaMalloc((void**)&ctx->d_scalar, 32));
-    CU(cudaMalloc((void**)&ctx->d_err, 4));
-    CU(cudaMalloc((void**)&ctx->d_xstat, 16));
+    CU(ctx->d_scalar.ensure(8));
+    CU(ctx->d_err.ensure(1));
+    CU(ctx->d_xstat.ensure(2));
     CU(cudaMemset(ctx->d_xstat, 0, 16));
-    CU(cudaMallocHost((void**)&ctx->h_scalar, 32));
+    CU(ctx->h_scalar.ensure(8));
     for (bool gather : {false, true})
         for (int consumers : {128, 256})
             for (bool has_wide : {false, true})
@@ -661,22 +677,13 @@ void msnv_destroy(msnv_ctx* ctx)
     cudaSetDevice(ctx->device);
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
-    for (auto& w : ctx->win) { release_window(ctx, w); cudaFree(w.d_samples); cudaFree(w.d_aligned); if (w.uploaded) cudaEventDestroy(w.uploaded); }
+    for (auto& w : ctx->win) { release_window(ctx, w); if (w.uploaded) cudaEventDestroy(w.uploaded); }
     drop_pool(ctx);
     for (auto& sl : ctx->slabs) cudaFree(sl.base);
-    cudaFree(ctx->d_ref);
-    cudaFree(ctx->d_items); cudaFree(ctx->d_tiles); cudaFree(ctx->d_expect); cudaFree(ctx->d_text_acgt); cudaFree(ctx->d_text_match);
-    cudaFree(ctx->d_tile_begin); cudaFree(ctx->d_tile_hits); cudaFree(ctx->d_flags); cudaFree(ctx->d_block_sums); cudaFree(ctx->d_range_cache); cudaFree(ctx->d_bitmap);
-    cudaFree(ctx->d_scalar); cudaFree(ctx->d_err); cudaFree(ctx->d_fix_list); cudaFree(ctx->d_raw); cudaFree(ctx->d_xstat);
-    cudaFree(ctx->d_cov_diff); cudaFree(ctx->d_cov_beg); cudaFree(ctx->d_cov_end); cudaFree(ctx->d_cov_meta); cudaFree(ctx->d_cov_out);
-    cudaFree(ctx->d_hit_pos); cudaFree(ctx->d_hit_total); cudaFree(ctx->d_hit_pop); cudaFree(ctx->d_hit_ind);
-    cudaFree(ctx->d_hit_cov); cudaFree(ctx->d_hit_allele);
-    cudaFreeHost(ctx->h_hit_pos); cudaFreeHost(ctx->h_hit_total); cudaFreeHost(ctx->h_hit_pop); cudaFreeHost(ctx->h_hit_ind);
-    cudaFreeHost(ctx->h_hit_cov); cudaFreeHost(ctx->h_hit_allele); cudaFreeHost(ctx->h_scalar);
     for (auto& e : ctx->ev) if (e) cudaEventDestroy(e);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
-    delete ctx;
+    delete ctx;                                   // (the work buffers free themselves)
 }
 
 void* msnv_pinned_alloc(size_t bytes)
@@ -702,11 +709,10 @@ int msnv_shard_begin(msnv_ctx* ctx, uint32_t n_samples, uint32_t n_positions, co
     ++ctx->gen;
     for (auto& w : ctx->win) release_window(ctx, w);
     ctx->S = n_samples; ctx->P = n_positions; ctx->n_tiles = n_positions / TILE;
-    ctx->has_run = false;
-    cudaFree(ctx->d_ref); cudaFree(ctx->d_expect);
-    ctx->d_ref = nullptr; ctx->d_expect = nullptr;
-    CU(cudaMalloc((void**)&ctx->d_ref, n_positions));
-    CU(cudaMalloc((void**)&ctx->d_expect, n_positions));
+    ctx->open = ctx->has_run = false;             // (a failure below leaves no shard open)
+    ctx->d_ref.reset(); ctx->d_expect.reset();
+    CU(ctx->d_ref.ensure(n_positions));
+    CU(ctx->d_expect.ensure(n_positions));
     CU(cudaMemcpyAsync(ctx->d_ref, ref, n_positions, cudaMemcpyHostToDevice, ctx->stream));
     ctx->open = true;
     // the whole shard as one window in slot 0 until msnv_window_begin says otherwise
@@ -736,70 +742,50 @@ int msnv_window_begin(msnv_ctx* ctx, uint32_t slot, uint32_t pos_lo, uint32_t po
 int msnv_window_add_sample(msnv_ctx* ctx, uint32_t slot, uint32_t sample, const msnv_sample_reads* r)
 {
     if (!ctx || !r) return MSNV_E_ARG;
-    if (!ctx->open || slot >= (uint32_t)N_SLOTS || !ctx->win[slot].open) return fail(ctx, MSNV_E_STATE, "msnv_window_add_sample: no open window in this slot");
-    msnv_ctx::Window& w = ctx->win[slot];
-    if (sample >= ctx->S) return fail(ctx, MSNV_E_ARG, "msnv_window_add_sample: sample %u out of range", sample);
-    if (w.h_samples[sample].n_reads) return fail(ctx, MSNV_E_STATE, "msnv_window_add_sample: sample %u added twice", sample);
+    if (int rc = check_add(ctx, slot, sample, r->n_reads, r->max_span, __func__)) return rc;
     if (r->n_reads == 0) return MSNV_OK;
-    if (r->max_span > (uint32_t)MSNV_MAX_READ_SPAN) return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit of %u", sample, r->max_span, (uint32_t)MSNV_MAX_READ_SPAN);
+    msnv_ctx::Window& w = ctx->win[slot];
     CU(cudaSetDevice(ctx->device));
     const size_t n = r->n_reads, n1 = n + 1;
     const size_t n_seg = r->seg_off[n] - r->seg_off[0], n_q4 = r->q4_off[n] - r->q4_off[0];
     if (r->seg_off[0] != 0 || r->q4_off[0] != 0) return fail(ctx, MSNV_E_ARG, "sample %u: seg_off / q4_off must start at 0", sample);
     if (n_seg < n || n_q4 < n_seg) return fail(ctx, MSNV_E_ARG, "sample %u: inconsistent offsets (%zu reads, %zu segments, %zu quads)", sample, n, n_seg, n_q4);
-    // one allocation per sample, sub-arrays 256-byte aligned, 32 spare bytes behind every array
-    // because the pileup kernel's bulk copies read whole 16-byte units
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes + 32, 256); return o; };
     bool has_mates = false;
     for (size_t i = 0; i < n && !has_mates; ++i) has_mates = r->mate[i] >= 0;
-    const size_t o_pos = take(n * 4), o_sgo = take(n1 * 4), o_q4 = take(n1 * 4), o_mate = take(n * 4),
-                 o_sp = take(n_seg * 4), o_sl = take(n_seg * 2), o_seq = take(n_q4), o_qual = take(n_q4 * 4),
-                 o_fix = has_mates ? take(n_q4) : 0;       // verdicts of the mate-overlap rule, rebuilt by every run
-    uint8_t* base = (uint8_t*)take_block(ctx, w, off);
-    if (!base) return fail(ctx, MSNV_E_NOMEM, "sample %u: cannot allocate %zu bytes of device memory; process the shard in smaller windows (msnv_window_begin) or smaller genome bins (metaSNV.py --n_splits)", sample, off);
+    // one allocation per sample (the fix verdicts of the mate-overlap rule are rebuilt by every run)
+    BlockLayout layout;
+    const ReadGroup g(layout, n);
+    const SegmentGroup sg(layout, n_seg, n_q4, has_mates);
+    uint8_t* base = (uint8_t*)take_block(ctx, w, layout.size);
+    if (!base) return fail(ctx, MSNV_E_NOMEM, "sample %u: cannot allocate %zu bytes of device memory; process the shard in smaller windows (msnv_window_begin) or smaller genome bins (metaSNV.py --n_splits)", sample, layout.size);
     cudaStream_t st = ctx->copy_stream;
-    {
-        // a caller that packed the arrays the way this block is laid out (same order, same spacing) gets ONE copy instead of eight
-        const uint8_t* h0 = reinterpret_cast<const uint8_t*>(r->pos);
-        auto at = [&](const void* p, size_t o) { return reinterpret_cast<const uint8_t*>(p) == h0 + (o - o_pos); };
-        if (at(r->seg_off, o_sgo) && at(r->q4_off, o_q4) && at(r->mate, o_mate) && at(r->seg_pos, o_sp) && at(r->seg_len, o_sl) && at(r->seq2, o_seq) && at(r->qual, o_qual)) {
-            CU(cudaMemcpyAsync(base + o_pos, h0, o_qual + n_q4 * 4 - o_pos, cudaMemcpyHostToDevice, st));
-        } else {
-            CU(cudaMemcpyAsync(base + o_pos, r->pos, n * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_sgo, r->seg_off, n1 * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_q4, r->q4_off, n1 * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_mate, r->mate, n * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_sp, r->seg_pos, n_seg * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_sl, r->seg_len, n_seg * 2, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_seq, r->seq2, n_q4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_qual, r->qual, n_q4 * 4, cudaMemcpyHostToDevice, st));
-        }
+    // a caller that packed the arrays the way this block is laid out gets ONE copy instead of eight
+    const void* h0 = r->pos;
+    if (at(r->seg_off, h0, g.seg_off) && at(r->q4_off, h0, g.q4_off) && at(r->mate, h0, g.mate) && at(r->seg_pos, h0, sg.seg_pos) &&
+        at(r->seg_len, h0, sg.seg_len) && at(r->seq2, h0, sg.seq2) && at(r->qual, h0, sg.qual)) {
+        CU(cudaMemcpyAsync(base + g.pos, h0, sg.end - g.pos, cudaMemcpyHostToDevice, st));
+    } else {
+        CU(cudaMemcpyAsync(base + g.pos, r->pos, n * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + g.seg_off, r->seg_off, n1 * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + g.q4_off, r->q4_off, n1 * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + g.mate, r->mate, n * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + sg.seg_pos, r->seg_pos, n_seg * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + sg.seg_len, r->seg_len, n_seg * 2, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + sg.seq2, r->seq2, n_q4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + sg.qual, r->qual, n_q4 * 4, cudaMemcpyHostToDevice, st));
     }
-    SampleDev& d = w.h_samples[sample];
-    d.pos = (const int32_t*)(base + o_pos);
-    d.seg_off = (const uint32_t*)(base + o_sgo); d.q4_off = (const uint32_t*)(base + o_q4);
-    d.mate = (const int32_t*)(base + o_mate);
-    d.seg_pos = (const int32_t*)(base + o_sp);   d.seg_len = (const uint16_t*)(base + o_sl);
-    d.seq2 = base + o_seq;                      d.qual = base + o_qual;
-    d.fix = has_mates ? base + o_fix : nullptr;
-    d.n_reads = r->n_reads; d.max_span = r->max_span ? r->max_span : 1;
-    w.n_reads += n; w.n_bases += 4ull * n_q4; w.n_segs += n_seg;
     uint64_t n_aligned = 0;
     for (size_t k = 0; k < n_seg; ++k) n_aligned += r->seg_len[k];
-    w.sizes[sample] = msnv_sample_sizes{r->n_reads, 0, d.max_span, 0, (uint64_t)n_seg, (uint64_t)n_q4, n_aligned};
+    attach_sample(w, sample, base, g, base, sg, msnv_sample_sizes{r->n_reads, 0, r->max_span ? r->max_span : 1, 0, (uint64_t)n_seg, (uint64_t)n_q4, n_aligned});
     return MSNV_OK;
 }
 
 int msnv_window_add_sample_raw(msnv_ctx* ctx, uint32_t slot, uint32_t sample, const msnv_raw_reads* r)
 {
     if (!ctx || !r) return MSNV_E_ARG;
-    if (!ctx->open || slot >= (uint32_t)N_SLOTS || !ctx->win[slot].open) return fail(ctx, MSNV_E_STATE, "msnv_window_add_sample_raw: no open window in this slot");
-    msnv_ctx::Window& w = ctx->win[slot];
-    if (sample >= ctx->S) return fail(ctx, MSNV_E_ARG, "msnv_window_add_sample_raw: sample %u out of range", sample);
-    if (w.h_samples[sample].n_reads) return fail(ctx, MSNV_E_STATE, "msnv_window_add_sample_raw: sample %u added twice", sample);
+    if (int rc = check_add(ctx, slot, sample, r->n_reads, r->max_span, __func__)) return rc;
     if (r->n_reads == 0) return MSNV_OK;
-    if (r->max_span > (uint32_t)MSNV_MAX_READ_SPAN) return fail(ctx, MSNV_E_LIMIT, "sample %u: reference span %u exceeds the limit of %u", sample, r->max_span, (uint32_t)MSNV_MAX_READ_SPAN);
+    msnv_ctx::Window& w = ctx->win[slot];
     CU(cudaSetDevice(ctx->device));
     const size_t n = r->n_reads, n1 = n + 1;
     if (r->seg_off[0] != 0 || r->q4_off[0] != 0 || r->raw_off[0] != 0) return fail(ctx, MSNV_E_ARG, "sample %u: seg_off / q4_off / raw_off must start at 0", sample);
@@ -808,69 +794,48 @@ int msnv_window_add_sample_raw(msnv_ctx* ctx, uint32_t slot, uint32_t sample, co
     // (the records themselves are checked by expand_kernel: CIGAR against sequence length, blob size, offsets)
     bool has_mates = false;
     for (size_t i = 0; i < n && !has_mates; ++i) has_mates = r->mate[i] >= 0;
-    if (w.cap_aligned < ctx->S) {
-        cudaFree(w.d_aligned); w.d_aligned = nullptr; w.cap_aligned = 0;
-        CU(cudaMalloc((void**)&w.d_aligned, (size_t)ctx->S * 8));
-        w.cap_aligned = ctx->S;
-    }
+    CU(w.d_aligned.ensure(ctx->S));
     if (!w.has_raw) { CU(cudaMemsetAsync(w.d_aligned, 0, (size_t)ctx->S * 8, ctx->copy_stream)); w.has_raw = true; }
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes + 32, 256); return o; };
-    const size_t o_pos = take(n * 4), o_sgo = take(n1 * 4), o_q4 = take(n1 * 4), o_mate = take(n * 4),
-                 o_sp = take(n_seg * 4), o_sl = take(n_seg * 2), o_seq = take(n_q4), o_qual = take(n_q4 * 4),
-                 o_fix = has_mates ? take(n_q4) : 0;
-    uint8_t* base = (uint8_t*)take_block(ctx, w, off);
-    if (!base) return fail(ctx, MSNV_E_NOMEM, "sample %u: cannot allocate %zu bytes of device memory; process the shard in smaller windows (msnv_window_begin) or smaller genome bins (metaSNV.py --n_splits)", sample, off);
-    // staging of the BAM-shaped arrays: raw_off | raw | n_cigar | l_seq
-    size_t soff = 0;
-    auto stake = [&](size_t bytes) { size_t o = soff; soff = align_up(soff + bytes + 32, 256); return o; };
-    const size_t s_off = stake(n1 * 4), s_raw = stake(raw_words * 4), s_nc = stake(n * 2), s_ls = stake(n * 2), s_end = soff;
-    if (s_end > ctx->cap_raw) {
-        const uint64_t cap = s_end + s_end / 4 + (1u << 20);
-        if (grow(ctx, ctx->d_raw, cap)) return MSNV_E_CUDA;
-        ctx->cap_raw = cap;
-    }
+    BlockLayout layout;
+    const ReadGroup g(layout, n);
+    const SegmentGroup sg(layout, n_seg, n_q4, has_mates);
+    uint8_t* base = (uint8_t*)take_block(ctx, w, layout.size);
+    if (!base) return fail(ctx, MSNV_E_NOMEM, "sample %u: cannot allocate %zu bytes of device memory; process the shard in smaller windows (msnv_window_begin) or smaller genome bins (metaSNV.py --n_splits)", sample, layout.size);
+    // staging of the BAM-shaped arrays
+    BlockLayout staging;
+    const RawGroup x(staging, n, raw_words);
+    CU(ctx->d_raw.ensure(staging.size, staging.size + staging.size / 4 + (1u << 20)));
+    uint8_t* raw = ctx->d_raw;
     cudaStream_t st = ctx->copy_stream;
-    {
-        // packed callers (same order and spacing as the device side): two copies instead of eight
-        const uint8_t* h0 = reinterpret_cast<const uint8_t*>(r->pos);
-        const uint8_t* g0 = reinterpret_cast<const uint8_t*>(r->raw_off);
-        auto at = [](const void* p, const uint8_t* b, size_t o) { return reinterpret_cast<const uint8_t*>(p) == b + o; };
-        if (at(r->seg_off, h0, o_sgo - o_pos) && at(r->q4_off, h0, o_q4 - o_pos) && at(r->mate, h0, o_mate - o_pos)) {
-            CU(cudaMemcpyAsync(base + o_pos, h0, o_mate + n * 4 - o_pos, cudaMemcpyHostToDevice, st));
-        } else {
-            CU(cudaMemcpyAsync(base + o_pos, r->pos, n * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_sgo, r->seg_off, n1 * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_q4, r->q4_off, n1 * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(base + o_mate, r->mate, n * 4, cudaMemcpyHostToDevice, st));
-        }
-        if (at(r->raw, g0, s_raw - s_off) && at(r->n_cigar, g0, s_nc - s_off) && at(r->l_seq, g0, s_ls - s_off)) {
-            CU(cudaMemcpyAsync(ctx->d_raw + s_off, g0, s_ls + n * 2 - s_off, cudaMemcpyHostToDevice, st));
-        } else {
-            CU(cudaMemcpyAsync(ctx->d_raw + s_off, r->raw_off, n1 * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(ctx->d_raw + s_raw, r->raw, raw_words * 4, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(ctx->d_raw + s_nc, r->n_cigar, n * 2, cudaMemcpyHostToDevice, st));
-            CU(cudaMemcpyAsync(ctx->d_raw + s_ls, r->l_seq, n * 2, cudaMemcpyHostToDevice, st));
-        }
+    // packed callers (same order and spacing as the device side): two copies instead of eight
+    const void* h0 = r->pos;
+    const void* g0 = r->raw_off;
+    if (at(r->seg_off, h0, g.seg_off) && at(r->q4_off, h0, g.q4_off) && at(r->mate, h0, g.mate)) {
+        CU(cudaMemcpyAsync(base + g.pos, h0, g.end - g.pos, cudaMemcpyHostToDevice, st));
+    } else {
+        CU(cudaMemcpyAsync(base + g.pos, r->pos, n * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + g.seg_off, r->seg_off, n1 * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + g.q4_off, r->q4_off, n1 * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(base + g.mate, r->mate, n * 4, cudaMemcpyHostToDevice, st));
+    }
+    if (at(r->raw, g0, x.raw) && at(r->n_cigar, g0, x.n_cigar) && at(r->l_seq, g0, x.l_seq)) {
+        CU(cudaMemcpyAsync(raw + x.raw_off, g0, x.end - x.raw_off, cudaMemcpyHostToDevice, st));
+    } else {
+        CU(cudaMemcpyAsync(raw + x.raw_off, r->raw_off, n1 * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(raw + x.raw, r->raw, raw_words * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(raw + x.n_cigar, r->n_cigar, n * 2, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(raw + x.l_seq, r->l_seq, n * 2, cudaMemcpyHostToDevice, st));
     }
     // the aligned arrays are built in place: padding bytes must be 0
-    CU(cudaMemsetAsync(base + o_seq, 0, n_q4 + 32, st));
+    CU(cudaMemsetAsync(base + sg.seq2, 0, n_q4 + 32, st));
     RawDev in;
-    in.pos = (const int32_t*)(base + o_pos); in.seg_off = (const uint32_t*)(base + o_sgo); in.q4_off = (const uint32_t*)(base + o_q4);
-    in.raw_off = (const uint32_t*)(ctx->d_raw + s_off); in.raw = (const uint32_t*)(ctx->d_raw + s_raw);
-    in.n_cigar = (const uint16_t*)(ctx->d_raw + s_nc); in.l_seq = (const uint16_t*)(ctx->d_raw + s_ls); in.n_reads = r->n_reads;
-    expand_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(in, (int32_t*)(base + o_sp), (uint16_t*)(base + o_sl), base + o_seq, (uint32_t*)(base + o_qual), ctx->d_xstat, w.d_aligned + sample);
+    in.pos = (const int32_t*)(base + g.pos); in.seg_off = (const uint32_t*)(base + g.seg_off); in.q4_off = (const uint32_t*)(base + g.q4_off);
+    in.raw_off = (const uint32_t*)(raw + x.raw_off); in.raw = (const uint32_t*)(raw + x.raw);
+    in.n_cigar = (const uint16_t*)(raw + x.n_cigar); in.l_seq = (const uint16_t*)(raw + x.l_seq); in.n_reads = r->n_reads;
+    expand_kernel<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(in, (int32_t*)(base + sg.seg_pos), (uint16_t*)(base + sg.seg_len), base + sg.seq2, (uint32_t*)(base + sg.qual), ctx->d_xstat, w.d_aligned + sample);
     CU(cudaGetLastError());
-    SampleDev& d = w.h_samples[sample];
-    d.pos = (const int32_t*)(base + o_pos);
-    d.seg_off = (const uint32_t*)(base + o_sgo); d.q4_off = (const uint32_t*)(base + o_q4);
-    d.mate = (const int32_t*)(base + o_mate);
-    d.seg_pos = (const int32_t*)(base + o_sp);   d.seg_len = (const uint16_t*)(base + o_sl);
-    d.seq2 = base + o_seq;                      d.qual = base + o_qual;
-    d.fix = has_mates ? base + o_fix : nullptr;
-    d.n_reads = r->n_reads; d.max_span = r->max_span ? r->max_span : 1;
-    w.n_reads += n; w.n_bases += 4ull * n_q4; w.n_segs += n_seg;
-    w.sizes[sample] = msnv_sample_sizes{r->n_reads, 0, d.max_span, 0, (uint64_t)n_seg, (uint64_t)n_q4, 0};      // n_aligned: see msnv_window_sample_sizes
+    // n_aligned: see msnv_window_sample_sizes
+    attach_sample(w, sample, base, g, base, sg, msnv_sample_sizes{r->n_reads, 0, r->max_span ? r->max_span : 1, 0, (uint64_t)n_seg, (uint64_t)n_q4, 0});
     return MSNV_OK;
 }
 
@@ -925,20 +890,14 @@ int msnv_call_counts(msnv_ctx* ctx, uint32_t n_samples, uint32_t n_positions, co
     const uint32_t nt = ctx->n_tiles;
     const uint64_t n_items = (uint64_t)nt * n_samples;
     if (n_items > 0xffffffffull) return fail(ctx, MSNV_E_LIMIT, "msnv_call_counts: batch too large");
-    if (n_items > ctx->cap_items) {
-        if (grow(ctx, ctx->d_items, n_items + 64)) return MSNV_E_CUDA;
-        ctx->cap_items = n_items + 64;
-    }
+    CU(ctx->d_items.ensure(n_items, n_items + 64));
     if (int rc = ensure_tile_slots(ctx, n_items)) return rc;
-    if (ensure_window_buffers(ctx, nt)) return MSNV_E_CUDA;
+    if (int rc = ensure_window_buffers(ctx, nt)) return rc;
     memset(hits, 0, sizeof *hits);
     uint32_t launches = 0;
     CU(cudaMemsetAsync(ctx->d_err, 0, 4, st));
-    if (n_items > ctx->cap_text) {
-        if (grow(ctx, ctx->d_text_acgt, n_items * TILE)) return MSNV_E_CUDA;
-        if (grow(ctx, ctx->d_text_match, n_items * TILE)) return MSNV_E_CUDA;
-        ctx->cap_text = n_items;
-    }
+    CU(ctx->d_text_acgt.ensure(n_items * TILE));
+    CU(ctx->d_text_match.ensure(n_items * TILE));
     CU(cudaMemcpyAsync(ctx->d_text_acgt, acgt, n_items * TILE * 8, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(ctx->d_text_match, matches, n_items * TILE * 2, cudaMemcpyHostToDevice, st));
     expect_kernel<<<(ctx->P + 255) / 256, 256, 0, st>>>(ctx->d_ref, ctx->P, ctx->d_expect);
@@ -996,14 +955,15 @@ int msnv_shard_synth_ref(msnv_ctx* ctx, const msnv_synth_desc* d, int64_t* first
         if (int rc = msnv_shard_begin(ctx, S, (uint32_t)P, zero.data())) return rc;
         CU(cudaStreamSynchronize(st));
     }
-    uint32_t *d_off = nullptr, *d_len = nullptr;
-    CU(cudaMalloc((void**)&d_off, ((size_t)K + 1) * 4));
-    CU(cudaMalloc((void**)&d_len, (size_t)K * 4));
-    CU(cudaMemcpyAsync(d_off, off.data(), ((size_t)K + 1) * 4, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_len, d->contig_len, (size_t)K * 4, cudaMemcpyHostToDevice, st));
-    synth_ref_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(m, d_off, d_len, K, (uint32_t)P, ctx->d_ref);
-    CU(cudaStreamSynchronize(st));
-    cudaFree(d_off); cudaFree(d_len);
+    {
+        DevBuf<uint32_t> d_off, d_len;
+        CU(d_off.ensure((uint64_t)K + 1));
+        CU(d_len.ensure(K));
+        CU(cudaMemcpyAsync(d_off, off.data(), ((size_t)K + 1) * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_len, d->contig_len, (size_t)K * 4, cudaMemcpyHostToDevice, st));
+        synth_ref_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(m, d_off, d_len, K, (uint32_t)P, ctx->d_ref);
+        CU(cudaStreamSynchronize(st));
+    }
     // first pileup column of the shard: the smallest first fragment start over the samples' first contigs
     int64_t first_col = -1;
     for (uint32_t s = 0; s < S; ++s) {
@@ -1058,57 +1018,46 @@ int msnv_window_synth(msnv_ctx* ctx, uint32_t slot, const msnv_synth_desc* d, ui
             if (n_reads > 0x7fffffffull) return fail(ctx, MSNV_E_LIMIT, "msnv_shard_synth: more than 2^31 reads in one sample");
         }
         if (blocks.empty()) continue;
-        const size_t n = (size_t)n_reads, n1 = n + 1, nb = blocks.size(), nft = frag0.back();
+        const size_t n = (size_t)n_reads, nb = blocks.size(), nft = frag0.back();
         // ---- phase 1: per-read metadata (segments and quads per read, then their prefix sums)
-        size_t o = 0;
-        auto take = [&](size_t bytes) { size_t r = o; o = align_up(o + bytes + 32, 256); return r; };
-        const size_t o_pos = take(n * 4), o_sgo = take(n1 * 4), o_q4 = take(n1 * 4), o_mate = take(n * 4);
-        uint8_t* meta = (uint8_t*)take_block(ctx, w, o);
+        BlockLayout meta_layout;
+        const ReadGroup g(meta_layout, n);
+        uint8_t* meta = (uint8_t*)take_block(ctx, w, meta_layout.size);
         if (!meta) return fail(ctx, MSNV_E_NOMEM, "msnv_shard_synth: out of device memory (sample %u)", s);
-        SynthSampleCtg* d_blocks = nullptr; uint32_t *d_frag0 = nullptr, *d_nq = nullptr, *d_nsegs = nullptr, *d_for = nullptr;
-        CU(cudaMalloc((void**)&d_blocks, nb * sizeof(SynthSampleCtg)));
-        CU(cudaMalloc((void**)&d_frag0, (nb + 1) * 4));
-        CU(cudaMalloc((void**)&d_nq, n * 4));
-        CU(cudaMalloc((void**)&d_nsegs, n * 4));
-        CU(cudaMalloc((void**)&d_for, n * 4));
+        DevBuf<SynthSampleCtg> d_blocks;
+        DevBuf<uint32_t> d_frag0, d_nq, d_nsegs, d_for;
+        CU(d_blocks.ensure(nb));
+        CU(d_frag0.ensure(nb + 1));
+        CU(d_nq.ensure(n));
+        CU(d_nsegs.ensure(n));
+        CU(d_for.ensure(n));
         CU(cudaMemcpyAsync(d_blocks, blocks.data(), nb * sizeof(SynthSampleCtg), cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(d_frag0, frag0.data(), (nb + 1) * 4, cudaMemcpyHostToDevice, st));
         synth_meta_kernel<<<(unsigned)((nft + 127) / 128), 128, 0, st>>>(m, (int)s, paired, D, overlap, d_blocks, d_frag0, (uint32_t)nb, (uint32_t)nft,
-            (int32_t*)(meta + o_pos), d_nsegs, d_nq, (int32_t*)(meta + o_mate), d_for);
-        synth_scan2_kernel<<<1, 1024, 0, st>>>(d_nsegs, d_nq, (uint32_t)n, (uint32_t*)(meta + o_sgo), (uint32_t*)(meta + o_q4));
+            (int32_t*)(meta + g.pos), d_nsegs, d_nq, (int32_t*)(meta + g.mate), d_for);
+        synth_scan2_kernel<<<1, 1024, 0, st>>>(d_nsegs, d_nq, (uint32_t)n, (uint32_t*)(meta + g.seg_off), (uint32_t*)(meta + g.q4_off));
         uint32_t n_seg = 0, n_q4_u = 0;
-        CU(cudaMemcpyAsync(&n_seg, meta + o_sgo + n * 4, 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(&n_q4_u, meta + o_q4 + n * 4, 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&n_seg, meta + g.seg_off + n * 4, 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&n_q4_u, meta + g.q4_off + n * 4, 4, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         // ---- phase 2: segment records, bases, qualities
         const size_t n_q4 = n_q4_u;
         const uint32_t q_slots = q4 + 4;          // upper bound of the quads of one read (two segments)
-        o = 0;
-        const size_t o_sp = take((size_t)n_seg * 4), o_sl = take((size_t)n_seg * 2), o_seq = take(n_q4), o_qual = take(n_q4 * 4),
-                     o_fix = n_mated ? take(n_q4) : 0;
-        uint8_t* data = (uint8_t*)take_block(ctx, w, o);
+        BlockLayout data_layout;
+        const SegmentGroup sg(data_layout, n_seg, n_q4, n_mated != 0);
+        uint8_t* data = (uint8_t*)take_block(ctx, w, data_layout.size);
         if (!data) return fail(ctx, MSNV_E_NOMEM, "msnv_shard_synth: out of device memory (sample %u)", s);
         synth_fill_kernel<<<(unsigned)((n * q_slots + 255) / 256), 256, 0, st>>>(m, (int)s, paired, d_blocks, d_frag0, (uint32_t)nb, (uint32_t)n, q_slots,
-            (const int32_t*)(meta + o_pos), (const uint32_t*)(meta + o_sgo), (const uint32_t*)(meta + o_q4), d_for,
-            (int32_t*)(data + o_sp), (uint16_t*)(data + o_sl), data + o_seq, data + o_qual);
-        unsigned long long* d_sum = reinterpret_cast<unsigned long long*>(d_nq);     // d_nq is free again: reuse it for the sum
+            (const int32_t*)(meta + g.pos), (const uint32_t*)(meta + g.seg_off), (const uint32_t*)(meta + g.q4_off), d_for,
+            (int32_t*)(data + sg.seg_pos), (uint16_t*)(data + sg.seg_len), data + sg.seq2, data + sg.qual);
+        unsigned long long* d_sum = reinterpret_cast<unsigned long long*>(d_nq.p);     // d_nq is free again: reuse it for the sum
         CU(cudaMemsetAsync(d_sum, 0, 8, st));
-        sum_u16_kernel<<<(unsigned)std::min<size_t>(1024, ((size_t)n_seg + 255) / 256), 256, 0, st>>>((const uint16_t*)(data + o_sl), n_seg, d_sum);
+        sum_u16_kernel<<<(unsigned)std::min<size_t>(1024, ((size_t)n_seg + 255) / 256), 256, 0, st>>>((const uint16_t*)(data + sg.seg_len), n_seg, d_sum);
         unsigned long long n_aligned = 0;
         CU(cudaMemcpyAsync(&n_aligned, d_sum, 8, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         CU(cudaGetLastError());
-        cudaFree(d_blocks); cudaFree(d_frag0); cudaFree(d_nq); cudaFree(d_nsegs); cudaFree(d_for);
-        SampleDev& sd = w.h_samples[s];
-        sd.pos = (const int32_t*)(meta + o_pos);
-        sd.seg_off = (const uint32_t*)(meta + o_sgo); sd.q4_off = (const uint32_t*)(meta + o_q4);
-        sd.mate = (const int32_t*)(meta + o_mate);
-        sd.seg_pos = (const int32_t*)(data + o_sp);  sd.seg_len = (const uint16_t*)(data + o_sl);
-        sd.seq2 = data + o_seq;                      sd.qual = data + o_qual;
-        sd.fix = n_mated ? data + o_fix : nullptr;
-        sd.n_reads = (uint32_t)n; sd.max_span = L + 3;
-        w.n_reads += n; w.n_bases += 4ull * n_q4; w.n_segs += n_seg;
-        w.sizes[s] = msnv_sample_sizes{(uint32_t)n, (uint32_t)n_mated, L + 3, 0, (uint64_t)n_seg, (uint64_t)n_q4, (uint64_t)n_aligned};
+        attach_sample(w, s, meta, g, data, sg, msnv_sample_sizes{(uint32_t)n, (uint32_t)n_mated, L + 3, 0, (uint64_t)n_seg, (uint64_t)n_q4, (uint64_t)n_aligned});
     }
     return MSNV_OK;
 }
@@ -1189,13 +1138,11 @@ int msnv_shard_counts(msnv_ctx* ctx, uint32_t sample, uint32_t first, uint32_t n
         return fail(ctx, MSNV_E_STATE, "msnv_shard_counts: positions %u..%llu are outside the last range of tiles the run kept (%llu..%llu; the tile budget split the run)",
                     first, (unsigned long long)first + n, (unsigned long long)lo, (unsigned long long)hi);
     CU(cudaSetDevice(ctx->device));
-    uint16_t* d = nullptr;
-    CU(cudaMalloc((void**)&d, (size_t)n * 10));
+    DevBuf<uint16_t> d;                           // 5 counts per position
+    CU(d.ensure((uint64_t)n * 5));
     counts_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(ctx->d_tiles, ctx->d_items, ctx->last_item0, ctx->d_tile_begin, w.t0, ctx->d_expect, sample, first, n, d);
-    cudaError_t e = cudaMemcpyAsync(out, d, (size_t)n * 10, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    cudaFree(d);
-    if (e != cudaSuccess) return fail(ctx, MSNV_E_CUDA, "msnv_shard_counts: %s", cudaGetErrorString(e));
+    CU(cudaMemcpyAsync(out, d, (size_t)n * 10, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
     return MSNV_OK;
 }
 
@@ -1229,54 +1176,44 @@ int msnv_cov_run(msnv_ctx* ctx, const msnv_cov_blocks* b, uint32_t max_cov, uint
     chunk_contig.resize(n_chunks);
     for (uint32_t k = 0; k < K; ++k) for (uint32_t c = chunk0[k]; c < chunk0[k + 1]; ++c) chunk_contig[c] = k;
 
-    int rc = MSNV_OK;
-#define CUC(call)                                                                                                   \
-    do {                                                                                                            \
-        cudaError_t e_ = (call);                                                                                    \
-        if (e_ != cudaSuccess) { rc = fail(ctx, MSNV_E_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)); return rc; } \
-    } while (0)
     const size_t hist_n = (size_t)K * (max_cov + 1);
     const uint64_t n_diff = n_chunks * COV_CHUNK, n_meta = ((uint64_t)K + 1) + n_chunks + K + 2 * ((uint64_t)K + 1), n_out = K + hist_n;
-    if (n_diff > ctx->cap_cov_diff) { if (grow(ctx, ctx->d_cov_diff, n_diff + n_diff / 8)) return MSNV_E_CUDA; ctx->cap_cov_diff = n_diff + n_diff / 8; }
-    if (n_blocks > ctx->cap_cov_blocks) {
-        const uint64_t cap = n_blocks + n_blocks / 8 + 1024;
-        if (grow(ctx, ctx->d_cov_beg, cap) || grow(ctx, ctx->d_cov_end, cap)) return MSNV_E_CUDA;
-        ctx->cap_cov_blocks = cap;
-    }
-    if (n_meta > ctx->cap_cov_meta) { if (grow(ctx, ctx->d_cov_meta, n_meta + 1024)) return MSNV_E_CUDA; ctx->cap_cov_meta = n_meta + 1024; }
-    if (n_out > ctx->cap_cov_out) { if (grow(ctx, ctx->d_cov_out, n_out + 1024)) return MSNV_E_CUDA; ctx->cap_cov_out = n_out + 1024; }
+    CU(ctx->d_cov_diff.ensure(n_diff, n_diff + n_diff / 8));
+    CU(ctx->d_cov_beg.ensure(n_blocks, n_blocks + n_blocks / 8 + 1024));
+    CU(ctx->d_cov_end.ensure(n_blocks, n_blocks + n_blocks / 8 + 1024));
+    CU(ctx->d_cov_meta.ensure(n_meta, n_meta + 1024));
+    CU(ctx->d_cov_out.ensure(n_out, n_out + 1024));
     int32_t* d_diff = ctx->d_cov_diff;
     uint32_t *d_beg = ctx->d_cov_beg, *d_end = ctx->d_cov_end;
     uint32_t *d_chunk0 = ctx->d_cov_meta, *d_cc = d_chunk0 + (K + 1), *d_len = d_cc + n_chunks;
     uint64_t* d_off = reinterpret_cast<uint64_t*>(ctx->d_cov_meta + (((uint64_t)K + 1) + n_chunks + K + 1) / 2 * 2);     // 8-byte aligned
     unsigned long long *d_sum = ctx->d_cov_out, *d_hist = d_sum + K;
-    CUC(cudaMemsetAsync(d_diff, 0, n_diff * 4, st));
-    CUC(cudaMemsetAsync(d_sum, 0, n_out * 8, st));
+    CU(cudaMemsetAsync(d_diff, 0, n_diff * 4, st));
+    CU(cudaMemsetAsync(d_sum, 0, n_out * 8, st));
     if (n_blocks) {
-        CUC(cudaMemcpyAsync(d_beg, b->beg, n_blocks * 4, cudaMemcpyHostToDevice, st));
-        CUC(cudaMemcpyAsync(d_end, b->end, n_blocks * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_beg, b->beg, n_blocks * 4, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_end, b->end, n_blocks * 4, cudaMemcpyHostToDevice, st));
     }
-    CUC(cudaMemcpyAsync(d_chunk0, chunk0.data(), ((size_t)K + 1) * 4, cudaMemcpyHostToDevice, st));
-    CUC(cudaMemcpyAsync(d_cc, chunk_contig.data(), n_chunks * 4, cudaMemcpyHostToDevice, st));
-    CUC(cudaMemcpyAsync(d_len, b->contig_len, (size_t)K * 4, cudaMemcpyHostToDevice, st));
-    CUC(cudaMemcpyAsync(d_off, b->blk_off, ((size_t)K + 1) * 8, cudaMemcpyHostToDevice, st));
-    CUC(cudaEventRecord(ctx->ev[0], st));
+    CU(cudaMemcpyAsync(d_chunk0, chunk0.data(), ((size_t)K + 1) * 4, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_cc, chunk_contig.data(), n_chunks * 4, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_len, b->contig_len, (size_t)K * 4, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_off, b->blk_off, ((size_t)K + 1) * 8, cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(ctx->ev[0], st));
     if (n_blocks)
         cov_scatter_kernel<<<(unsigned)((n_blocks + 255) / 256), 256, 0, st>>>(d_beg, d_end, d_off, d_chunk0, K, n_blocks, d_diff);
-    CUC(cudaEventRecord(ctx->ev[1], st));
+    CU(cudaEventRecord(ctx->ev[1], st));
     cov_scan_kernel<<<(unsigned)n_chunks, COV_THREADS, 0, st>>>(d_diff, d_cc, d_chunk0, d_len, max_cov, d_sum, d_hist);
-    CUC(cudaEventRecord(ctx->ev[2], st));
-    CUC(cudaMemcpyAsync(cov_sum, d_sum, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
-    CUC(cudaMemcpyAsync(hist, d_hist, hist_n * 8, cudaMemcpyDeviceToHost, st));
-    CUC(cudaStreamSynchronize(st));
-    CUC(cudaGetLastError());
+    CU(cudaEventRecord(ctx->ev[2], st));
+    CU(cudaMemcpyAsync(cov_sum, d_sum, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(hist, d_hist, hist_n * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
     ctx->tm = msnv_timings{};
     cudaEventElapsedTime(&ctx->tm.ms_cov_scatter, ctx->ev[0], ctx->ev[1]);
     cudaEventElapsedTime(&ctx->tm.ms_cov_scan, ctx->ev[1], ctx->ev[2]);
     ctx->tm.cov_blocks = n_blocks; ctx->tm.kernel_launches = n_blocks ? 2u : 1u;
     for (uint32_t k = 0; k < K; ++k) ctx->tm.cov_positions += b->contig_len[k];
-#undef CUC
-    return rc;
+    return MSNV_OK;
 }
 
 }  // extern "C"
@@ -1287,30 +1224,15 @@ struct msnv_inflater {
     size_t max_bytes = 0;
     cudaStream_t stream = nullptr;
     std::string err;
-    uint8_t *h_comp = nullptr, *h_out = nullptr;                // page-locked staging, max_bytes each
-    uint8_t *d_comp = nullptr, *d_out = nullptr;
-    msnv_bgzf_member *h_m = nullptr, *d_m = nullptr;
-    int32_t *h_status = nullptr, *d_status = nullptr;
-    uint32_t cap_m = 0;
+    PinnedBuf<uint8_t> h_comp, h_out;                 // page-locked staging, max_bytes each
+    DevBuf<uint8_t> d_comp, d_out;
+    PinnedBuf<msnv_bgzf_member> h_m; DevBuf<msnv_bgzf_member> d_m;
+    PinnedBuf<int32_t> h_status; DevBuf<int32_t> d_status;
     cudaEvent_t ev[2] = {};
     float kernel_ms = 0;
 };
 
-namespace {
-int inf_fail(msnv_inflater* f, int code, const char* fmt, ...)
-{
-    char buf[512];
-    va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
-    if (f) f->err = buf;
-    return code;
-}
-#define CUI(call)                                                                                        \
-    do {                                                                                                 \
-        cudaError_t e_ = (call);                                                                         \
-        if (e_ != cudaSuccess) return inf_fail(inf, MSNV_E_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
-}  // namespace
-
+// (the inflater's functions call it `ctx`, the name CU records an error on)
 extern "C" {
 
 uint32_t msnv_inflater_max_members(size_t max_batch_bytes) { return (uint32_t)std::min<uint64_t>(max_batch_bytes / 64 + 1024, 0xffffffffu); }
@@ -1322,25 +1244,24 @@ int msnv_inflater_create(int device, size_t max_batch_bytes, msnv_inflater** out
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0 || device < 0 || device >= n) return MSNV_E_CUDA;
     if (max_batch_bytes == 0) return MSNV_E_ARG;
-    msnv_inflater* inf = new msnv_inflater();
-    inf->device = device;
-    inf->max_bytes = max_batch_bytes;
-    *out = inf;                                   // returned even on failure so the caller can read the error
-    CUI(cudaSetDevice(device));
-    CUI(cudaStreamCreateWithFlags(&inf->stream, cudaStreamNonBlocking));
-    for (auto& e : inf->ev) CUI(cudaEventCreate(&e));
-    CUI(cudaMallocHost((void**)&inf->h_comp, max_batch_bytes));
-    CUI(cudaMallocHost((void**)&inf->h_out, max_batch_bytes));
-    CUI(cudaMalloc((void**)&inf->d_comp, max_batch_bytes));
-    CUI(cudaMalloc((void**)&inf->d_out, max_batch_bytes));
+    msnv_inflater* ctx = new msnv_inflater();
+    ctx->device = device;
+    ctx->max_bytes = max_batch_bytes;
+    *out = ctx;                                   // returned even on failure so the caller can read the error
+    CU(cudaSetDevice(device));
+    CU(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
+    for (auto& e : ctx->ev) CU(cudaEventCreate(&e));
+    CU(ctx->h_comp.ensure(max_batch_bytes));
+    CU(ctx->h_out.ensure(max_batch_bytes));
+    CU(ctx->d_comp.ensure(max_batch_bytes));
+    CU(ctx->d_out.ensure(max_batch_bytes));
     // member arrays sized once for the largest batch: growing them later would free memory, which waits for the whole
     // device, including a context's work on another thread
     const uint64_t cap = msnv_inflater_max_members(max_batch_bytes);
-    CUI(cudaMallocHost((void**)&inf->h_m, cap * sizeof(msnv_bgzf_member)));
-    CUI(cudaMallocHost((void**)&inf->h_status, cap * 4));
-    CUI(cudaMalloc((void**)&inf->d_m, cap * sizeof(msnv_bgzf_member)));
-    CUI(cudaMalloc((void**)&inf->d_status, cap * 4));
-    inf->cap_m = (uint32_t)cap;
+    CU(ctx->h_m.ensure(cap));
+    CU(ctx->h_status.ensure(cap));
+    CU(ctx->d_m.ensure(cap));
+    CU(ctx->d_status.ensure(cap));
     return MSNV_OK;
 }
 
@@ -1349,11 +1270,9 @@ void msnv_inflater_destroy(msnv_inflater* inf)
     if (!inf) return;
     cudaSetDevice(inf->device);
     if (inf->stream) cudaStreamSynchronize(inf->stream);
-    cudaFreeHost(inf->h_comp); cudaFreeHost(inf->h_out); cudaFreeHost(inf->h_m); cudaFreeHost(inf->h_status);
-    cudaFree(inf->d_comp); cudaFree(inf->d_out); cudaFree(inf->d_m); cudaFree(inf->d_status);
     for (auto& e : inf->ev) if (e) cudaEventDestroy(e);
     if (inf->stream) cudaStreamDestroy(inf->stream);
-    delete inf;
+    delete inf;                                   // (the buffers free themselves)
 }
 
 const char* msnv_inflater_last_error(const msnv_inflater* inf) { return inf ? inf->err.c_str() : "no inflater (no CUDA device?)"; }
@@ -1365,40 +1284,40 @@ int msnv_inflater_kernel_ms(const msnv_inflater* inf, float* ms)
     return MSNV_OK;
 }
 
-int msnv_inflate(msnv_inflater* inf, const uint8_t* comp, size_t comp_bytes, const msnv_bgzf_member* m, uint32_t n,
+int msnv_inflate(msnv_inflater* ctx, const uint8_t* comp, size_t comp_bytes, const msnv_bgzf_member* m, uint32_t n,
                  uint8_t* out, int32_t* status)
 {
-    if (!inf || (n && (!comp || !m || !out || !status))) return MSNV_E_ARG;
-    inf->kernel_ms = 0;
+    if (!ctx || (n && (!comp || !m || !out || !status))) return MSNV_E_ARG;
+    ctx->kernel_ms = 0;
     if (n == 0) return MSNV_OK;
-    if (n > inf->cap_m) return inf_fail(inf, MSNV_E_LIMIT, "msnv_inflate: %u members exceed the inflater's %u", n, inf->cap_m);
-    if (comp_bytes > inf->max_bytes) return inf_fail(inf, MSNV_E_ARG, "msnv_inflate: %zu compressed bytes exceed the inflater's batch of %zu", comp_bytes, inf->max_bytes);
+    if (n > ctx->d_m.cap) return fail(ctx, MSNV_E_LIMIT, "msnv_inflate: %u members exceed the inflater's %u", n, (uint32_t)ctx->d_m.cap);
+    if (comp_bytes > ctx->max_bytes) return fail(ctx, MSNV_E_ARG, "msnv_inflate: %zu compressed bytes exceed the inflater's batch of %zu", comp_bytes, ctx->max_bytes);
     uint64_t out_bytes = 0;
     for (uint32_t i = 0; i < n; ++i) {
         if (m[i].coff > comp_bytes || m[i].clen > comp_bytes - m[i].coff)
-            return inf_fail(inf, MSNV_E_ARG, "msnv_inflate: member %u lies outside the %zu compressed bytes", i, comp_bytes);
-        if (m[i].ooff > inf->max_bytes || m[i].isize > inf->max_bytes - m[i].ooff)
-            return inf_fail(inf, MSNV_E_ARG, "msnv_inflate: member %u's output exceeds the inflater's batch of %zu bytes", i, inf->max_bytes);
+            return fail(ctx, MSNV_E_ARG, "msnv_inflate: member %u lies outside the %zu compressed bytes", i, comp_bytes);
+        if (m[i].ooff > ctx->max_bytes || m[i].isize > ctx->max_bytes - m[i].ooff)
+            return fail(ctx, MSNV_E_ARG, "msnv_inflate: member %u's output exceeds the inflater's batch of %zu bytes", i, ctx->max_bytes);
         out_bytes = std::max<uint64_t>(out_bytes, m[i].ooff + m[i].isize);
     }
-    CUI(cudaSetDevice(inf->device));
-    cudaStream_t st = inf->stream;
-    memcpy(inf->h_comp, comp, comp_bytes);
-    memcpy(inf->h_m, m, (size_t)n * sizeof(msnv_bgzf_member));
-    CUI(cudaMemcpyAsync(inf->d_comp, inf->h_comp, comp_bytes, cudaMemcpyHostToDevice, st));
-    CUI(cudaMemcpyAsync(inf->d_m, inf->h_m, (size_t)n * sizeof(msnv_bgzf_member), cudaMemcpyHostToDevice, st));
-    CUI(cudaEventRecord(inf->ev[0], st));
-    inflate_kernel<<<(n + INFLATE_WARPS - 1) / INFLATE_WARPS, INFLATE_WARPS * 32, 0, st>>>(inf->d_comp, inf->d_m, n, inf->d_out, inf->d_status);
-    CUI(cudaGetLastError());
-    CUI(cudaEventRecord(inf->ev[1], st));
-    CUI(cudaMemcpyAsync(inf->h_out, inf->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
-    CUI(cudaMemcpyAsync(inf->h_status, inf->d_status, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-    CUI(cudaStreamSynchronize(st));
-    cudaEventElapsedTime(&inf->kernel_ms, inf->ev[0], inf->ev[1]);
-    memcpy(out, inf->h_out, out_bytes);
-    memcpy(status, inf->h_status, (size_t)n * 4);
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    memcpy(ctx->h_comp, comp, comp_bytes);
+    memcpy(ctx->h_m, m, (size_t)n * sizeof(msnv_bgzf_member));
+    CU(cudaMemcpyAsync(ctx->d_comp, ctx->h_comp, comp_bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(ctx->d_m, ctx->h_m, (size_t)n * sizeof(msnv_bgzf_member), cudaMemcpyHostToDevice, st));
+    CU(cudaEventRecord(ctx->ev[0], st));
+    inflate_kernel<<<(n + INFLATE_WARPS - 1) / INFLATE_WARPS, INFLATE_WARPS * 32, 0, st>>>(ctx->d_comp, ctx->d_m, n, ctx->d_out, ctx->d_status);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(ctx->ev[1], st));
+    CU(cudaMemcpyAsync(ctx->h_out, ctx->d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(ctx->h_status, ctx->d_status, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    cudaEventElapsedTime(&ctx->kernel_ms, ctx->ev[0], ctx->ev[1]);
+    memcpy(out, ctx->h_out, out_bytes);
+    memcpy(status, ctx->h_status, (size_t)n * 4);
     return MSNV_OK;
 }
 
 }  // extern "C"
-#undef CUI
+#undef CU

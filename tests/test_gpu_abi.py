@@ -141,6 +141,28 @@ def test_cov_run_refuses_histograms_above_the_limit(built):
     assert s.tolist() == [10, 0] and h[0].tolist() == [4990, 10, 0, 0] and h[1].tolist() == [7000, 0, 0, 0]
 
 
+def test_cov_run_failed_allocation_leaves_the_context_usable(built):
+    """A call whose difference array cannot be allocated (64 contigs of 2^32 - 1 positions: about 1.1 TiB) returns
+    MSNV_E_CUDA. The buffer it could not grow is left empty and the runtime's error is cleared, so the next call on the
+    same context allocates it again and gives the result it gave before."""
+    import ctypes as C
+    from metasnv_b200 import abi
+    lens = np.array([5000, 7000], np.uint32)
+    off = np.array([0, 1, 2], np.uint64)
+    beg, end = np.array([10, 100], np.uint32), np.array([20, 4000], np.uint32)
+    huge = np.full(64, 0xFFFFFFFF, np.uint32)
+    huge_off = np.zeros(65, np.uint64)
+    b = abi.CovBlocks(64, abi._ptr(huge), abi._ptr(huge_off), None, None)
+    cov_sum, hist = np.zeros(64, np.uint64), np.zeros(64, np.uint64)
+    with abi.Context(0) as ctx:
+        s0, h0 = ctx.cov_run(lens, off, beg, end, 3)
+        assert ctx.lib.msnv_cov_run(ctx.h, C.byref(b), 0, abi._ptr(cov_sum), abi._ptr(hist)) == -1     # MSNV_E_CUDA
+        assert "out of memory" in ctx.lib.msnv_last_error(ctx.h).decode()
+        s1, h1 = ctx.cov_run(lens, off, beg, end, 3)
+    assert s0.tolist() == [10, 3900] and s1.tolist() == s0.tolist()
+    assert np.array_equal(h1, h0)
+
+
 def _called_positions(path, offsets):
     out = []
     for line in open(path):
